@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - exact k-NN QPS of the B200 path next to the reference's CPU path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c3] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c3] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic queries against the resident
 corpus. Default workload: BASELINE.json configs[2] "10M x 768 cosine, k=10, 4096-query batch,
@@ -19,6 +19,10 @@ Besides the contract's keys the line carries
           C5 at batch 1 and 64 - and for SURVEY section 8d's stress inputs at C2 scale (clustered rows, duplicated rows,
           queries drawn from the corpus, 0.1 % rows with 100x the norm), each with its own parity check and
           refined / fallback counters.
+
+--dump-outputs DIR writes what the last timed step returned (see dump_outputs), so that two builds can be compared
+output for output: the corpus and the queries depend only on the arguments (seeded), never on the run.
+The library is the one build() left next to the package; bench.py compiles and caches nothing in the tree.
 """
 from __future__ import annotations
 
@@ -52,6 +56,7 @@ for _b in (1, 2, 4, 8, 16, 32, 64):
                                label=f"latency sweep batch {_b}, k=10 over 10M x 768")
 GEN_CHUNK = 65_536  # rows per seeded generation chunk (BASELINE.md §3.1)
 STRESS = ("clustered", "duplicates", "queries_from_corpus", "norm_outliers")
+DUMP_MAX_BYTES = 64 << 20
 
 
 def peaks() -> dict:
@@ -606,12 +611,26 @@ def also_block(args, ctx, c3_corpus, device, pk) -> dict:
     return out
 
 
+def dump_outputs(out_dir: str, rows: np.ndarray, dist: np.ndarray) -> None:
+    """The search result a caller receives, one line per query of the batch: `neighbour_rows.npy` (global row numbers as
+    float64, exact below 2^53; -1 pads), `neighbour_distances.npy` (float32) and `query_index.npy` (float64: which query of
+    the batch each line answers). Above DUMP_MAX_BYTES in all, a fixed sample of the queries (seed 0, in batch order)."""
+    n_q, k = rows.shape
+    per_query = k * (8 + 4) + 8
+    index = np.arange(n_q)
+    if n_q * per_query > DUMP_MAX_BYTES:
+        index = np.sort(np.random.default_rng(0).choice(n_q, DUMP_MAX_BYTES // per_query, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "neighbour_rows.npy"), rows[index].astype(np.float64))
+    np.save(os.path.join(out_dir, "neighbour_distances.npy"), dist[index].astype(np.float32))
+    np.save(os.path.join(out_dir, "query_index.npy"), index.astype(np.float64))
+
+
 def run_ours(args, cfg: dict) -> dict:
     import torch
     import torch.distributed as td
 
     from fenix_b200 import knn
-    from fenix_b200.csrc.build import build as build_lib
     from fenix_b200.dist import ReplicaSearcher, ShardedSearcher, shard_bounds
 
     rank = int(os.environ.get("RANK", 0))
@@ -621,8 +640,6 @@ def run_ours(args, cfg: dict) -> dict:
         raise SystemExit(f"--gpus {args.gpus} but WORLD_SIZE={world}: launch with torchrun --nproc-per-node {args.gpus}")
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a B200: the search path has no CPU fallback")
-    if rank == 0:
-        build_lib()
     device = torch.device("cuda", local)
     torch.cuda.set_device(device)
     if world > 1:
@@ -700,6 +717,8 @@ def run_ours(args, cfg: dict) -> dict:
     if rank == 0:   # the two paths must agree (same kernels, different plumbing)
         assert np.array_equal(h_rows.numpy(), rows_h) and np.array_equal(h_dist.numpy(), dist_h), \
             "e2e result differs from the device-resident result"
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, rows_h, dist_h)
 
     def rank_max(x: float) -> float:
         if world == 1:
@@ -828,7 +847,14 @@ def main() -> None:
                     help="tuning only: a stress variant of the synthetic corpus (SURVEY.md section 8d)")
     ap.add_argument("--rows", type=int, default=0, help="tuning only: override the corpus row count of the config")
     ap.add_argument("--queries", type=int, default=0, help="tuning only: override the query batch of the config")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the neighbour rows and distances of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the GPU path: the reference arm's last step depends on its time budget")
+    sys.dont_write_bytecode = True      # the tree may be read-only: nothing is cached in it
     cfg = dict(CONFIGS[args.config])
     if args.rows or args.queries or args.variant:
         cfg["n"] = args.rows or cfg["n"]

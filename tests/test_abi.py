@@ -37,7 +37,11 @@ def test_abi_version_and_no_torch_dependency(built_library):
 
 
 def test_sass_is_sm100a(built_library):
-    out = subprocess.run(["cuobjdump", "-lelf", built_library], capture_output=True, text=True).stdout
+    from fenix_b200.csrc.build import nvcc_path
+
+    # the toolkit that built the library, whether or not its bin/ is on PATH
+    cuobjdump = os.path.join(os.path.dirname(os.path.realpath(nvcc_path())), "cuobjdump")
+    out = subprocess.run([cuobjdump, "-lelf", built_library], capture_output=True, text=True).stdout
     assert "sm_100a" in out, out
 
 

@@ -2,6 +2,7 @@
 outputs of the live reference. Bar: neighbour ids bit-exact under (distance, row) order,
 distances within 1e-5 relative (BASELINE.json north_star), tolerance written in conftest."""
 import os
+import socket
 
 import numpy as np
 import pyarrow as pa
@@ -18,6 +19,14 @@ pytestmark = pytest.mark.gpu
 
 def client_root(served):
     return served[3]
+
+
+def free_port():
+    """A port no one listens on now: runs of the suite that share a host do not collide."""
+    with socket.socket() as s:
+        s.bind(("127.0.0.1", 0))
+        return s.getsockname()[1]
+
 
 # "fp32": the library's own routing (a handful of queries over a small shard take the single-launch direct scan);
 # "fp32_tc": the same exact mode with the direct scan switched off, so the tensor-core path answers; "scan": the checker
@@ -991,12 +1000,13 @@ class TestFlightDropIn:
     """The reference's own acceptance test (tests/test_flight.py:42-50, 88-114, 151-154) re-run against
     this package, plus result parity it does not check."""
 
-    VECTOR_SIZE, NUM_VECTORS, BATCH_SIZE, PORT = 256, 20_000, 1_000, 9137
+    VECTOR_SIZE, NUM_VECTORS, BATCH_SIZE = 256, 20_000, 1_000
 
     @pytest.fixture(scope="class")
     def served(self, tmp_path_factory, built_library):
         root = str(tmp_path_factory.mktemp("fenix"))
-        server = fenix.Server(root, "127.0.0.1", self.PORT)
+        port = free_port()
+        server = fenix.Server(root, "127.0.0.1", port)
         rng = np.random.default_rng(42)
         parts = []
         for _ in range(self.NUM_VECTORS // self.BATCH_SIZE):
@@ -1004,7 +1014,7 @@ class TestFlightDropIn:
             parts.append(x + 10 * x[0, :])
         corpus = np.concatenate(parts)
         source = table_of(corpus, self.BATCH_SIZE)
-        client = fenix.Flight("127.0.0.1", self.PORT)
+        client = fenix.Flight("127.0.0.1", port)
         client.make_table("test/table", source.to_reader())
         yield client, source, corpus, root
         client.remove()
@@ -1106,7 +1116,7 @@ def test_flight_serves_the_row_sharded_path(built_library, tmp_path, monkeypatch
     n_dev = min(torch.cuda.device_count(), 4)
     monkeypatch.setenv("FENIX_DEVICES", ",".join(str(i) for i in range(n_dev)))
     root = str(tmp_path / "served")
-    port = 9151
+    port = free_port()
     server = fenix.Server(root, "127.0.0.1", port)
     client = fenix.Flight("127.0.0.1", port)
     rng = np.random.default_rng(314)

@@ -7,6 +7,19 @@ from conftest import METRICS, golden_cases, golden_filter, load_golden, table_of
 from oracle import brute_force_f64, call, canonical, distance, search_rows
 from oracle.fenix_oracle import _cdist_mm
 
+# torch threads of the run that recorded the ref_*.npz outputs (tests/golden/PROVENANCE.txt)
+GOLDEN_TORCH_THREADS = 8
+
+
+@pytest.fixture
+def golden_torch_threads():
+    """MKL divides an sgemm's work by the intra-op thread count, so the last bits of a distance depend on that count
+    (D = 100 differs at 1, 2 or 4 threads): replay the recorded calls with the count they ran with."""
+    before = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_TORCH_THREADS)
+    yield
+    torch.set_num_threads(before)
+
 
 @pytest.mark.parametrize("shape", [(1, 1000, 128), (1, 1000, 256), (1, 513, 100), (4, 2000, 96), (30, 40, 8)])
 def test_l2_restatement_is_bitwise_torch_cdist(shape):
@@ -25,7 +38,7 @@ def test_unknown_metric_raises_value_error():
 
 @pytest.mark.parametrize("case", golden_cases())
 @pytest.mark.parametrize("metric", METRICS)
-def test_oracle_reproduces_live_reference(case, metric):
+def test_oracle_reproduces_live_reference(case, metric, golden_torch_threads):
     """ids and distances bit-identical to what fenix.io.index.call returned, in its own order."""
     g = load_golden(case)
     table = table_of(g["corpus"], int(g["chunk"]))
