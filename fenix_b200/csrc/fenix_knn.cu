@@ -134,7 +134,10 @@ struct fx_corpus {
   float* X = nullptr;
   void* Xb = nullptr;              // bf16 shadow of X (+ three -|x|^2/2 columns) for the bf16 filter, tiled (tc_filter.cuh)
   void* Xn = nullptr;              // bf16 shadow of the normalised rows (cosine), built by the first cosine search
+  void* X8 = nullptr;              // int8 shadow of the normalised rows (exact cosine at small k), built by the first search that takes it
+  float2* x8_tile = nullptr;       // (S_t, E_t) of every tile of X8 (tc_filter.cuh, i8_scale)
   bool xn_failed = false;          // no memory for Xn: cosine keeps the plain shadow + multiplicative epilogue
+  bool x8_failed = false;          // no memory for X8: cosine keeps the bf16 shadows
   bool xb_failed = false;          // no memory for Xb: the TF32 filter over the fp32 rows serves L2 / inner product
   int shadow_mode = -1;            // FENIX_BF16_SHADOW at finalize: -1 lazy (default), 0 never, 1 plain shadow built at finalize
   int pitch_b = 0;                 // elements per row of the bf16 QUERY matrix that goes with the shadows (ShadowGeom::pitch_q)
@@ -155,7 +158,7 @@ struct fx_corpus {
     cudaGraphExec_t exec = nullptr;
     void* ptrs[7] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // buffers baked into the graph
     uint64_t knob_epoch = 0;
-    int path = 0, variant = 0, launches = 0;
+    int path = 0, variant = 0, launches = 0, operand = 0;
   };
   std::vector<GraphEntry> graphs;
   // inverted index for batched IVF searches (fx_corpus_set_cells): local rows grouped by cell
@@ -466,6 +469,8 @@ extern "C" int fx_corpus_destroy(fx_corpus* c) {
   if (c->X) cudaFree(c->X);
   if (c->Xb) cudaFree(c->Xb);
   if (c->Xn) cudaFree(c->Xn);
+  if (c->X8) cudaFree(c->X8);
+  if (c->x8_tile) cudaFree(c->x8_tile);
   if (c->hx) cudaFree(c->hx);
   if (c->rx) cudaFree(c->rx);
   if (c->max_n2_bits) cudaFree(c->max_n2_bits);
@@ -638,14 +643,60 @@ static bool ensure_norm_shadow(fx_corpus* c) {
   return true;
 }
 
+// The int8 normalised shadow (kind 2: 128 int8 columns per k-block, a (S_t, E_t) pair per tile): operand of exact cosine
+// searches at small k over rows wider than the resident-query kernel's (int8_wanted). Half the bytes of the bf16
+// normalised shadow and twice its tensor rate; its scores are certified upper bounds with a looser error than bf16's,
+// so K' grows (TC_KP_I8) and large k keeps the bf16 shadow. FENIX_BF16_SHADOW=0 and FENIX_NO_NORM_SHADOW stop it too.
+static bool ensure_i8_shadow(fx_corpus* c) {
+  fx_ctx* ctx = c->ctx;
+  if (c->tc.ok_8) return true;
+  if (c->x8_failed || !shadow_allowed(c) || ctx->tc.knobs.no_norm_shadow) return false;
+  NvtxRange nvtx("fenix:build_int8_shadow");
+  const int n_kb = fx::i8_n_kb(c->dim);
+  const int64_t n_tiles = (c->n + fx::TC_BN - 1) / fx::TC_BN;
+  const size_t shadow_bytes = size_t(n_tiles) * n_kb * fx::TC_BN * fx::I8_KB, tile_bytes = size_t(n_tiles) * sizeof(float2);
+  size_t free_b = 0, total_b = 0;
+  if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess || free_b < shadow_bytes + tile_bytes + (size_t(4) << 30) ||
+      cudaMalloc(&c->X8, shadow_bytes) != cudaSuccess || cudaMalloc(&c->x8_tile, tile_bytes) != cudaSuccess) {
+    cudaGetLastError();
+    if (c->X8) cudaFree(c->X8);
+    c->X8 = nullptr; c->x8_tile = nullptr; c->x8_failed = true;
+    return false;
+  }
+  const int blocks = int(std::min<int64_t>(n_tiles, int64_t(ctx->sm_count) * 8));
+  fx::to_i8_tiled_kernel<<<blocks, 256, 0, ctx->stream>>>(c->X, c->n, c->pitch, c->dim, n_kb, n_tiles,
+                                                          static_cast<int8_t*>(c->X8), c->x8_tile);
+  std::string err;
+  if (cudaGetLastError() != cudaSuccess || cudaStreamSynchronize(ctx->stream) != cudaSuccess ||
+      !fx::tc_bind_shadow(&ctx->tc, &c->tc.map_x8, &c->tc.map_x8_h, c->X8, c->n, n_kb, &err, 1)) {
+    cudaGetLastError(); cudaFree(c->X8); cudaFree(c->x8_tile); c->X8 = nullptr; c->x8_tile = nullptr; c->x8_failed = true;
+    return false;
+  }
+  ctx->launches++; c->stats.kernel_launches++;
+  c->stats.device_bytes += int64_t(shadow_bytes + tile_bytes);
+  c->tc.ok_8 = true;
+  return true;
+}
+
+// Exact cosine searches the int8 filter takes (FENIX_INT8 -1): rows wider than 192 columns - narrower ones take the
+// resident-query kernel, which its epilogue binds - and k <= 16, where K' = TC_KP_I8 covers the rows the int8 bound lets
+// past the k-th neighbour (k = 32 would need ~700).
+static bool int8_wanted(const fx_corpus* c, int metric, int k, int precision) {
+  const int knob = c->ctx->tc.knobs.int8;
+  if (metric != 1 || precision != FX_PREC_FP32 || knob == 0 || c->ctx->tc.knobs.fp32_filter_tf32) return false;
+  return knob > 0 || (c->dim > 192 && k <= 16);
+}
+
 // Operand kind, shadow and epilogue form of one filter launch (see TcSearch). With a row mask the per-row
 // epilogue term carries the mask: masked rows get -inf (additive forms) or NaN (multiplicative form), which can
 // never pass the threshold test.
 static int configure_filter(fx_corpus* c, int metric, int kind, const uint8_t* d_mask, fx::TcSearch* s) {
   fx_ctx* ctx = c->ctx;
   s->kind = kind; s->pitch_b = c->pitch_b; s->shadow = 0; s->aug = 0; s->epi = metric;
-  s->hx = c->hx; s->rx = c->rx; s->Xb = c->Xb; s->Xn = c->Xn;
-  if (kind == 1) {
+  s->hx = c->hx; s->rx = c->rx; s->Xb = c->Xb; s->Xn = c->Xn; s->X8 = c->X8; s->i8_tile = c->x8_tile;
+  if (kind == 2) {   // cosine over the int8 normalised shadow: upper bounds straight out of the MMA and the tile constants
+    s->epi = 2; s->pitch_b = fx::I8_KB * fx::i8_n_kb(c->dim);
+  } else if (kind == 1) {
     const int errcol = ctx->tc.knobs.errcol;
     if (metric == 0) { s->aug = 1; s->epi = 2; }                       // -|x|^2/2 and the row's error weight ride in the shadow's extra columns
     else if (metric == 1) { if (ensure_norm_shadow(c)) { s->shadow = 1; s->epi = 2; s->Xn = c->Xn; } else ensure_plain_shadow(c); }
@@ -659,8 +710,8 @@ static int configure_filter(fx_corpus* c, int metric, int kind, const uint8_t* d
     const int64_t n_alloc = ((c->n + 255) / 256) * 256;
     FX_TRY(ctx->d_maskn.ensure(size_t(n_alloc) * sizeof(float)));
     float* mn = static_cast<float*>(ctx->d_maskn.p);
-    // mode 0: hx or -inf (added), 1: rx or NaN (multiplied), 2: 0 or -inf (added)
-    const int mode = s->epi == 2 ? 2 : s->epi;
+    // mode 0: hx or -inf (added), 1: rx or NaN (multiplied), 2: 0 or -inf (added), 3: int8 filter's integer term
+    const int mode = kind == 2 ? 3 : (s->epi == 2 ? 2 : s->epi);
     fx::masked_norms_kernel<<<int(std::min<int64_t>((n_alloc + 255) / 256, int64_t(ctx->sm_count) * 8)), 256, 0, ctx->stream>>>(
         d_mask, mode == 1 ? c->rx : c->hx, c->n, n_alloc, mode, mn);
     FX_CUDA(cudaGetLastError());
@@ -704,7 +755,8 @@ static fx::DirectPlan direct_plan_for(const fx_corpus* c, int64_t n_q, int k, in
 
 struct SearchRun {
   bool tc = false;            // the tensor-core path ran (flags are meaningful)
-  int path = 0;               // 0 exact scan, 1 tensor-core TF32 filter, 2 tensor-core bf16 filter, 3 direct scan (one launch)
+  int path = 0;               // 0 exact scan, 1 tensor-core TF32 filter, 2 tensor-core shadow filter (bf16 or int8), 3 direct scan (one launch)
+  int operand = 0;            // operand kind of the filter: 0 fp32 / TF32, 1 bf16, 2 int8
   fx::TcSearch s{};
   fx::TcLaunch L{};
   const float* d_q = nullptr; int64_t n_q = 0; int metric = 0, k = 0;
@@ -717,7 +769,7 @@ struct SearchRun {
 static int search_enqueue(fx_corpus* c, const float* d_q, int64_t n_q, int metric, int k, int precision,
                           const uint8_t* d_mask, int64_t* d_out_rows, float* d_out_dist, SearchRun* run) {
   fx_ctx* ctx = c->ctx;
-  run->tc = false; run->path = 0; run->d_q = d_q; run->n_q = n_q; run->metric = metric; run->k = k;
+  run->tc = false; run->path = 0; run->operand = 0; run->d_q = d_q; run->n_q = n_q; run->metric = metric; run->k = k;
   run->d_mask = d_mask; run->d_out_rows = d_out_rows; run->d_out_dist = d_out_dist;
   ctx->h_word[0] = 0;
   const unsigned ev_flags = ctx->capturing ? cudaEventRecordExternal : cudaEventRecordDefault;
@@ -771,11 +823,13 @@ static int search_enqueue(fx_corpus* c, const float* d_q, int64_t n_q, int metri
     s.row_base = c->row_base; s.max_norm = c->max_norm; s.Q = d_q; s.n_q = int(n_q); s.metric = metric; s.k = k;
     s.certify = precision == FX_PREC_FP32; s.out_rows = d_out_rows; s.out_dist = d_out_dist;
     s.stream = ctx->stream; s.ev_k0 = ctx->ev_k0; s.ev_k1 = ctx->ev_k1; s.ev_flags = ev_flags; s.dbg = nullptr; s.tau_fixed = nullptr;
-    // operand kind of the filter: exact mode takes the bf16 shadow when the shard has one
-    // (the shadow this metric streams is built here, by its first search: normalised rows for cosine, else the plain one)
+    // operand kind of the filter: exact mode takes the int8 normalised shadow for cosine at small k (int8_wanted), else the
+    // bf16 shadow when the shard has one (the shadow a search streams is built here, by its first search: normalised rows
+    // for cosine, else the plain one)
+    const bool have_i8 = int8_wanted(c, metric, k, precision) && ensure_i8_shadow(c);
     const bool want_bf16 = precision == FX_PREC_BF16 || (precision == FX_PREC_FP32 && !ctx->tc.knobs.fp32_filter_tf32);
-    const bool have_shadow = want_bf16 && ((metric == 1 && ensure_norm_shadow(c)) || ensure_plain_shadow(c));
-    const int kind = have_shadow ? 1 : 0;
+    const bool have_shadow = !have_i8 && want_bf16 && ((metric == 1 && ensure_norm_shadow(c)) || ensure_plain_shadow(c));
+    const int kind = have_i8 ? 2 : (have_shadow ? 1 : 0);
     if (precision == FX_PREC_BF16 && !have_shadow)
       return fail(FX_ESTATE, "fx_search: FX_PREC_BF16 needs a bf16 shadow (none could be built: FENIX_BF16_SHADOW=0, a tiny shard, or no HBM left)");
     FX_TRY(configure_filter(c, metric, kind, d_mask, &s));
@@ -784,7 +838,7 @@ static int search_enqueue(fx_corpus* c, const float* d_q, int64_t n_q, int metri
     std::string err;
     int launched = 0, variant = 0;
     if (!fx::tc_search(&ctx->tc, &c->tc, s, run->L, ctx->d_tc.p, &launched, &err, &variant)) return fail(FX_ECUDA, "fx_search: %s", err.c_str());
-    run->tc = true; run->path = 1 + kind;
+    run->tc = true; run->path = kind == 0 ? 1 : 2; run->operand = kind;
     c->stats.last_variant = variant;
     ctx->launches += launched; c->stats.kernel_launches += launched;
     if (s.certify) FX_CUDA(cudaMemcpyAsync(ctx->h_word, fx::tc_flag_count(ctx->d_tc.p), sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
@@ -855,7 +909,7 @@ static int search_settle(fx_corpus* c, SearchRun* run, bool* changed) {
     double c_err = 0.0, c_add = 0.0;
     fx::tc_cert_consts(s, &c_err, &c_add);
     fx::refine_prep_kernel<<<n_f, 128, 0, ctx->stream>>>(d_q, static_cast<const int*>(ctx->d_qlist.p), c->dim, metric, k,
-                                                        d_out_dist, c->max_norm, c_err, c_add, q_r, tau_fixed);
+                                                        d_out_dist, c->max_norm, c_err, c_add, q_r, tau_fixed, s.kind == 2 ? 1 : 0);
     FX_CUDA(cudaGetLastError());
     fx::TcSearch s2 = s;
     s2.Q = q_r; s2.n_q = n_f; s2.out_rows = rows2; s2.out_dist = dist2; s2.certify = true;
@@ -933,7 +987,7 @@ static void search_account(fx_corpus* c, const SearchRun& run) {
   else cudaEventElapsedTime(&ms, ctx->ev_start, ctx->ev_stop);
   if (run.path == 3) kms = ms;   // the direct scan is its one kernel (no inner events: they cost host time on the latency path)
   else cudaEventElapsedTime(&kms, ctx->ev_k0, ctx->ev_k1);
-  c->stats.last_search_ms = ms; c->stats.last_main_kernel_ms = kms; c->stats.last_path = run.path;
+  c->stats.last_search_ms = ms; c->stats.last_main_kernel_ms = kms; c->stats.last_path = run.path; c->stats.last_operand = run.operand;
   c->stats.searches++; c->stats.queries += run.n_q;
 }
 
@@ -1017,7 +1071,7 @@ static bool graph_capture(fx_corpus* c, fx_corpus::GraphEntry* g, int64_t n_q, i
   g->exec = exec; g->state = 1; g->knob_epoch = ctx->knob_epoch;
   const void* now[7] = {ctx->d_q.p, ctx->d_rows.p, ctx->d_dist.p, ctx->d_tc.p, ctx->h_q.p, ctx->h_rows.p, ctx->h_dist.p};
   for (int i = 0; i < 7; ++i) g->ptrs[i] = const_cast<void*>(now[i]);
-  g->path = run->path; g->variant = c->stats.last_variant; g->launches = int(c->stats.kernel_launches - launches0);
+  g->path = run->path; g->operand = run->operand; g->variant = c->stats.last_variant; g->launches = int(c->stats.kernel_launches - launches0);
   c->stats.kernel_launches = launches0;   // counted when the graph runs
   return true;
 }
@@ -1108,7 +1162,7 @@ extern "C" int fx_search(fx_corpus* c, const float* queries, int64_t n_q, int32_
       std::memcpy(ctx->h_q.p, queries, q_bytes);
       ctx->h_word[0] = 0;
       FX_CUDA(cudaGraphLaunch(g->exec, ctx->stream));
-      run.tc = true; run.path = g->path; run.n_q = n_q;
+      run.tc = true; run.path = g->path; run.operand = g->operand; run.n_q = n_q;
       c->stats.last_variant = g->variant;
       ctx->launches += g->launches; c->stats.kernel_launches += g->launches;
       launched = true;
@@ -1331,7 +1385,10 @@ extern "C" int fx_debug_scores(fx_corpus* c, const float* queries, int64_t n_q, 
   s.metric = metric; s.k = 10; s.certify = false; s.out_rows = static_cast<int64_t*>(ctx->d_rows.p);
   s.out_dist = static_cast<float*>(ctx->d_dist.p); s.stream = ctx->stream; s.ev_k0 = ctx->ev_k0; s.ev_k1 = ctx->ev_k1;
   s.dbg = d_dbg; s.tau_fixed = nullptr;
-  FX_TRY(configure_filter(c, metric, (ctx->tc.knobs.debug_bf16 && ((metric == 1 && ensure_norm_shadow(c)) || ensure_plain_shadow(c))) ? 1 : 0, nullptr, &s));
+  // operand: FENIX_INT8=1 and cosine - the int8 filter's upper bounds; FENIX_DEBUG_BF16 - the bf16 filter; else TF32
+  const bool i8 = metric == 1 && ctx->tc.knobs.int8 > 0 && ensure_i8_shadow(c);
+  const bool b16 = !i8 && ctx->tc.knobs.debug_bf16 && ((metric == 1 && ensure_norm_shadow(c)) || ensure_plain_shadow(c));
+  FX_TRY(configure_filter(c, metric, i8 ? 2 : (b16 ? 1 : 0), nullptr, &s));
   const fx::TcLaunch L = fx::tc_prepare(&ctx->tc, s);
   FX_TRY(ctx->d_tc.ensure(L.scratch_bytes));
   std::string err; int launched = 0;

@@ -88,6 +88,32 @@ inline ShadowGeom shadow_geom(int dim) {
   return g;
 }
 
+// The int8 normalised shadow (cosine, operand kind 2) and its quantised queries. ONE format, used by the shadow builder,
+// the query quantiser, the filter epilogue and the certificate: a vector v (a corpus row or a query) is normalised in
+// fp64, v^ = v / max(|v|, 1e-12) (the rerank's eps), and quantised with a scale S shared by its group (a 256-row tile of
+// the shard, or the query alone), S = 127 / max |v^_i| over the group:  v~ = clamp(rint(S v^_i), -127, 127). With the
+// residuals r_x = x^ - x~/S_t and r_q = q^ - q~/S_q, exactly
+//     cos(q, x) = q~.x~ / (S_t S_q) + (q~/S_q).r_x + r_q.x^   <=   acc / (S_t S_q) + a_q E_t + e_q
+// where acc = q~.x~ (exact in the int32 accumulator), E_t = max |r_x| over the tile's rows, a_q = |q~| / S_q and
+// e_q = |r_q| (|x^| <= 1), all rounded up. So the filter score of a row is a certified UPPER bound of its exact cosine.
+// Rows: 128 int8 columns per k-block (128 B, as a bf16 k-block), tiles of 256 rows; a tile's (S_t, E_t) is a float2.
+constexpr int I8_KB = 128;                 // int8 columns per k-block
+inline int i8_n_kb(int dim) { return (dim + I8_KB - 1) / I8_KB; }
+__host__ __device__ __forceinline__ float i8_scale(double max_abs) { return max_abs > 0.0 ? float(127.0 / max_abs) : 1.f; }
+__device__ __forceinline__ int i8_quant(double v, float scale) {
+  return int(fmin(fmax(rint(v * double(scale)), -127.0), 127.0));
+}
+// acc -> the row's certified upper bound (ae = a_q E_t + e_q, padded for the rounding of this expression)
+__device__ __forceinline__ float i8_upper(int acc, double inv_ss, double ae) { return __double2float_ru(fma(double(acc), inv_ss, ae)); }
+// Integer admission threshold of one (query, tile): every acc whose upper bound can exceed tau is above it (the margin
+// covers the fp32 rounding of the bound). Never below I8_FLOOR, so a masked row (row term I8_MASKED) can never pass.
+constexpr int I8_FLOOR = -(1 << 29);       // below every unmasked acc: |acc| <= 127^2 D < 2^28 for D <= 16384
+constexpr int I8_MASKED = -(1 << 30);
+__device__ __forceinline__ int i8_threshold(float tau, double ss, double ae) {
+  const double x = (double(tau) - ae) * ss - ss * 0x1p-21 - 2.0;
+  return x >= 2147483647.0 ? 0x7fffffff : (x > double(I8_FLOOR) ? int(floor(x)) : I8_FLOOR);
+}
+
 // Tuning knobs. Read from the environment ONCE per context (fx_init) - the search path never calls getenv - and
 // settable per context afterwards through fx_set_option (same names).
 struct TcKnobs {
@@ -126,6 +152,8 @@ struct TcKnobs {
   int merge_rank_min = 0;  // FENIX_MERGE_RANK_MIN candidates per query (lists x k) from which the exchange merges by rank (binary searches
                            //                      over the sorted lists) instead of a shared-memory sort; 0: built-in default
   int debug_direct = 0;    // FENIX_DEBUG_DIRECT   stderr timeline (globaltimer stamps) of every direct scan launched by fx_search
+  int int8 = -1;           // FENIX_INT8           exact cosine filters with int8 MMAs over the int8 normalised shadow: -1 auto (rows
+                           //                      wider than 192 columns, k <= 16), 0 never, 1 whenever the metric and precision allow
 };
 // name = the environment variable's name; value = its text, or null to restore the default. False: unknown name.
 inline bool tc_set_knob(TcKnobs* k, const char* name, const char* value) {
@@ -164,6 +192,7 @@ inline bool tc_set_knob(TcKnobs* k, const char* name, const char* value) {
   else if (n == "FENIX_DIRECT_SPIN") k->direct_spin = as_int(d.direct_spin);
   else if (n == "FENIX_DIRECT_QREG") k->direct_qreg = as_int(d.direct_qreg);
   else if (n == "FENIX_MERGE_RANK_MIN") k->merge_rank_min = as_int(d.merge_rank_min);
+  else if (n == "FENIX_INT8") k->int8 = as_int(d.int8);
   else return false;
   return true;
 }
@@ -172,7 +201,7 @@ inline void tc_knobs_from_env(TcKnobs* k) {
       "FENIX_TC_KP", "FENIX_TC_FULLK", "FENIX_TC_NO_RQ", "FENIX_TC_SLICES", "FENIX_TC_MAX_WAVES", "FENIX_TC_ORDER", "FENIX_TC_KP_LIST",
       "FENIX_TC_PRE_WIDE", "FENIX_TC_PRE", "FENIX_TC_PRE_SMALL", "FENIX_TC_PRE_SAFETY", "FENIX_TC_PRE_M", "FENIX_TC_PF", "FENIX_RQ_STAGES",
       "FENIX_FIN_THREADS", "FENIX_TC_WARM", "FENIX_TC_PAIR", "FENIX_TC_ERRCOL", "FENIX_FP32_FILTER_TF32", "FENIX_NO_REFINE",
-      "FENIX_NO_NORM_SHADOW", "FENIX_DEBUG_BF16", "FENIX_DEBUG_TIERS", "FENIX_GRAPH", "FENIX_DIRECT", "FENIX_DIRECT_MAX_MB", "FENIX_DEBUG_DIRECT", "FENIX_DIRECT_SPIN", "FENIX_DIRECT_QREG", "FENIX_MERGE_RANK_MIN"};
+      "FENIX_NO_NORM_SHADOW", "FENIX_DEBUG_BF16", "FENIX_DEBUG_TIERS", "FENIX_GRAPH", "FENIX_DIRECT", "FENIX_DIRECT_MAX_MB", "FENIX_DEBUG_DIRECT", "FENIX_DIRECT_SPIN", "FENIX_DIRECT_QREG", "FENIX_MERGE_RANK_MIN", "FENIX_INT8"};
   for (const char* name : names) {
     if (const char* v = std::getenv(name)) tc_set_knob(k, name, v);
   }
@@ -188,9 +217,11 @@ struct TcCorpus {
   CUtensorMap map_xb;      // bf16 shadow, tiled [tile][k-block][256 rows][64], box 64 x 256 = one contiguous 32 KB block
   CUtensorMap map_xn;      // bf16 shadow of the NORMALISED rows x/|x| (cosine), same layout, built on first use
   CUtensorMap map_xb_h, map_xn_h;   // the same shadows seen through 128-row boxes (resident-query kernel)
+  CUtensorMap map_x8, map_x8_h;     // int8 shadow of the normalised rows (cosine, kind 2), same tiling with 128 columns per k-block
   bool ok = false;
   bool ok_b = false;
   bool ok_n = false;
+  bool ok_8 = false;
 };
 struct TcSearch {
   const float* X; const float* hx; const float* rx; int64_t n_rows; int dim; int pitch; int64_t row_base;
@@ -198,12 +229,14 @@ struct TcSearch {
   int64_t* out_rows; float* out_dist; cudaStream_t stream; cudaEvent_t ev_k0, ev_k1;
   unsigned ev_flags;       // cudaEventRecordExternal while the search is being captured into a CUDA graph, else 0
   float* dbg;              // optional [128][256] raw score dump (diagnostics)
-  int kind;                // 0: TF32 filter over the fp32 rows, 1: bf16 filter over the bf16 shadow
-  int pitch_b;             // elements per row of the bf16 shadow (multiple of 8)
+  int kind;                // 0: TF32 filter over the fp32 rows, 1: bf16 filter over a bf16 shadow, 2: int8 filter over the int8
+                           // normalised shadow (cosine; scores are certified upper bounds of the exact cosine)
+  int pitch_b;             // elements per row of the bf16 (kind 2: int8) query matrix (whole 128-byte k-blocks)
+  const float2* i8_tile;   // kind 2: (S_t, E_t) of every shard tile
   const uint32_t* tau_fixed; // refinement pass: preset per-query admission thresholds (ordered encoding) or null
   int epi;                   // epilogue form: 0 score = acc + hx[row], 1 score = acc * rx[row], 2 score = acc
   int shadow;                // kind 1: 0 = plain shadow (+ augmented columns), 1 = normalised shadow
-  const void* Xb; const void* Xn;   // device addresses of the two shadows (L2 prefetch)
+  const void* Xb; const void* Xn; const void* X8;   // device addresses of the shadows (L2 prefetch)
   int aug;                   // kind 1: the query's augmented columns. 1 (L2): [1, 1, 1, u] pick up the shadow's -|x|^2/2 terms
                              // and the row's error weight; 2 (inner product, rows of very different norm): [0, 0, 0, u];
                              // u = c |q| rounded up, so that the filter score is a certified UPPER bound of the exact score
@@ -315,6 +348,14 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t desc_a, uint
       "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t"
       "}" ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate) : "memory");
 }
+__device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t"
+      ".reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t"
+      "}" ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate) : "memory");
+}
 // Arrive on an mbarrier once every previously issued tcgen05.mma of this thread has completed.
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
@@ -362,6 +403,14 @@ __device__ __forceinline__ void umma_bf16_pair(uint32_t tmem_d, uint64_t desc_a,
       "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t"
       "}" ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate) : "memory");
 }
+__device__ __forceinline__ void umma_i8_pair(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t"
+      ".reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p;\n\t"
+      "}" ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate) : "memory");
+}
 // Arrive (once the pair's previously issued MMAs have completed) on the mbarrier at this offset in BOTH CTAs.
 __device__ __forceinline__ void umma_commit_pair(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
@@ -385,6 +434,11 @@ __host__ __device__ constexpr uint32_t make_idesc_tf32(int m, int n) {
 // kind::f16 with bf16 operands, fp32 accumulate, both operands K-major.
 __host__ __device__ constexpr uint32_t make_idesc_bf16(int m, int n) {
   return (1u << 4) | (1u << 7) | (1u << 10) | (uint32_t(n >> 3) << 17) | (uint32_t(m >> 4) << 24);
+}
+// kind::i8 with signed 8-bit operands, s32 accumulate, both operands K-major: D format S32 = 2 in bits [4,6), A and B
+// format signed = 1 in bits [7,10) and [10,13), no saturation (bit 3: the sums are far from the int32 range).
+__host__ __device__ constexpr uint32_t make_idesc_i8(int m, int n) {
+  return (2u << 4) | (1u << 7) | (1u << 10) | (uint32_t(n >> 3) << 17) | (uint32_t(m >> 4) << 24);
 }
 
 __device__ __forceinline__ void tmem_ld_32x32b_x32(uint32_t taddr, uint32_t (&v)[32]) {
@@ -467,6 +521,8 @@ struct TcParams {
   int fixed;              // refinement pass: thresholds are preset in tau_g, no selection; buffer overflow sets flags[q]
   int* flags;             // [n_q]
   float* dbg;             // diagnostics: raw scores of (query tile 0) x (corpus tile 0), [128][256], or null
+  const float2* i8_tile;  // kind 2: (S_t, E_t) per shard tile
+  const float4* i8_q;     // kind 2: (S_q, a_q, e_q, 0) per query
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -648,6 +704,95 @@ __device__ __forceinline__ void epi_tile(uint32_t t_acc, int ncols, const float*
   if (MODE == 2) { if (pre_out != nullptr) *pre_out = ncols >= TC_HALF_COLS ? blk_max : -INFINITY; }
 }
 
+// The same tile for the int8 filter (kind 2): the accumulators are int32 and the scan stays in the integer domain -
+// quad maxima and the compare against the (query, tile) threshold thr (i8_threshold) are one integer instruction per
+// element, as in epi_tile. Only appended hits are converted, to the float upper bound (i8_upper), so candidate lists,
+// tau_g and the finish kernel keep their float order encoding. METRIC 0 (masked searches): nrm holds an integer row
+// term, 0 or I8_MASKED. MODE 2 records block maxima in upper-bound units, MODE 1 dumps upper bounds.
+template <int METRIC, int MODE, int PAIR = 0>
+__device__ __forceinline__ void epi_tile_i8(uint32_t t_acc, int ncols, const float* nrm, int col0, float tau, int thr,
+                                            double inv_ss, double ae, uint2* buf, uint32_t& wn, uint64_t* release_bar,
+                                            uint32_t release_leader, uint64_t* norm_release, uint32_t lane, float* dbg_row,
+                                            float* pre_out) {
+  int blk_max = I8_FLOOR;
+  const int* term = reinterpret_cast<const int*>(nrm);
+  auto release = [&]() {
+    tc_fence_before();
+    __syncwarp();
+    if (lane == 0) {
+      if (PAIR) {
+        mbar_arrive_cluster(release_leader);
+        if (METRIC != 2) mbar_arrive(norm_release);
+      } else {
+        mbar_arrive(release_bar);
+      }
+    }
+  };
+  auto scan = [&](uint32_t (&v)[TC_CW], int c) {
+    if (METRIC == 0) {
+#pragma unroll
+      for (int j = 0; j < TC_CW; j += 4) {
+        const int4 n4 = *reinterpret_cast<const int4*>(term + c + j);
+        v[j + 0] += uint32_t(n4.x); v[j + 1] += uint32_t(n4.y); v[j + 2] += uint32_t(n4.z); v[j + 3] += uint32_t(n4.w);
+      }
+    }
+    if (MODE == 1) {
+      if (dbg_row != nullptr) {
+#pragma unroll
+        for (int j = 0; j < TC_CW; ++j) dbg_row[c + j] = i8_upper(int(v[j]), inv_ss, ae);
+      }
+    }
+    int qm[TC_CW / 4];
+#pragma unroll
+    for (int g = 0; g < TC_CW / 4; ++g)
+      qm[g] = max(max(int(v[4 * g + 0]), int(v[4 * g + 1])), max(int(v[4 * g + 2]), int(v[4 * g + 3])));
+    int m = qm[0];
+#pragma unroll
+    for (int g = 1; g < TC_CW / 4; ++g) m = max(m, qm[g]);
+    if (MODE == 2) { blk_max = max(blk_max, m); return; }
+    if (__any_sync(0xffffffffu, m > thr)) {
+      uint32_t mine = 0;
+#pragma unroll
+      for (int g = 0; g < TC_CW / 4; ++g) mine |= (qm[g] > thr) ? (1u << g) : 0u;
+      uint32_t quads = __reduce_or_sync(0xffffffffu, mine);
+      while (quads) {                       // warp-uniform
+        const int g = __ffs(quads) - 1;
+        quads &= quads - 1;
+        const int cq = c + 4 * g;
+        uint32_t w[4];
+        tmem_ld_32x32b_x4(t_acc + uint32_t(cq), w);
+        tmem_ld_wait();
+        int4 n4 = make_int4(0, 0, 0, 0);
+        if (METRIC == 0) n4 = *reinterpret_cast<const int4*>(term + cq);
+        const int nn[4] = {n4.x, n4.y, n4.z, n4.w};
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          const int a = int(w[j]);
+          if (a + nn[j] > thr && cq + j < ncols) {
+            const float sc = i8_upper(a, inv_ss, ae);
+            if (sc > tau) { buf[wn] = make_uint2(__float_as_uint(sc), uint32_t(col0 + cq + j)); ++wn; }
+          }
+        }
+      }
+    }
+  };
+  if (ncols > 0) {
+    uint32_t va[TC_CW], vb[TC_CW];
+    tmem_ld_32x32b_x32(t_acc, va);
+#pragma unroll TC_EPI_UNROLL
+    for (int c = 0; c < TC_HALF_COLS; c += 2 * TC_CW) {
+      tmem_ld_wait_dep(va);
+      tmem_ld_32x32b_x32(t_acc + uint32_t(c + TC_CW), vb);
+      scan(va, c);
+      tmem_ld_wait_dep(vb);
+      if (c + 2 * TC_CW < TC_HALF_COLS) tmem_ld_32x32b_x32(t_acc + uint32_t(c + 2 * TC_CW), va);
+      scan(vb, c + TC_CW);
+    }
+  }
+  release();
+  if (MODE == 2) { if (pre_out != nullptr) *pre_out = ncols >= TC_HALF_COLS ? i8_upper(blk_max, inv_ss, ae) : -INFINITY; }
+}
+
 // Tighten thresholds after a tile. The common case costs one compare and one vote: every lane keeps the entry count
 // at which it needs attention (wn_trig): K' while it has no threshold yet, cap - 127 (the next tile could overflow
 // the buffer) afterwards. A lane that got there receives a warp-cooperative selection; its new threshold is shared
@@ -688,7 +833,8 @@ __device__ __forceinline__ void epi_tighten(const TcParams& p, bool active, int 
 // ---------------------------------------------------------------------------------------------
 // KIND 0: fp32 operands read as TF32 (k-block = 32 elements, UMMA K = 8)
 // KIND 1: bf16 operands          (k-block = 64 elements, UMMA K = 16); both are 128 B rows / 32 B per MMA
-// PAIR 1: CTA pairs (cluster of 2, tcgen05 cta_group::2, bf16 shadow only). The pair computes a 256-query x 256-row
+// KIND 2: int8 operands          (k-block = 128 elements, UMMA K = 32, int32 accumulators; epilogue epi_tile_i8)
+// PAIR 1: CTA pairs (cluster of 2, tcgen05 cta_group::2, bf16 or int8 shadow). The pair computes a 256-query x 256-row
 //         tile per MMA: each CTA stages ITS query tile (A, 16 KB per k-block) and HALF of the corpus block (B, 128 of
 //         the 256 rows, 16 KB); the tensor cores of both SMs read both halves. Per SM and k-block that is 32 KB of
 //         L2 -> SM operand traffic instead of 48 KB, at the same tensor work (measured on C3, one CTA per tile:
@@ -701,7 +847,7 @@ __device__ __forceinline__ void epi_tighten(const TcParams& p, bool active, int 
 template <int METRIC, int KIND, int MODE, int PAIR>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 knn_tc_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_x, TcParams p) {
-  static_assert(!PAIR || KIND == 1, "CTA pairs stream the bf16 shadow");
+  static_assert(!PAIR || KIND >= 1, "CTA pairs stream a shadow");
   constexpr int STAGES = PAIR ? TC2_STAGES : TC_STAGES;
   constexpr uint32_t B_BYTES = PAIR ? TC2_B_BYTES : TC_B_BYTES;
   constexpr uint32_t STAGE_BYTES = TC_A_BYTES + B_BYTES;
@@ -775,7 +921,7 @@ knn_tc_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
           for (int kb = 0; kb < p.n_kblocks; ++kb) {
             mbar_wait_backoff(&empty_bar[stage], phase ^ 1, p.sleep_ns);
             unsigned char* a_dst = tiles + stage * STAGE_BYTES;
-            constexpr int kElemsPerBlock = KIND == 0 ? TC_BK : 2 * TC_BK;
+            constexpr int kElemsPerBlock = KIND == 0 ? TC_BK : (KIND == 1 ? 2 * TC_BK : 4 * TC_BK);
             // tiled shadow: one contiguous block of 256 (PAIR: this CTA's 128) rows x 128 B
             const int line = kb < p.n_kb_data ? (t * p.n_kb_data + kb) * TC_BN : p.aug_line0 + t * TC_BN;
             if (PAIR) {
@@ -810,7 +956,8 @@ knn_tc_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
     // under `if (lane == 0)` the compiler wraps every MMA in a register-broadcast loop), one elected lane issues.
     {
       constexpr uint32_t idesc = KIND == 0 ? make_idesc_tf32(TC_BM, TC_BN)
-                                           : make_idesc_bf16(PAIR ? 2 * TC_BM : TC_BM, TC_BN);
+                                           : KIND == 1 ? make_idesc_bf16(PAIR ? 2 * TC_BM : TC_BM, TC_BN)
+                                                       : make_idesc_i8(PAIR ? 2 * TC_BM : TC_BM, TC_BN);
       const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
       const uint64_t desc0 = make_smem_desc(0);
       const uint32_t tiles_lo = smem_u32(tiles) >> 4;
@@ -831,7 +978,14 @@ knn_tc_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
             const int nk = kb < n_kb_data - 1 ? TC_BK / TC_UMMA_K : (kb == n_kb_data - 1 ? nk_last : 1);
             if (elect_one()) {
               // advance 32 B along K inside the 128 B swizzle row: +2 in the (>>4) address field
-              if (PAIR) {
+              if (PAIR && KIND == 2) {
+                umma_i8_pair(d_tmem, a_desc, b_desc, idesc, kb != 0 ? 1u : 0u);
+                if (nk > 1) umma_i8_pair(d_tmem, a_desc + 2, b_desc + 2, idesc, 1u);
+                if (nk > 2) umma_i8_pair(d_tmem, a_desc + 4, b_desc + 4, idesc, 1u);
+                if (nk > 3) umma_i8_pair(d_tmem, a_desc + 6, b_desc + 6, idesc, 1u);
+                umma_commit_pair(&empty_bar[stage]);
+                if (kb == n_kb - 1) umma_commit_pair(&tmem_full[acc]);
+              } else if (PAIR) {
                 umma_bf16_pair(d_tmem, a_desc, b_desc, idesc, kb != 0 ? 1u : 0u);
                 if (nk > 1) umma_bf16_pair(d_tmem, a_desc + 2, b_desc + 2, idesc, 1u);
                 if (nk > 2) umma_bf16_pair(d_tmem, a_desc + 4, b_desc + 4, idesc, 1u);
@@ -844,11 +998,16 @@ knn_tc_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
                   if (nk > 1) umma_tf32(d_tmem, a_desc + 2, b_desc + 2, idesc, 1u);
                   if (nk > 2) umma_tf32(d_tmem, a_desc + 4, b_desc + 4, idesc, 1u);
                   if (nk > 3) umma_tf32(d_tmem, a_desc + 6, b_desc + 6, idesc, 1u);
-                } else {
+                } else if (KIND == 1) {
                   umma_bf16(d_tmem, a_desc, b_desc, idesc, kb != 0 ? 1u : 0u);
                   if (nk > 1) umma_bf16(d_tmem, a_desc + 2, b_desc + 2, idesc, 1u);
                   if (nk > 2) umma_bf16(d_tmem, a_desc + 4, b_desc + 4, idesc, 1u);
                   if (nk > 3) umma_bf16(d_tmem, a_desc + 6, b_desc + 6, idesc, 1u);
+                } else {
+                  umma_i8(d_tmem, a_desc, b_desc, idesc, kb != 0 ? 1u : 0u);
+                  if (nk > 1) umma_i8(d_tmem, a_desc + 2, b_desc + 2, idesc, 1u);
+                  if (nk > 2) umma_i8(d_tmem, a_desc + 4, b_desc + 4, idesc, 1u);
+                  if (nk > 3) umma_i8(d_tmem, a_desc + 6, b_desc + 6, idesc, 1u);
                 }
                 umma_commit(&empty_bar[stage]);                       // frees the smem stage once these MMAs retire
                 if (kb == n_kb - 1) umma_commit(&tmem_full[acc]);     // accumulator ready for the epilogue
@@ -890,6 +1049,8 @@ knn_tc_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
       // (hundreds of cycles) never sits on the critical path of the first compare
       const bool poll = active && !p.fixed;
       uint32_t tg_next = poll ? ld_relaxed_u32(p.tau_g + q) : ORD_NEG_INF;
+      float4 qs = make_float4(1.f, 0.f, 0.f, 0.f);   // kind 2: (S_q, a_q, e_q) of this lane's query
+      if (KIND == 2) { if (active) qs = p.i8_q[q]; }
 
       for (int tv = t0; tv < t1; ++tv) {
         const int t = tv * p.tile_stride;
@@ -897,6 +1058,8 @@ knn_tc_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
           tau = fmaxf(tau, ord2f(tg_next));
           tg_next = ld_relaxed_u32(p.tau_g + q);
         }
+        float2 ts = make_float2(1.f, 0.f);            // kind 2: (S_t, E_t) of this tile
+        if (KIND == 2) ts = __ldg(p.i8_tile + t);
         mbar_wait(&tmem_full[acc], acc_phase);
         if (METRIC != 2) mbar_wait(&norm_full[acc], acc_phase);
         tc_fence_after();
@@ -907,8 +1070,16 @@ knn_tc_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
         if (MODE == 1) { if (u == 0 && tv == t0) dbg_row = p.dbg + (int(lane) * 4 + lane_grp) * TC_BN + half * TC_HALF_COLS; }
         float* pre_out = nullptr;
         if (MODE == 2) { if (active) pre_out = p.pre_max + size_t(q) * p.pre_pitch + (tv * TC_SPLIT + half); }
-        epi_tile<METRIC, MODE, PAIR>(t_lane + uint32_t(acc * TC_BN), any_active ? ncols : 0, nrm, col0, tau, buf, wn,
-                                     &tmem_empty[acc], tmem_empty_leader + uint32_t(acc) * 8u, &norm_empty[acc], lane, dbg_row, pre_out);
+        if (KIND == 2) {
+          const double ss = double(ts.x) * double(qs.x);
+          const double ae = fma(double(qs.y), double(ts.y), double(qs.z)) + 0x1p-48;   // a_q E_t + e_q (+ rounding pad)
+          epi_tile_i8<METRIC, MODE, PAIR>(t_lane + uint32_t(acc * TC_BN), any_active ? ncols : 0, nrm, col0, tau,
+                                          i8_threshold(tau, ss, ae), 1.0 / ss, ae, buf, wn, &tmem_empty[acc],
+                                          tmem_empty_leader + uint32_t(acc) * 8u, &norm_empty[acc], lane, dbg_row, pre_out);
+        } else {
+          epi_tile<METRIC, MODE, PAIR>(t_lane + uint32_t(acc * TC_BN), any_active ? ncols : 0, nrm, col0, tau, buf, wn,
+                                       &tmem_empty[acc], tmem_empty_leader + uint32_t(acc) * 8u, &norm_empty[acc], lane, dbg_row, pre_out);
+        }
         if (++acc == TC_ACC_STAGES) { acc = 0; acc_phase ^= 1; }
         if (MODE != 2) epi_tighten(p, active, q, buf, wn, wn_trig, tau, lane);
       }
@@ -1194,6 +1365,48 @@ __global__ void knn_prep_kernel(const float* __restrict__ Q, int n_q, int n_rows
   }
 }
 
+// Quantised queries of the int8 filter (kind 2, format above i8_scale): one warp per row of the padded int8 query matrix
+// (tile order, as knn_prep_kernel; pitch8 bytes per row, zeros past the data and in pad rows), and (S_q, a_q, e_q) per
+// query. A zero query quantises to zeros with a_q = e_q = 0.
+__global__ void __launch_bounds__(256)
+knn_qprep_i8_kernel(const float* __restrict__ Q, int n_q, int n_rows_p, int dim, int pitch8, int8_t* __restrict__ Q8,
+                    float4* __restrict__ qstat) {
+  const int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+  if (row >= n_rows_p) return;
+  const int j = row % TC_BM;
+  const int q = row - j + (j % 32) * 4 + j / 32;
+  int8_t* out = Q8 + size_t(row) * pitch8;
+  if (q >= n_q) {
+    for (int d = lane; d < pitch8; d += 32) out[d] = 0;
+    return;
+  }
+  const float* qv = Q + size_t(q) * dim;
+  double s = 0.0; float mx = 0.f;
+  for (int d = lane; d < dim; d += 32) { const float v = qv[d]; s = fma(double(v), double(v), s); mx = fmaxf(mx, fabsf(v)); }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) { s += __shfl_xor_sync(0xffffffffu, s, o); mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o)); }
+  const double nq = sqrt(s), inv = 1.0 / (nq > 1e-12 ? nq : 1e-12);
+  const float scale = i8_scale(double(mx) * inv);
+  const double inv_s = 1.0 / double(scale);
+  double rr = 0.0, qq = 0.0;   // |q^ - q~/S|^2, |q~|^2
+  for (int d = lane; d < pitch8; d += 32) {
+    int v = 0;
+    if (d < dim) {
+      const double h = double(qv[d]) * inv;
+      v = i8_quant(h, scale);
+      const double r = h - double(v) * inv_s;
+      rr = fma(r, r, rr); qq += double(v * v);
+    }
+    out[d] = int8_t(v);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) { rr += __shfl_xor_sync(0xffffffffu, rr, o); qq += __shfl_xor_sync(0xffffffffu, qq, o); }
+  if (lane == 0) {
+    const double pad = 1.0 + 0x1p-40;   // the fp64 sums' rounding
+    qstat[q] = make_float4(scale, __double2float_ru(sqrt(qq) * inv_s * pad), __double2float_ru(sqrt(rr) * pad), 0.f);
+  }
+}
+
 // ---------------------------------------------------------------------------------------------
 // finish: select K' by approximate score, exact rerank, sort, certificate
 // ---------------------------------------------------------------------------------------------
@@ -1206,6 +1419,7 @@ struct FinishParams {
   int* flags; int certify; float max_norm; double c_err; double c_add;
   int64_t* out_rows; float* out_dist;
   int* n_flagged;   // counts the queries this launch flags (read back by the host together with the results)
+  int unit_q;       // 1: scores are cosine upper bounds of the NORMALISED query (int8 filter), not scaled by |q|
 };
 
 // One CTA per query. The query's candidates live in 2 * n_slices buffers (one per unit-half).
@@ -1436,7 +1650,7 @@ knn_tc_finish_kernel(FinishParams p) {
     if (p.certify) {
       // every row that is not a candidate has approximate score <= T
       const float t_score = ord2f(pivot);
-      const double nq = sqrt(qq);
+      const double nq = p.unit_q ? 1.0 : sqrt(qq);
       const double xm = double(p.max_norm);
       double e_abs, lb;
       if (p.metric == 0) {
@@ -1509,7 +1723,7 @@ knn_tc_tau0_kernel(const float* __restrict__ pre_max, int n_q, int n_rec, int m,
 __global__ void __launch_bounds__(128)
 refine_prep_kernel(const float* __restrict__ Q, const int* __restrict__ qlist, int dim, int metric, int k,
                    const float* __restrict__ dist, float max_norm, double c_err, double c_add,
-                   float* __restrict__ Qr, uint32_t* __restrict__ tau_fixed) {
+                   float* __restrict__ Qr, uint32_t* __restrict__ tau_fixed, int unit_q) {
   __shared__ double part[4];
   const int i = blockIdx.x, q = qlist[i];
   double s = 0.0;
@@ -1524,7 +1738,7 @@ refine_prep_kernel(const float* __restrict__ Q, const int* __restrict__ qlist, i
   __syncthreads();
   if (threadIdx.x == 0) {
     const double qq = part[0] + part[1] + part[2] + part[3];
-    const double nq = sqrt(qq), xm = double(max_norm);
+    const double nq = unit_q ? 1.0 : sqrt(qq), xm = double(max_norm);   // unit_q: see FinishParams
     double dk = double(dist[size_t(q) * k + (k - 1)]);
     dk = dk + 1e-6 * fabs(dk) + 1e-37;            // a row at distance <= dk (after fp32 rounding) must survive
     double score, e_abs;
@@ -1562,13 +1776,15 @@ __global__ void refine_scatter_kernel(const int* __restrict__ qlist, const int* 
 
 // Masked search (reference: `data.filter(expr)` before the distance column, index.py:161): fold the row mask
 // into the per-row epilogue term so masked rows can never pass the threshold test:
-//   additive term (L2: -0.5|x|^2, IP: 0) -> -inf;  multiplicative term (cosine 1/|x|) -> NaN (NaN > tau is false)
+//   additive term (L2: -0.5|x|^2, IP: 0) -> -inf;  multiplicative term (cosine 1/|x|) -> NaN (NaN > tau is false);
+//   the int8 filter's integer row term (mode 3): 0 -> I8_MASKED, below every integer threshold (i8_threshold)
 __global__ void masked_norms_kernel(const uint8_t* __restrict__ mask, const float* __restrict__ base, int64_t n_rows,
-                                    int64_t n_alloc, int mode /*0 add-from-base, 1 mul-from-base, 2 add-zero*/,
+                                    int64_t n_alloc, int mode /*0 add-from-base, 1 mul-from-base, 2 add-zero, 3 int8 term*/,
                                     float* __restrict__ out) {
   for (int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; i < n_alloc; i += int64_t(gridDim.x) * blockDim.x) {
     float v;
     if (i >= n_rows) v = 0.f;
+    else if (mode == 3) v = __int_as_float(mask[i] ? 0 : I8_MASKED);
     else if (mask[i]) v = mode == 2 ? 0.f : base[i];
     else v = mode == 1 ? __int_as_float(0x7fc00000) : -INFINITY;
     out[i] = v;
@@ -1631,6 +1847,79 @@ __global__ void to_bf16_tiled_kernel(const float* __restrict__ X, int64_t n_rows
   }
 }
 
+// fp32 rows -> int8 normalised shadow (format above i8_scale) in the bf16 shadows' streaming layout with 128 columns per
+// k-block: element (r, d) at ((tile * n_kb + kb) * 256 + r % 256) * 128 + d % 128. One CTA (8 warps, 32 rows each) per
+// tile: pass 1 finds the tile's largest |x^_i| (fp64 row norms, the rerank's definition of x^), pass 2 quantises and takes
+// the largest residual norm. Pad rows and columns are zero. tile[t] = (S_t, E_t).
+__global__ void __launch_bounds__(256)
+to_i8_tiled_kernel(const float* __restrict__ X, int64_t n_rows, int pitch, int dim, int n_kb, int64_t n_tiles,
+                   int8_t* __restrict__ X8, float2* __restrict__ tile) {
+  __shared__ double s_inv[TC_BN];
+  __shared__ double s_max[8], s_err[8];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int64_t t = blockIdx.x; t < n_tiles; t += gridDim.x) {
+    double wmax = 0.0;
+    for (int rr = warp * 32; rr < warp * 32 + 32; ++rr) {
+      const int64_t r = t * TC_BN + rr;
+      double s = 0.0; float mx = 0.f;
+      if (r < n_rows) {
+        const float4* xp = reinterpret_cast<const float4*>(X + size_t(r) * pitch);
+        for (int j = lane; j < (pitch >> 2); j += 32) {
+          const float4 v = __ldg(xp + j);
+          s = fma(double(v.x), double(v.x), s); s = fma(double(v.y), double(v.y), s);
+          s = fma(double(v.z), double(v.z), s); s = fma(double(v.w), double(v.w), s);
+          mx = fmaxf(fmaxf(mx, fmaxf(fabsf(v.x), fabsf(v.y))), fmaxf(fabsf(v.z), fabsf(v.w)));
+        }
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) { s += __shfl_xor_sync(0xffffffffu, s, o); mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o)); }
+      const double n = sqrt(s), inv = 1.0 / (n > 1e-12 ? n : 1e-12);
+      if (lane == 0) s_inv[rr] = inv;
+      wmax = fmax(wmax, double(mx) * inv);
+    }
+    if (lane == 0) s_max[warp] = wmax;
+    __syncthreads();
+    double tmax = 0.0;
+    for (int w = 0; w < 8; ++w) tmax = fmax(tmax, s_max[w]);
+    const float scale = i8_scale(tmax);
+    double werr = 0.0;
+    for (int rr = warp * 32; rr < warp * 32 + 32; ++rr) {
+      const int64_t r = t * TC_BN + rr;
+      const bool live = r < n_rows;
+      const double inv = s_inv[rr], inv_s = 1.0 / double(scale);
+      double e2 = 0.0;
+      for (int kb = 0; kb < n_kb; ++kb) {
+        const int d0 = kb * I8_KB + 4 * lane;   // four columns per lane: one 128-byte line per warp and k-block
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (live && d0 < pitch) v = __ldg(reinterpret_cast<const float4*>(X + size_t(r) * pitch + d0));
+        const float f[4] = {v.x, v.y, v.z, v.w};
+        char4 o;
+        int qv[4];
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+          const double h = double(f[e]) * inv;
+          qv[e] = (d0 + e < dim) ? i8_quant(h, scale) : 0;
+          const double res = h - double(qv[e]) * inv_s;
+          e2 = fma(res, res, e2);
+        }
+        o.x = char(qv[0]); o.y = char(qv[1]); o.z = char(qv[2]); o.w = char(qv[3]);
+        reinterpret_cast<char4*>(X8 + ((size_t(t) * n_kb + kb) * TC_BN + rr) * I8_KB)[lane] = o;
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) e2 += __shfl_xor_sync(0xffffffffu, e2, o);
+      werr = fmax(werr, e2);
+    }
+    if (lane == 0) s_err[warp] = werr;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      double e2 = 0.0;
+      for (int w = 0; w < 8; ++w) e2 = fmax(e2, s_err[w]);
+      tile[t] = make_float2(scale, __double2float_ru(sqrt(e2) * (1.0 + 0x1p-40)));
+    }
+    __syncthreads();
+  }
+}
+
 // ---------------------------------------------------------------------------------------------
 // host glue
 // ---------------------------------------------------------------------------------------------
@@ -1639,13 +1928,16 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
 inline bool tc_encode_2d(const TcState* st, CUtensorMap* map, const void* base, uint64_t inner, uint64_t outer,
-                         uint64_t pitch_elems, uint32_t box_inner, uint32_t box_outer, std::string* err, bool bf16 = false) {
+                         uint64_t pitch_elems, uint32_t box_inner, uint32_t box_outer, std::string* err, int esize = 4) {
+  // esize: bytes per element - 4 fp32, 2 bf16, 1 int8 (moved as raw bytes)
   cuuint64_t dims[2] = {inner, outer};
-  cuuint64_t strides[1] = {pitch_elems * (bf16 ? 2 : sizeof(float))};
+  cuuint64_t strides[1] = {pitch_elems * uint64_t(esize)};
+  const CUtensorMapDataType dt = esize == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32
+                                 : (esize == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_UINT8);
   cuuint32_t box[2] = {box_inner, box_outer};
   cuuint32_t estr[2] = {1, 1};
   CUresult r = reinterpret_cast<EncodeTiledFn>(st->encode)(
-      map, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(base), dims, strides, box, estr,
+      map, dt, 2, const_cast<void*>(base), dims, strides, box, estr,
       CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
       CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
@@ -1679,6 +1971,10 @@ inline bool tc_init(TcState* st, int sm_count, std::string* err) {
   attr(knn_tc_filter_kernel<2, 1, 0, 1>, TC2_SMEM_BYTES);
   attr(knn_tc_filter_kernel<0, 1, 2, 1>, TC2_SMEM_BYTES); attr(knn_tc_filter_kernel<1, 1, 2, 1>, TC2_SMEM_BYTES);
   attr(knn_tc_filter_kernel<2, 1, 2, 1>, TC2_SMEM_BYTES);
+  attr(knn_tc_filter_kernel<0, 2, 0, 0>, TC_SMEM_BYTES); attr(knn_tc_filter_kernel<2, 2, 0, 0>, TC_SMEM_BYTES);
+  attr(knn_tc_filter_kernel<2, 2, 2, 0>, TC_SMEM_BYTES);
+  attr(knn_tc_filter_kernel<0, 2, 0, 1>, TC2_SMEM_BYTES); attr(knn_tc_filter_kernel<2, 2, 0, 1>, TC2_SMEM_BYTES);
+  attr(knn_tc_filter_kernel<2, 2, 2, 1>, TC2_SMEM_BYTES);
   if (a == cudaSuccess) a = cudaFuncSetAttribute(knn_rq_filter_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, RQ_SMEM_MAX);
   if (a == cudaSuccess) a = cudaFuncSetAttribute(knn_rq_filter_kernel<0, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, RQ_SMEM_MAX);
   if (a == cudaSuccess) a = cudaFuncSetAttribute(knn_rq_filter_kernel<2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, RQ_SMEM_MAX);
@@ -1688,13 +1984,14 @@ inline bool tc_init(TcState* st, int sm_count, std::string* err) {
   return true;
 }
 
-// tiled shadow: a flat list of 128-byte lines, 256 lines per (tile, k-block)
+// tiled shadow: a flat list of 128-byte lines, 256 lines per (tile, k-block); esize: 2 bf16, 1 int8
 inline bool tc_bind_shadow(const TcState* st, CUtensorMap* map, CUtensorMap* map_half, const void* Xb, int64_t n_rows,
-                           int blocks_per_tile, std::string* err) {
+                           int blocks_per_tile, std::string* err, int esize = 2) {
   const uint64_t lines = uint64_t((n_rows + TC_BN - 1) / TC_BN) * uint64_t(blocks_per_tile) * TC_BN;
-  if (lines >= (uint64_t(1) << 31)) { *err = "shard too large for the tiled bf16 shadow (32-bit TMA coordinates)"; return false; }
-  if (!tc_encode_2d(st, map_half, Xb, uint64_t(2 * TC_BK), lines, uint64_t(2 * TC_BK), 2 * TC_BK, TC_BN / 2, err, true)) return false;
-  return tc_encode_2d(st, map, Xb, uint64_t(2 * TC_BK), lines, uint64_t(2 * TC_BK), 2 * TC_BK, TC_BN, err, true);
+  if (lines >= (uint64_t(1) << 31)) { *err = "shard too large for a tiled shadow (32-bit TMA coordinates)"; return false; }
+  const uint32_t line = 128 / esize;   // elements per 128-byte line
+  if (!tc_encode_2d(st, map_half, Xb, line, lines, line, line, TC_BN / 2, err, esize)) return false;
+  return tc_encode_2d(st, map, Xb, line, lines, line, line, TC_BN, err, esize);
 }
 
 inline bool tc_bind_corpus(TcState* st, TcCorpus* tc, const float* X, int64_t n_rows, int dim, int pitch,
@@ -1712,9 +2009,12 @@ inline bool tc_bind_corpus(TcState* st, TcCorpus* tc, const float* X, int64_t n_
 }
 
 // K' (candidates kept by each selection) and the buffer capacity that goes with it
+constexpr int TC_KP_I8 = 256;   // int8 filter, k <= 16: rows above the k-th exact cosine that the bound lets through (K' sweep)
 inline int tc_kp(int k, bool certify, int kind = 0) {
   // slack so that the certificate holds for (nearly) every query in one pass: the bf16 bound is ~1.8x looser than
-  // the TF32 one (measured on C3: K' = 32 flags 25 of 4096 queries per batch with bf16, K' = 64 none)
+  // the TF32 one (measured on C3: K' = 32 flags 25 of 4096 queries per batch with bf16, K' = 64 none); the int8 bound
+  // (~0.02 in cosine units at D = 768) needs a few hundred rows, see TC_KP_I8
+  if (kind == 2) return certify ? std::max(TC_KP_I8, (k + k / 2 + 31) & ~31) : ((k + 31) & ~31);
   int kp = certify ? k + std::max(kind == 1 ? 48 : 16, k / 2) : k;
   return (kp + 31) & ~31;
 }
@@ -1739,6 +2039,8 @@ struct TcPlan {
   int n_qt_lists;// query tiles the candidate-list layout is indexed with (2 n_qp for the pair kernel, else n_qt)
   int n_qp;      // query pairs
   int kp_list;   // candidates each (query, list) keeps at a selection (<= kp)
+  int kb_bf16;   // the row width in bf16 k-blocks (64 columns; the plain shadow's augmented block counted), whatever the
+                 // operand kind: what the CTA-pair and sample-prepass rules were measured against
   size_t off_qp, off_qb, off_tau, off_flags, off_qerr, off_wcnt, off_wbuf, off_pre, total;
   int n_rec, pre_pitch;   // threshold prepass: block-maximum records per query (= row pitch of the record matrix)
 };
@@ -1759,6 +2061,10 @@ inline TcPlan tc_plan(const TcState* st, const TcSearch& s) {
     pl.n_kb_data = (s.pitch + TC_BK - 1) / TC_BK;
     pl.nk_last = (s.pitch - TC_BK * (pl.n_kb_data - 1) + TC_UMMA_K - 1) / TC_UMMA_K;
     pl.n_kblocks = pl.n_kb_data;
+  } else if (s.kind == 2) {
+    pl.n_kb_data = i8_n_kb(s.dim);
+    pl.nk_last = (s.dim - I8_KB * (pl.n_kb_data - 1) + 31) / 32;
+    pl.n_kblocks = pl.n_kb_data;
   } else {
     const ShadowGeom g = shadow_geom(s.dim);
     pl.n_kb_data = g.n_kb_data;
@@ -1769,6 +2075,7 @@ inline TcPlan tc_plan(const TcState* st, const TcSearch& s) {
     pl.aug_col = g.aug_col;
   }
   if (kn.fullk) pl.nk_last = TC_BK / TC_UMMA_K;   // tuning knob: multiply the zero padding too
+  pl.kb_bf16 = s.kind == 2 ? (s.dim + 63) / 64 : pl.n_kblocks;
   // narrow rows and at least two query tiles: the resident-query kernel (operand traffic, not the tensor pipe, binds
   // the streaming kernel there); its tiles are 128 corpus rows, its units pair two query tiles
   pl.rq = (s.kind == 1 && pl.n_kblocks <= RQ_MAX_KB && pl.n_qt >= 2 && s.epi != 1 && s.dbg == nullptr && !kn.no_rq) ? 1 : 0;
@@ -1778,7 +2085,7 @@ inline TcPlan tc_plan(const TcState* st, const TcSearch& s) {
   // (auto: from 7 k-blocks per row on. A tile of D = 384 is 24 MMAs and the pair's cluster-wide hand-offs cost more than
   // the halved B traffic saves - 1452 vs 1541 TFLOP/s at uncapped clocks; from D = 512 the pair wins, 1645 vs 1519 TFLOP/s at
   // D = 768: scripts/ubench/width_sweep.py, profiles/r02_sweep_row_width.txt)
-  pl.pair = (!pl.rq && s.kind == 1 && pl.n_qt >= 2 && s.dbg == nullptr && (kn.pair == 1 || (kn.pair < 0 && pl.n_kblocks >= 7))) ? 1 : 0;
+  pl.pair = (!pl.rq && s.kind >= 1 && pl.n_qt >= 2 && s.dbg == nullptr && (kn.pair == 1 || (kn.pair < 0 && pl.kb_bf16 >= 7))) ? 1 : 0;
   pl.n_qt_lists = pl.pair ? 2 * pl.n_qp : pl.n_qt;
   const int n_tiles_full = pl.rq ? int((s.n_rows + RQ_BN - 1) / RQ_BN) : pl.n_tiles;   // tiles in the kernel's own unit
   pl.tile_stride = pre ? s.sample_stride : 1;
@@ -1842,10 +2149,10 @@ inline TcPlan tc_plan(const TcState* st, const TcSearch& s) {
   take(TC_HDR_BYTES);   // header: word 0 counts the queries the finish kernel flagged (read back with the results)
   const size_t q_rows_p = size_t(pl.n_qp) * 2 * TC_BM;   // queries are stored in whole tile pairs
   pl.off_qp = take(q_rows_p * s.pitch * 4);
-  pl.off_qb = take(s.kind == 1 ? q_rows_p * s.pitch_b * 2 : 0);
+  pl.off_qb = take(s.kind == 1 ? q_rows_p * s.pitch_b * 2 : (s.kind == 2 ? q_rows_p * s.pitch_b : 0));
   pl.off_tau = take(size_t(s.n_q) * 4);
   pl.off_flags = take(size_t(s.n_q) * 4);
-  pl.off_qerr = take(size_t(s.n_q) * 4);
+  pl.off_qerr = take(size_t(s.n_q) * 16);   // per query: the error weight (augmented queries), or (S_q, a_q, e_q) (kind 2)
   pl.n_rec = pl.n_vtiles * (pl.rq ? 1 : TC_SPLIT);
   pl.pre_pitch = pl.n_rec;
   if (pre) {
@@ -1906,7 +2213,7 @@ inline double tc_c_err(int dim, int kind = 0) {
 // so nothing is added on top and the certificate no longer depends on the largest norm of the shard: one 100x-norm
 // outlier (or clustered rows far from the origin) inflates only its own row's score.
 inline void tc_cert_consts(const TcSearch& s, double* c_err, double* c_add) {
-  if (s.kind == 1 && s.aug != 0) { *c_err = 0.0; *c_add = 0.0; return; }
+  if ((s.kind == 1 && s.aug != 0) || s.kind == 2) { *c_err = 0.0; *c_add = 0.0; return; }
   *c_err = tc_c_err(s.dim, s.kind);
   *c_add = tc_c_add(s.dim, false);
 }
@@ -1923,7 +2230,7 @@ inline double tc_c_pair(int dim, int aug) {
 // a refinement pass, one that is too loose more appends - exactness never depends on the sample).
 inline bool tc_prepass_config(const TcState* st, const TcSearch& s, const TcPlan& main_pl, TcSearch* pre) {
   const TcKnobs& kn = st->knobs;
-  if (s.tau_fixed || s.no_prepass || s.sample_stride > 1 || s.kind != 1 || s.dbg != nullptr) return false;
+  if (s.tau_fixed || s.no_prepass || s.sample_stride > 1 || s.kind == 0 || s.dbg != nullptr) return false;
   // Wide rows: small batches are HBM-bound with a lightly loaded tensor pipe, and there the epilogue's hit path and the
   // finish kernel's candidate volume show (C5 batch 64 +18 %, batch 8 +6 %). Large batches are tensor-bound and the
   // sample costs 1/stride of the scan (3 %); on a whole 10M x 768 shard it pays that back and no more (round 1: neutral),
@@ -1931,7 +2238,7 @@ inline bool tc_prepass_config(const TcState* st, const TcSearch& s, const TcPlan
   // list keeps its own 32 best, ~2400 admitted rows per query over 74 lists - stay loose for most of a unit: measured on
   // one 8-GPU shard of C3 the filter kernel takes 6.35 ms without and 5.09 ms with the sample's GLOBAL thresholds
   // (0.76 -> 0.95 of the burst bf16 peak, profiles/r02_sweep_prepass.txt). On by default; FENIX_TC_PRE_WIDE=0 disables.
-  const bool wide = main_pl.n_kblocks > 4;
+  const bool wide = main_pl.kb_bf16 > 4;
   if (wide && main_pl.n_qt > 3 && !kn.pre_wide) return false;
   if (s.epi != 2) return false;                            // a row mask (predicate / IVF cells) of unknown selectivity: the
                                                            // sample says nothing about how many LIVE rows pass a threshold
@@ -1983,7 +2290,9 @@ inline bool tc_run_pass(TcState* st, TcCorpus* tc, const TcSearch& s, const TcPl
   p.tiles_per_slice = pl.tiles_per_slice; p.n_vtiles = pl.n_vtiles; p.tile_stride = pl.tile_stride;
   p.n_kblocks = pl.n_kblocks; p.n_kb_data = pl.n_kb_data; p.nk_last = pl.nk_last;
   p.aug_line0 = pl.aug_line0;
-  p.xb = s.kind == 1 ? static_cast<const unsigned char*>(s.shadow == 1 ? s.Xn : s.Xb) : nullptr;
+  p.xb = s.kind == 1 ? static_cast<const unsigned char*>(s.shadow == 1 ? s.Xn : s.Xb)
+                     : (s.kind == 2 ? static_cast<const unsigned char*>(s.X8) : nullptr);
+  p.i8_tile = s.i8_tile; p.i8_q = reinterpret_cast<const float4*>(base + pl.off_qerr);
   p.pf_tiles = 0;   // off: measured neutral where operands come from L2 (C2, C4) and 1.9x slower where HBM binds (C5)
   if (st->knobs.pf > 0 && p.xb) p.pf_tiles = st->knobs.pf;
   p.kp = pl.kp_list; p.cap = pl.cap;
@@ -2016,6 +2325,17 @@ inline bool tc_run_pass(TcState* st, TcCorpus* tc, const TcSearch& s, const TcPl
       if (epi == 0) launch(knn_rq_filter_kernel<0, 0>, map_h, rq_smem, 1);
       else launch(knn_rq_filter_kernel<2, 0>, map_h, rq_smem, 1);
     }
+  } else if (pl.pair && s.kind == 2) {
+    if (epi == 0) launch(knn_tc_filter_kernel<0, 2, 0, 1>, tc->map_x8_h, TC2_SMEM_BYTES, 2);   // (masked: no prepass)
+    else if (pre) launch(knn_tc_filter_kernel<2, 2, 2, 1>, tc->map_x8_h, TC2_SMEM_BYTES, 2);
+    else launch(knn_tc_filter_kernel<2, 2, 0, 1>, tc->map_x8_h, TC2_SMEM_BYTES, 2);
+  } else if (s.kind == 2) {
+    if (dbg) {
+      cudaFuncSetAttribute(knn_tc_filter_kernel<2, 2, 1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_BYTES);
+      launch(knn_tc_filter_kernel<2, 2, 1, 0>, tc->map_x8, TC_SMEM_BYTES, 1);
+    } else if (epi == 0) launch(knn_tc_filter_kernel<0, 2, 0, 0>, tc->map_x8, TC_SMEM_BYTES, 1);
+    else if (pre) launch(knn_tc_filter_kernel<2, 2, 2, 0>, tc->map_x8, TC_SMEM_BYTES, 1);
+    else launch(knn_tc_filter_kernel<2, 2, 0, 0>, tc->map_x8, TC_SMEM_BYTES, 1);
   } else if (pl.pair) {
     // CTA pairs: each CTA loads 128-row half blocks of the tiled shadow
     const CUtensorMap& map_h = s.shadow == 1 ? tc->map_xn_h : tc->map_xb_h;
@@ -2062,6 +2382,7 @@ inline bool tc_run_pass(TcState* st, TcCorpus* tc, const TcSearch& s, const TcPl
   int sort2 = 2; while (sort2 < pl.kp) sort2 <<= 1;
   f.sort2 = sort2; f.tau_g = tau_g; f.wbuf = wbuf; f.wcnt = wcnt; f.qt_major = pl.qt_major; f.rq = pl.rq; f.n_qp = pl.n_qp; f.flags = flags; f.certify = s.certify ? 1 : 0;
   f.max_norm = s.max_norm; tc_cert_consts(s, &f.c_err, &f.c_add); f.out_rows = s.out_rows; f.out_dist = s.out_dist;
+  f.unit_q = s.kind == 2 ? 1 : 0;
   const size_t fin_smem = size_t(sort2) * 12 + size_t(s.pitch) * 4 + size_t(FIN_POOL) * 8 + 16;
   // many short lists per query (small batches split over all SMs): more warps sweep them in parallel
   // few lists, many candidates to rerank (K' >= 128: k = 100): 128-thread CTAs - more of them per SM cover the scattered
@@ -2086,9 +2407,12 @@ inline bool tc_search(TcState* st, TcCorpus* tc, const TcSearch& s, const TcLaun
   CUtensorMap map_q;
   if (s.kind == 0) {
     if (!tc_encode_2d(st, &map_q, qp, uint64_t(s.pitch), uint64_t(pl.n_qp) * 2 * TC_BM, uint64_t(s.pitch), TC_BK, TC_BM, err)) return false;
+  } else if (s.kind == 2) {
+    if (!tc->ok_8) { *err = "int8 filter requested but the shard has no int8 shadow"; return false; }
+    if (!tc_encode_2d(st, &map_q, base + pl.off_qb, uint64_t(s.pitch_b), uint64_t(pl.n_qp) * 2 * TC_BM, uint64_t(s.pitch_b), I8_KB, TC_BM, err, 1)) return false;
   } else {
     if (s.shadow == 1 ? !tc->ok_n : !tc->ok_b) { *err = "bf16 filter requested but the shard has no bf16 shadow"; return false; }
-    if (!tc_encode_2d(st, &map_q, qb, uint64_t(s.pitch_b), uint64_t(pl.n_qp) * 2 * TC_BM, uint64_t(s.pitch_b), 2 * TC_BK, TC_BM, err, true)) return false;
+    if (!tc_encode_2d(st, &map_q, qb, uint64_t(s.pitch_b), uint64_t(pl.n_qp) * 2 * TC_BM, uint64_t(s.pitch_b), 2 * TC_BK, TC_BM, err, 2)) return false;
   }
 
   const int n_rows_p = pl.n_qp * 2 * TC_BM;
@@ -2103,6 +2427,11 @@ inline bool tc_search(TcState* st, TcCorpus* tc, const TcSearch& s, const TcLaun
   knn_prep_kernel<<<std::max(prep_blocks, 1), 256, 0, s.stream>>>(s.Q, s.n_q, n_rows_p, s.dim, s.pitch, qp, tau_g, flags, qb, s.pitch_b, s.tau_fixed,
                                                                   (!s.tau_fixed && st->knobs.warm) ? 1 : 0,
                                                                   aug ? pl.aug_col : 0, reinterpret_cast<int*>(base), s.aug, qerr);
+  if (s.kind == 2) {
+    knn_qprep_i8_kernel<<<(n_rows_p + 7) / 8, 256, 0, s.stream>>>(s.Q, s.n_q, n_rows_p, s.dim, s.pitch_b,
+                                                                 reinterpret_cast<int8_t*>(base + pl.off_qb), reinterpret_cast<float4*>(qerr));
+    *launched += 1;
+  }
   // threshold prepass over a strided sample (the padded queries and tau_g sit at the same scratch offsets in both plans)
   if (variant) *variant = (pl.rq ? 1 : 0) | (L.with_pre ? 2 : 0) | (pl.pair ? 4 : 0);
   if (L.with_pre) {

@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define FX_ABI_VERSION 3
+#define FX_ABI_VERSION 4
 
 /* error codes */
 #define FX_OK 0
@@ -87,11 +87,13 @@ typedef struct fx_stats {
   int64_t kernel_launches;   /* kernels of this library launched so far */
   double last_search_ms;     /* device time of the last search (CUDA events) */
   double last_main_kernel_ms;/* device time of the dominant kernel of the last search */
-  int32_t last_path;         /* 0 = exact scan, 1 = tcgen05 TF32 filter + rerank, 2 = tcgen05 bf16 filter + rerank,
+  int32_t last_path;         /* 0 = exact scan, 1 = tcgen05 TF32 filter + rerank, 2 = tcgen05 shadow filter (bf16 or int8) + rerank,
                               * 3 = direct scan: one launch, fp64 distances of every row (<= 8 queries over a small shard) */
   int32_t last_variant;      /* tcgen05 paths: bit 0 = resident-query kernel (narrow rows; else the streaming kernel),
                               * bit 1 = thresholds seeded by the sample prepass, bit 2 = CTA-pair (cta_group::2) streaming kernel */
   double last_exchange_ms;   /* sharded searches: device time of all-gather + merge of the last search (CUDA events) */
+  int32_t last_operand;      /* operand of the last search's filter: 0 = fp32 / TF32 (or no filter), 1 = bf16 shadow,
+                              * 2 = int8 normalised shadow (exact cosine at small k) */
 } fx_stats;
 
 /* ---- lifetime -------------------------------------------------------------------------- */
