@@ -167,6 +167,12 @@ struct fx_corpus {
   int64_t n_inv = 0, n_cells = 0;
 };
 
+// variant of fx::tc_search (bit 3: resident query tiles) -> fx_stats
+static void set_variant(fx_corpus* c, int variant) {
+  c->stats.last_variant = variant & 7;
+  c->stats.last_resident_queries = (variant >> 3) & 1;
+}
+
 static int bind(fx_ctx* ctx) {
   FX_CUDA(cudaSetDevice(ctx->device));
   return FX_OK;
@@ -839,7 +845,7 @@ static int search_enqueue(fx_corpus* c, const float* d_q, int64_t n_q, int metri
     int launched = 0, variant = 0;
     if (!fx::tc_search(&ctx->tc, &c->tc, s, run->L, ctx->d_tc.p, &launched, &err, &variant)) return fail(FX_ECUDA, "fx_search: %s", err.c_str());
     run->tc = true; run->path = kind == 0 ? 1 : 2; run->operand = kind;
-    c->stats.last_variant = variant;
+    set_variant(c, variant);
     ctx->launches += launched; c->stats.kernel_launches += launched;
     if (s.certify) FX_CUDA(cudaMemcpyAsync(ctx->h_word, fx::tc_flag_count(ctx->d_tc.p), sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
   } else {
@@ -1071,7 +1077,7 @@ static bool graph_capture(fx_corpus* c, fx_corpus::GraphEntry* g, int64_t n_q, i
   g->exec = exec; g->state = 1; g->knob_epoch = ctx->knob_epoch;
   const void* now[7] = {ctx->d_q.p, ctx->d_rows.p, ctx->d_dist.p, ctx->d_tc.p, ctx->h_q.p, ctx->h_rows.p, ctx->h_dist.p};
   for (int i = 0; i < 7; ++i) g->ptrs[i] = const_cast<void*>(now[i]);
-  g->path = run->path; g->operand = run->operand; g->variant = c->stats.last_variant; g->launches = int(c->stats.kernel_launches - launches0);
+  g->path = run->path; g->operand = run->operand; g->variant = c->stats.last_variant | (c->stats.last_resident_queries << 3); g->launches = int(c->stats.kernel_launches - launches0);
   c->stats.kernel_launches = launches0;   // counted when the graph runs
   return true;
 }
@@ -1163,7 +1169,7 @@ extern "C" int fx_search(fx_corpus* c, const float* queries, int64_t n_q, int32_
       ctx->h_word[0] = 0;
       FX_CUDA(cudaGraphLaunch(g->exec, ctx->stream));
       run.tc = true; run.path = g->path; run.operand = g->operand; run.n_q = n_q;
-      c->stats.last_variant = g->variant;
+      set_variant(c, g->variant);
       ctx->launches += g->launches; c->stats.kernel_launches += g->launches;
       launched = true;
     } else if (g->state == 2) {

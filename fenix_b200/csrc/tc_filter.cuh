@@ -8,6 +8,7 @@
 //                                                      on the raw rows, fp32 accumulators in TMEM, double-buffered)
 //                            warp 2     TMEM allocator
 //                            warps 4-11 epilogue      (epi_tile / epi_tighten below)
+//                          PAIR 1: CTA pairs (cta_group::2); PAIR 2: the same over the int8 shadow with the query tiles resident
 //   knn_rq_filter_kernel   resident-query kernel (narrow rows, >= 2 query tiles): two query tiles stay in shared memory,
 //                          128-row corpus blocks stream through a deep ring and feed two MMAs each (warps 1 and 3 issue)
 //   MODE 2 of both + knn_tc_tau0_kernel   threshold prepass over a strided sample (narrow rows)
@@ -62,6 +63,21 @@ constexpr uint32_t TC2_B_BYTES = TC_B_BYTES / 2;
 constexpr uint32_t TC2_STAGE_BYTES = TC_A_BYTES + TC2_B_BYTES;
 constexpr uint32_t TC2_SMEM_BYTES = 1024 /*align slack*/ + TC2_STAGES * TC2_STAGE_BYTES +
                                     TC_ACC_STAGES * TC_NORM_BYTES + 512 /*barriers*/;
+// Resident-query CTA-pair kernel (int8 shadow): each CTA keeps its whole query tile (n_kblocks blocks of 16 KB) for a
+// unit, and the ring carries only corpus half blocks (16 KB); the ring gets whatever shared memory the query tile leaves.
+constexpr int TC3_MAX_STAGES = 12;
+constexpr uint32_t TC3_SMEM_MAX = 227 * 1024;
+constexpr uint32_t TC3_FIXED_BYTES = 1024 /*align slack*/ + TC_ACC_STAGES * TC_NORM_BYTES + 512 /*barriers*/;
+constexpr int TC3_MIN_STAGES = 4;
+inline int tc3_stages(int n_kblocks) {
+  const int s = (int(TC3_SMEM_MAX) - int(TC3_FIXED_BYTES) - n_kblocks * int(TC_A_BYTES)) / int(TC2_B_BYTES);
+  return s < TC3_MAX_STAGES ? s : TC3_MAX_STAGES;
+}
+inline uint32_t tc3_smem_bytes(int n_kblocks) {
+  return TC3_FIXED_BYTES + uint32_t(n_kblocks) * TC_A_BYTES + uint32_t(tc3_stages(n_kblocks)) * TC2_B_BYTES;
+}
+static_assert(TC3_FIXED_BYTES + 6 * TC_A_BYTES + 7 * TC2_B_BYTES <= TC3_SMEM_MAX, "D = 768 (6 int8 k-blocks): 7 corpus stages");
+static_assert(TC3_FIXED_BYTES + 9 * TC_A_BYTES + TC3_MIN_STAGES * TC2_B_BYTES <= TC3_SMEM_MAX, "D <= 1152: 4 corpus stages");
 constexpr size_t TC_HDR_BYTES = 256;        // scratch header (word 0: flagged-query counter of the last finish launch)
 constexpr int TC_MAX_WAVES = 4;            // units per CTA at most (bounds the candidate-buffer scratch)
 constexpr uint32_t ORD_NEG_INF = 0x007fffffu;  // f2ord(-inf)
@@ -154,6 +170,8 @@ struct TcKnobs {
   int debug_direct = 0;    // FENIX_DEBUG_DIRECT   stderr timeline (globaltimer stamps) of every direct scan launched by fx_search
   int int8 = -1;           // FENIX_INT8           exact cosine filters with int8 MMAs over the int8 normalised shadow: -1 auto (rows
                            //                      wider than 192 columns, k <= 16), 0 never, 1 whenever the metric and precision allow
+  int resident = -1;       // FENIX_TC_RESIDENT    int8 CTA-pair kernel with the query tiles resident in shared memory: -1 auto (wherever
+                           //                      the CTA-pair kernel runs and the tile fits), 0 never, 1 whenever it fits
 };
 // name = the environment variable's name; value = its text, or null to restore the default. False: unknown name.
 inline bool tc_set_knob(TcKnobs* k, const char* name, const char* value) {
@@ -193,6 +211,7 @@ inline bool tc_set_knob(TcKnobs* k, const char* name, const char* value) {
   else if (n == "FENIX_DIRECT_QREG") k->direct_qreg = as_int(d.direct_qreg);
   else if (n == "FENIX_MERGE_RANK_MIN") k->merge_rank_min = as_int(d.merge_rank_min);
   else if (n == "FENIX_INT8") k->int8 = as_int(d.int8);
+  else if (n == "FENIX_TC_RESIDENT") k->resident = as_int(d.resident);
   else return false;
   return true;
 }
@@ -201,7 +220,7 @@ inline void tc_knobs_from_env(TcKnobs* k) {
       "FENIX_TC_KP", "FENIX_TC_FULLK", "FENIX_TC_NO_RQ", "FENIX_TC_SLICES", "FENIX_TC_MAX_WAVES", "FENIX_TC_ORDER", "FENIX_TC_KP_LIST",
       "FENIX_TC_PRE_WIDE", "FENIX_TC_PRE", "FENIX_TC_PRE_SMALL", "FENIX_TC_PRE_SAFETY", "FENIX_TC_PRE_M", "FENIX_TC_PF", "FENIX_RQ_STAGES",
       "FENIX_FIN_THREADS", "FENIX_TC_WARM", "FENIX_TC_PAIR", "FENIX_TC_ERRCOL", "FENIX_FP32_FILTER_TF32", "FENIX_NO_REFINE",
-      "FENIX_NO_NORM_SHADOW", "FENIX_DEBUG_BF16", "FENIX_DEBUG_TIERS", "FENIX_GRAPH", "FENIX_DIRECT", "FENIX_DIRECT_MAX_MB", "FENIX_DEBUG_DIRECT", "FENIX_DIRECT_SPIN", "FENIX_DIRECT_QREG", "FENIX_MERGE_RANK_MIN", "FENIX_INT8"};
+      "FENIX_NO_NORM_SHADOW", "FENIX_DEBUG_BF16", "FENIX_DEBUG_TIERS", "FENIX_GRAPH", "FENIX_DIRECT", "FENIX_DIRECT_MAX_MB", "FENIX_DEBUG_DIRECT", "FENIX_DIRECT_SPIN", "FENIX_DIRECT_QREG", "FENIX_MERGE_RANK_MIN", "FENIX_INT8", "FENIX_TC_RESIDENT"};
   for (const char* name : names) {
     if (const char* v = std::getenv(name)) tc_set_knob(k, name, v);
   }
@@ -506,7 +525,7 @@ struct TcParams {
   int aug_line0;          // first 128-byte line of the separate augmented region of the shadow (one block per tile)
   const unsigned char* xb; // base of the tiled bf16 shadow in use (L2 prefetch), or null
   int pf_tiles;           // L2 prefetch distance in tiles (0: off): the TMA ring only covers ~2 tiles, far less than a DRAM miss
-  int rq_stages;          // resident-query kernel: depth of the corpus-block ring
+  int rq_stages;          // resident-query kernels (rq, CTA pair with resident query tiles): depth of the corpus-block ring
   uint32_t sleep_ns;      // producer / MMA polling loops sleep this long between polls (0: spin). Sleeping keeps their
                           // spin loops out of the epilogue warps' issue slots where the epilogue binds (narrow rows);
                           // where the tensor pipe binds (wide rows) a late wake-up costs ~2 % instead
@@ -844,27 +863,39 @@ __device__ __forceinline__ void epi_tighten(const TcParams& p, bool active, int 
 //         tcgen05.commit, "accumulator empty" collects the epilogue warps of both CTAs in the leader.
 //         Units: (query-tile pair) x (corpus slice); CTA r of the pair owns query tile 2*qp + r and keeps the
 //         candidate lists of "CTA unit" slice * (2 n_qp) + 2 qp + r, the layout the finish kernel reads.
+// PAIR 2: CTA pairs over the int8 shadow with the query tiles RESIDENT. An int8 query tile (n_kblocks x 16 KB, 96 KB at
+//         D = 768) fits in shared memory next to a corpus ring, so each CTA loads ITS tile once per unit (a_full: both
+//         CTAs' bytes counted in the leader; a_empty: committed to both CTAs by the leader after the unit's last MMA)
+//         and the ring carries only corpus half blocks: per SM and k-block 16 KB of L2 -> SM operand traffic instead of
+//         32 KB, and the ring (p.rq_stages deep, tc3_stages) looks further ahead. MMAs, commits, TMEM double buffer,
+//         epilogue and the candidate-list layout are those of PAIR 1.
 template <int METRIC, int KIND, int MODE, int PAIR>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 knn_tc_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_x, TcParams p) {
   static_assert(!PAIR || KIND >= 1, "CTA pairs stream a shadow");
-  constexpr int STAGES = PAIR ? TC2_STAGES : TC_STAGES;
+  constexpr bool RES = PAIR == 2;
+  static_assert(!RES || KIND == 2, "resident query tiles: int8 shadow");
+  constexpr int STAGES = RES ? TC3_MAX_STAGES : (PAIR ? TC2_STAGES : TC_STAGES);   // (RES: barriers; p.rq_stages are used)
   constexpr uint32_t B_BYTES = PAIR ? TC2_B_BYTES : TC_B_BYTES;
-  constexpr uint32_t STAGE_BYTES = TC_A_BYTES + B_BYTES;
+  constexpr uint32_t STAGE_BYTES = (RES ? 0u : TC_A_BYTES) + B_BYTES;
+  const int n_stages = RES ? p.rq_stages : STAGES;
   extern __shared__ unsigned char smem_raw[];
   // 1024-byte alignment for the 128B-swizzled operand tiles (the offset is the same in both CTAs of a pair:
   // the dynamic shared memory window starts at the same offset in every CTA of a kernel)
   unsigned char* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  unsigned char* tiles = smem;
-  float* norm_smem = reinterpret_cast<float*>(smem + STAGES * STAGE_BYTES);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + STAGES * STAGE_BYTES + TC_ACC_STAGES * TC_NORM_BYTES);
+  unsigned char* a_res = smem;                                                  // RES: [n_kblocks] query blocks
+  unsigned char* tiles = RES ? smem + p.n_kblocks * TC_A_BYTES : smem;
+  float* norm_smem = reinterpret_cast<float*>(tiles + n_stages * STAGE_BYTES);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(tiles + n_stages * STAGE_BYTES + TC_ACC_STAGES * TC_NORM_BYTES);
   uint64_t* full_bar = bars;                         // [STAGES]      TMA -> MMA          (PAIR: the leader's is used)
   uint64_t* empty_bar = bars + STAGES;               // [STAGES]      MMA -> TMA          (PAIR: multicast to both CTAs)
   uint64_t* tmem_full = bars + 2 * STAGES;           // [2]           MMA -> epilogue     (PAIR: multicast to both CTAs)
   uint64_t* tmem_empty = tmem_full + TC_ACC_STAGES;  // [2]           epilogue -> MMA     (PAIR: both CTAs' warps, in the leader)
   uint64_t* norm_full = tmem_empty + TC_ACC_STAGES;  // [2]           TMA(norms) -> epilogue
   uint64_t* norm_empty = norm_full + TC_ACC_STAGES;  // [2]           epilogue -> TMA(norms) (PAIR only; otherwise tmem_empty serves)
-  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(norm_empty + TC_ACC_STAGES);
+  uint64_t* a_full = norm_empty + TC_ACC_STAGES;     // RES [1]       query tiles of the unit landed (the leader's is used)
+  uint64_t* a_empty = a_full + 1;                    // RES [1]       the unit's last MMAs retired (multicast to both CTAs)
+  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(a_full + (RES ? 2 : 0));
 
   const int warp = threadIdx.x >> 5;
   const uint32_t lane = lane_id();
@@ -875,13 +906,14 @@ knn_tc_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
   if (warp == 0 && lane == 0) {
     prefetch_tmap(&map_q);
     prefetch_tmap(&map_x);
-    for (int i = 0; i < STAGES; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
+    for (int i = 0; i < n_stages; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
     for (int i = 0; i < TC_ACC_STAGES; ++i) {
       mbar_init(&tmem_full[i], 1);
       mbar_init(&tmem_empty[i], PAIR ? 2 * TC_EPI_WARPS : TC_EPI_WARPS);
       mbar_init(&norm_full[i], 1);
       mbar_init(&norm_empty[i], TC_EPI_WARPS);
     }
+    if (RES) { mbar_init(a_full, 1); mbar_init(a_empty, 1); }
     fence_barrier_init();
   }
   if (warp == 2) { if (PAIR) tmem_alloc_pair(tmem_ptr, 512); else tmem_alloc(tmem_ptr, 512); }
@@ -906,9 +938,22 @@ knn_tc_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
       int stage = 0; uint32_t phase = 0;
       int acc = 0; uint32_t acc_phase = 0;
       const uint32_t full_leader = PAIR ? mapa_u32(smem_u32(full_bar), 0) : 0u;   // the leader's full_bar[0]
+      constexpr int kElemsPerBlock = KIND == 0 ? TC_BK : (KIND == 1 ? 2 * TC_BK : 4 * TC_BK);
+      uint32_t a_phase = 0;
       for (int u = cid; u < n_units; u += n_workers) {
         int qt, slice, cu; decode(u, qt, slice, cu);
         const int t0 = slice * p.tiles_per_slice, t1 = min(p.n_vtiles, t0 + p.tiles_per_slice);
+        if (RES) {
+          // this CTA's query tile for the whole unit, once the previous unit's MMAs have retired. Deliberately simple: the
+          // ring drains once per unit here (no corpus block of the next unit is issued before its query tile), one
+          // ~2 us L2/HBM round trip per unit against ~2000 tiles of MMA work per unit at C3 (~5 ms), i.e. < 0.1 %
+          mbar_wait_backoff(a_empty, a_phase ^ 1, p.sleep_ns);
+          if (rank == 0) mbar_expect_tx(a_full, 2u * uint32_t(p.n_kblocks) * TC_A_BYTES);   // both CTAs' tiles
+          const uint32_t a_bar = mapa_u32(smem_u32(a_full), 0);
+          for (int kb = 0; kb < p.n_kblocks; ++kb)
+            tma_load_2d_pair(&map_q, a_bar, a_res + kb * TC_A_BYTES, kb * kElemsPerBlock, qt * TC_BM);
+          a_phase ^= 1;
+        }
         for (int tv = t0; tv < t1; ++tv) {
           const int t = tv * p.tile_stride;
           if (METRIC != 2) {
@@ -921,10 +966,12 @@ knn_tc_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
           for (int kb = 0; kb < p.n_kblocks; ++kb) {
             mbar_wait_backoff(&empty_bar[stage], phase ^ 1, p.sleep_ns);
             unsigned char* a_dst = tiles + stage * STAGE_BYTES;
-            constexpr int kElemsPerBlock = KIND == 0 ? TC_BK : (KIND == 1 ? 2 * TC_BK : 4 * TC_BK);
             // tiled shadow: one contiguous block of 256 (PAIR: this CTA's 128) rows x 128 B
             const int line = kb < p.n_kb_data ? (t * p.n_kb_data + kb) * TC_BN : p.aug_line0 + t * TC_BN;
-            if (PAIR) {
+            if (RES) {
+              if (rank == 0) mbar_expect_tx(&full_bar[stage], 2 * STAGE_BYTES);    // both CTAs' corpus half blocks
+              tma_load_2d_pair(&map_x, full_leader + uint32_t(stage) * 8u, a_dst, 0, line + int(rank) * (TC_BN / 2));
+            } else if (PAIR) {
               if (rank == 0) mbar_expect_tx(&full_bar[stage], 2 * STAGE_BYTES);    // both CTAs' query + corpus blocks
               const uint32_t bar = full_leader + uint32_t(stage) * 8u;
               tma_load_2d_pair(&map_q, bar, a_dst, kb * kElemsPerBlock, qt * TC_BM);
@@ -944,7 +991,7 @@ knn_tc_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
 #endif
               }
             }
-            if (++stage == STAGES) { stage = 0; phase ^= 1; }
+            if (++stage == n_stages) { stage = 0; phase ^= 1; }
           }
           if (++acc == TC_ACC_STAGES) { acc = 0; acc_phase ^= 1; }
         }
@@ -961,20 +1008,25 @@ knn_tc_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
       const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
       const uint64_t desc0 = make_smem_desc(0);
       const uint32_t tiles_lo = smem_u32(tiles) >> 4;
+      const uint32_t a_lo = smem_u32(a_res) >> 4;   // RES: query k-block kb at + kb * 1024
       const int n_kb = p.n_kblocks, n_kb_data = p.n_kb_data, nk_last = p.nk_last;
       int stage = 0; uint32_t phase = 0;
       int acc = 0; uint32_t acc_phase = 0;
+      uint32_t a_phase = 0;
       for (int u = cid; u < n_units; u += n_workers) {
         int qt, slice, cu; decode(u, qt, slice, cu);
         const int t0 = slice * p.tiles_per_slice, t1 = min(p.n_vtiles, t0 + p.tiles_per_slice);
+        if (RES) { mbar_wait(a_full, a_phase); a_phase ^= 1; }
         for (int t = t0; t < t1; ++t) {
           mbar_wait_backoff(&tmem_empty[acc], acc_phase ^ 1, p.sleep_ns >> 1);
           const uint32_t d_tmem = tmem_u + uint32_t(acc * TC_BN);
           for (int kb = 0; kb < n_kb; ++kb) {
             mbar_wait(&full_bar[stage], phase);
             tc_fence_after();
-            const uint64_t a_desc = desc0 | uint64_t(tiles_lo + uint32_t(stage) * (STAGE_BYTES >> 4));
-            const uint64_t b_desc = a_desc + (TC_A_BYTES >> 4);
+            const uint64_t a_desc = RES ? desc0 | uint64_t(a_lo + uint32_t(kb) * (TC_A_BYTES >> 4))
+                                        : desc0 | uint64_t(tiles_lo + uint32_t(stage) * (STAGE_BYTES >> 4));
+            const uint64_t b_desc = RES ? desc0 | uint64_t(tiles_lo + uint32_t(stage) * (STAGE_BYTES >> 4))
+                                        : a_desc + (TC_A_BYTES >> 4);
             const int nk = kb < n_kb_data - 1 ? TC_BK / TC_UMMA_K : (kb == n_kb_data - 1 ? nk_last : 1);
             if (elect_one()) {
               // advance 32 B along K inside the 128 B swizzle row: +2 in the (>>4) address field
@@ -1014,9 +1066,15 @@ knn_tc_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
               }
             }
             __syncwarp();
-            if (++stage == STAGES) { stage = 0; phase ^= 1; }
+            if (++stage == n_stages) { stage = 0; phase ^= 1; }
           }
           if (++acc == TC_ACC_STAGES) { acc = 0; acc_phase ^= 1; }
+        }
+        // RES: both CTAs may replace their query tiles once everything issued so far has retired (not after the
+        // worker's last unit: no reload waits for it, and no signal may reach a CTA that is leaving)
+        if (RES && u + n_workers < n_units) {
+          if (elect_one()) umma_commit_pair(a_empty);
+          __syncwarp();
         }
       }
     }
@@ -1073,12 +1131,12 @@ knn_tc_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
         if (KIND == 2) {
           const double ss = double(ts.x) * double(qs.x);
           const double ae = fma(double(qs.y), double(ts.y), double(qs.z)) + 0x1p-48;   // a_q E_t + e_q (+ rounding pad)
-          epi_tile_i8<METRIC, MODE, PAIR>(t_lane + uint32_t(acc * TC_BN), any_active ? ncols : 0, nrm, col0, tau,
-                                          i8_threshold(tau, ss, ae), 1.0 / ss, ae, buf, wn, &tmem_empty[acc],
-                                          tmem_empty_leader + uint32_t(acc) * 8u, &norm_empty[acc], lane, dbg_row, pre_out);
+          epi_tile_i8<METRIC, MODE, (PAIR != 0)>(t_lane + uint32_t(acc * TC_BN), any_active ? ncols : 0, nrm, col0, tau,
+                                                    i8_threshold(tau, ss, ae), 1.0 / ss, ae, buf, wn, &tmem_empty[acc],
+                                                    tmem_empty_leader + uint32_t(acc) * 8u, &norm_empty[acc], lane, dbg_row, pre_out);
         } else {
-          epi_tile<METRIC, MODE, PAIR>(t_lane + uint32_t(acc * TC_BN), any_active ? ncols : 0, nrm, col0, tau, buf, wn,
-                                       &tmem_empty[acc], tmem_empty_leader + uint32_t(acc) * 8u, &norm_empty[acc], lane, dbg_row, pre_out);
+          epi_tile<METRIC, MODE, (PAIR != 0)>(t_lane + uint32_t(acc * TC_BN), any_active ? ncols : 0, nrm, col0, tau, buf, wn,
+                                                 &tmem_empty[acc], tmem_empty_leader + uint32_t(acc) * 8u, &norm_empty[acc], lane, dbg_row, pre_out);
         }
         if (++acc == TC_ACC_STAGES) { acc = 0; acc_phase ^= 1; }
         if (MODE != 2) epi_tighten(p, active, q, buf, wn, wn_trig, tau, lane);
@@ -1975,6 +2033,8 @@ inline bool tc_init(TcState* st, int sm_count, std::string* err) {
   attr(knn_tc_filter_kernel<2, 2, 2, 0>, TC_SMEM_BYTES);
   attr(knn_tc_filter_kernel<0, 2, 0, 1>, TC2_SMEM_BYTES); attr(knn_tc_filter_kernel<2, 2, 0, 1>, TC2_SMEM_BYTES);
   attr(knn_tc_filter_kernel<2, 2, 2, 1>, TC2_SMEM_BYTES);
+  attr(knn_tc_filter_kernel<0, 2, 0, 2>, TC3_SMEM_MAX); attr(knn_tc_filter_kernel<2, 2, 0, 2>, TC3_SMEM_MAX);
+  attr(knn_tc_filter_kernel<2, 2, 2, 2>, TC3_SMEM_MAX);
   if (a == cudaSuccess) a = cudaFuncSetAttribute(knn_rq_filter_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, RQ_SMEM_MAX);
   if (a == cudaSuccess) a = cudaFuncSetAttribute(knn_rq_filter_kernel<0, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, RQ_SMEM_MAX);
   if (a == cudaSuccess) a = cudaFuncSetAttribute(knn_rq_filter_kernel<2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, RQ_SMEM_MAX);
@@ -2036,6 +2096,7 @@ struct TcPlan {
   int qt_major;
   int rq;        // 1: resident-query kernel (units = query pairs x slices of 128-row tiles, one list per unit and query)
   int pair;      // 1: CTA-pair streaming kernel (units = query pairs x slices; candidate lists per CTA as in the one-CTA kernel)
+  int resident;  // 1: the CTA-pair kernel with resident query tiles (int8 shadow; same units and candidate lists as pair)
   int n_qt_lists;// query tiles the candidate-list layout is indexed with (2 n_qp for the pair kernel, else n_qt)
   int n_qp;      // query pairs
   int kp_list;   // candidates each (query, list) keeps at a selection (<= kp)
@@ -2085,7 +2146,17 @@ inline TcPlan tc_plan(const TcState* st, const TcSearch& s) {
   // (auto: from 7 k-blocks per row on. A tile of D = 384 is 24 MMAs and the pair's cluster-wide hand-offs cost more than
   // the halved B traffic saves - 1452 vs 1541 TFLOP/s at uncapped clocks; from D = 512 the pair wins, 1645 vs 1519 TFLOP/s at
   // D = 768: scripts/ubench/width_sweep.py, profiles/r02_sweep_row_width.txt)
-  pl.pair = (!pl.rq && s.kind >= 1 && pl.n_qt >= 2 && s.dbg == nullptr && (kn.pair == 1 || (kn.pair < 0 && pl.kb_bf16 >= 7))) ? 1 : 0;
+  const bool pair_ok = !pl.rq && s.kind >= 1 && pl.n_qt >= 2 && s.dbg == nullptr;
+  pl.pair = (pair_ok && (kn.pair == 1 || (kn.pair < 0 && pl.kb_bf16 >= 7))) ? 1 : 0;
+  // int8 shadow: the query tile (16 KB per k-block) stays in shared memory for the whole unit when it leaves room for
+  // TC3_MIN_STAGES corpus stages (D <= 1152). Auto: where the CTA-pair kernel runs over a shard of >= 4M rows. Measured
+  // (4096 queries, D = 512 / 768 / 1024, profiles/r04_int8_widths.txt): 10M rows 7.7 / 6.6 / -0.3 % less filter time than
+  // the streaming pair, 5M rows 1.4 / 7.9 / 4.4 % (4.4 % at D = 768 with the sample prepass off), but 2.5M and 1M rows
+  // 2 - 25 % MORE, with or without the prepass
+  constexpr int64_t TC3_MIN_ROWS = int64_t(1) << 22;
+  const bool res_fits = s.kind == 2 && tc3_stages(pl.n_kblocks) >= TC3_MIN_STAGES;
+  pl.resident = (pair_ok && res_fits && (kn.resident == 1 || (kn.resident < 0 && pl.pair && s.n_rows >= TC3_MIN_ROWS))) ? 1 : 0;
+  if (pl.resident) pl.pair = 1;
   pl.n_qt_lists = pl.pair ? 2 * pl.n_qp : pl.n_qt;
   const int n_tiles_full = pl.rq ? int((s.n_rows + RQ_BN - 1) / RQ_BN) : pl.n_tiles;   // tiles in the kernel's own unit
   pl.tile_stride = pre ? s.sample_stride : 1;
@@ -2325,6 +2396,12 @@ inline bool tc_run_pass(TcState* st, TcCorpus* tc, const TcSearch& s, const TcPl
       if (epi == 0) launch(knn_rq_filter_kernel<0, 0>, map_h, rq_smem, 1);
       else launch(knn_rq_filter_kernel<2, 0>, map_h, rq_smem, 1);
     }
+  } else if (pl.resident) {
+    p.rq_stages = tc3_stages(pl.n_kblocks);
+    const uint32_t smem = tc3_smem_bytes(pl.n_kblocks);
+    if (epi == 0) launch(knn_tc_filter_kernel<0, 2, 0, 2>, tc->map_x8_h, smem, 2);   // (masked: no prepass)
+    else if (pre) launch(knn_tc_filter_kernel<2, 2, 2, 2>, tc->map_x8_h, smem, 2);
+    else launch(knn_tc_filter_kernel<2, 2, 0, 2>, tc->map_x8_h, smem, 2);
   } else if (pl.pair && s.kind == 2) {
     if (epi == 0) launch(knn_tc_filter_kernel<0, 2, 0, 1>, tc->map_x8_h, TC2_SMEM_BYTES, 2);   // (masked: no prepass)
     else if (pre) launch(knn_tc_filter_kernel<2, 2, 2, 1>, tc->map_x8_h, TC2_SMEM_BYTES, 2);
@@ -2433,7 +2510,7 @@ inline bool tc_search(TcState* st, TcCorpus* tc, const TcSearch& s, const TcLaun
     *launched += 1;
   }
   // threshold prepass over a strided sample (the padded queries and tau_g sit at the same scratch offsets in both plans)
-  if (variant) *variant = (pl.rq ? 1 : 0) | (L.with_pre ? 2 : 0) | (pl.pair ? 4 : 0);
+  if (variant) *variant = (pl.rq ? 1 : 0) | (L.with_pre ? 2 : 0) | (pl.pair ? 4 : 0) | (pl.resident ? 8 : 0);
   if (L.with_pre) {
     if (!tc_run_pass(st, tc, L.pre, L.ppl, scratch, map_q, err)) return false;
     *launched += 2;

@@ -25,7 +25,7 @@ __all__ = [
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB_NAME = "libfenix_knn.so"
 COMM_ID_BYTES = 128
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 FX_OK = 0
 FX_EINVAL, FX_ECUDA, FX_ENOMEM, FX_ESTATE, FX_EUNSUP = -1, -2, -3, -4, -5
@@ -68,7 +68,7 @@ class _FxStats(ctypes.Structure):
         ("fallback_queries", ctypes.c_int64), ("refined_queries", ctypes.c_int64), ("kernel_launches", ctypes.c_int64),
         ("last_search_ms", ctypes.c_double), ("last_main_kernel_ms", ctypes.c_double),
         ("last_path", ctypes.c_int32), ("last_variant", ctypes.c_int32), ("last_exchange_ms", ctypes.c_double),
-        ("last_operand", ctypes.c_int32),
+        ("last_operand", ctypes.c_int32), ("last_resident_queries", ctypes.c_int32),
     ]
 
 
@@ -89,6 +89,7 @@ class Stats:
     last_variant: int = 0
     last_exchange_ms: float = 0.0
     last_operand: int = 0          # filter operand of the last search: 0 fp32 / TF32, 1 bf16, 2 int8
+    last_resident_queries: int = 0 # 1: int8 CTA-pair filter with resident query tiles
 
 
 _lib_lock = threading.Lock()

@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define FX_ABI_VERSION 4
+#define FX_ABI_VERSION 5
 
 /* error codes */
 #define FX_OK 0
@@ -94,6 +94,8 @@ typedef struct fx_stats {
   double last_exchange_ms;   /* sharded searches: device time of all-gather + merge of the last search (CUDA events) */
   int32_t last_operand;      /* operand of the last search's filter: 0 = fp32 / TF32 (or no filter), 1 = bf16 shadow,
                               * 2 = int8 normalised shadow (exact cosine at small k) */
+  int32_t last_resident_queries; /* 1 = the last search's filter was the int8 CTA-pair kernel with its query tiles resident in
+                              * shared memory (last_variant bit 2 is set too), else 0 */
 } fx_stats;
 
 /* ---- lifetime -------------------------------------------------------------------------- */

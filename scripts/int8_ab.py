@@ -1,11 +1,12 @@
 """int8 against bf16 shadow filter for exact cosine (k = 10, 4096 queries, Gaussian rows), and the K' sweep that sets
 TC_KP_I8 (tc_filter.cuh).
 
-    python scripts/int8_ab.py widths [--rows 1000000] [--dims 256,384,512,768]
+    python scripts/int8_ab.py widths [--rows 1000000] [--dims 256,384,512,768,1024]
     python scripts/int8_ab.py kp [--rows 10000000,1250000] [--ks 10,16] [--kps 128,160,192,224,256,320]
 
 widths: for each row width, the bf16 and the int8 filter (FENIX_INT8=0 / 1) through the CTA-pair and the one-CTA streaming
-kernel (FENIX_TC_PAIR=1 / 0): the main filter kernel's time (mean of 4 searches after 2 warm-up searches), its rate and
+kernel (FENIX_TC_PAIR=1 / 0), and for int8 also the CTA-pair kernel with resident query tiles (FENIX_TC_RESIDENT=1; the
+two others run with it off): the main filter kernel's time (mean of 4 searches after 2 warm-up searches), its rate and
 share of the data sheet's dense int8 peak (ops = 2 Q N D, bytes = N D of the int8 shadow), the queries refined and sent to
 the fp64 scan per search, and the SM clock / power limit read right after the runs.
 kp: refined and scanned queries per search of the int8 filter at D = 768 for each forced K' (FENIX_TC_KP). TC_KP_I8 is the
@@ -71,16 +72,19 @@ def widths(args):
         ref = None
         for op, i8 in (("bf16", 0), ("int8", 1)):
             ctx.set_option("FENIX_INT8", i8)
-            for kern, pair in (("pair", 1), ("one-CTA", 0)):
+            kernels = (("pair", 1, 0), ("one-CTA", 0, 0)) if i8 == 0 else (("resident", 1, 1), ("pair", 1, 0), ("one-CTA", 0, 0))
+            for kern, pair, res in kernels:
                 ctx.set_option("FENIX_TC_PAIR", pair)
+                ctx.set_option("FENIX_TC_RESIDENT", res)
                 ms, st, refd, fb, rows = run(ctx, c, q, 10)
                 same = "-" if ref is None else str(torch.equal(rows, ref))
                 ref = rows if ref is None else ref
                 tops = ops / ms / 1e9
-                print(f"D={d} N={args.rows} {op:4s} {kern:7s} kernel {ms:8.3f} ms  {tops:7.0f} TOPS  {tops / INT8_PEAK_TOPS:.3f} of int8 peak"
+                print(f"D={d} N={args.rows} {op:4s} {kern:8s} kernel {ms:8.3f} ms  {tops:7.0f} TOPS  {tops / INT8_PEAK_TOPS:.3f} of int8 peak"
                       f"  {args.rows * d / ms / 1e9:6.2f} TB/s int8 bytes  operand {st.last_operand} variant {st.last_variant}"
-                      f"  refined {refd:.1f} scanned {fb:.1f} per search  same ids {same}", flush=True)
+                      f" resident {st.last_resident_queries}  refined {refd:.1f} scanned {fb:.1f} per search  same ids {same}", flush=True)
         ctx.set_option("FENIX_TC_PAIR", None)
+        ctx.set_option("FENIX_TC_RESIDENT", None)
         ctx.set_option("FENIX_INT8", None)
         print(f"  gpu: {gpu_state()}", flush=True)
         c.close()
@@ -107,7 +111,7 @@ if __name__ == "__main__":
     ap = argparse.ArgumentParser()
     ap.add_argument("what", choices=["widths", "kp"])
     ap.add_argument("--rows", default=None)
-    ap.add_argument("--dims", default="256,384,512,768")
+    ap.add_argument("--dims", default="256,384,512,768,1024")
     ap.add_argument("--ks", default="10,16")
     ap.add_argument("--kps", default="128,160,192,224,256,320")
     a = ap.parse_args()
