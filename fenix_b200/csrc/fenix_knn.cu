@@ -32,6 +32,9 @@
 #include "exact_scan.cuh"
 #include "direct_scan.cuh"
 #include "tc_filter.cuh"
+#include "range_search.cuh"
+
+#include <cub/device/device_segmented_sort.cuh>
 
 // ----------------------------------------------------------------------------------------
 // error plumbing
@@ -113,6 +116,8 @@ struct fx_ctx {
   std::mutex mu;                   // one search at a time per device context
   cudaEvent_t ev_x0 = nullptr, ev_x1 = nullptr;   // exchange (all-gather + merge) of a sharded search
   DevBuf d_q, d_rows, d_dist, d_mask, d_partial, d_qlist, d_tc, d_ref, d_maskn, d_floor, d_xchg, d_hdr, d_tickets;
+  DevBuf d_hits, d_hits2, d_col, d_rmeta, d_rbatch, d_cub;   // range search: hit keys (+ sorted copy), distance columns,
+                                                              // per-query and per-batch arrays, CUB scratch
   HostBuf h_q, h_rows, h_dist, h_flags;
   unsigned int* d_ticket = nullptr;   // direct scan: "last CTA merges" counter (zero between launches)
   unsigned long long* h_done = nullptr;   // pinned: direct scan completion word [0] = sequence number, [1] = kernel ns
@@ -280,6 +285,7 @@ extern "C" int fx_shutdown(fx_ctx* ctx) {
   ctx->d_q.release(); ctx->d_rows.release(); ctx->d_dist.release(); ctx->d_mask.release();
   ctx->d_partial.release(); ctx->d_qlist.release(); ctx->d_tc.release(); ctx->d_ref.release(); ctx->d_maskn.release();
   ctx->d_floor.release(); ctx->d_xchg.release(); ctx->d_hdr.release(); ctx->d_tickets.release();
+  ctx->d_hits.release(); ctx->d_hits2.release(); ctx->d_col.release(); ctx->d_rmeta.release(); ctx->d_rbatch.release(); ctx->d_cub.release();
   ctx->h_q.release(); ctx->h_rows.release(); ctx->h_dist.release(); ctx->h_flags.release();
   if (ctx->h_word) cudaFreeHost(ctx->h_word);
   if (ctx->d_ticket) cudaFree(ctx->d_ticket);
@@ -1365,6 +1371,238 @@ extern "C" int fx_distances(fx_corpus* c, const float* query, int32_t metric, fl
   FX_CUDA(cudaMemcpyAsync(ctx->h_dist.p, ctx->d_dist.p, d_bytes, cudaMemcpyDeviceToHost, ctx->stream));
   FX_CUDA(cudaStreamSynchronize(ctx->stream));
   std::memcpy(out_dist, ctx->h_dist.p, d_bytes);
+  return FX_OK;
+}
+
+// ----------------------------------------------------------------------------------------
+// range search: every row within a radius (DESIGN.md, "Range search")
+// ----------------------------------------------------------------------------------------
+// Grows `b` to `need` bytes keeping its first `used` bytes (the hit buffer fills in several steps).
+static int grow_keep(fx_ctx* ctx, DevBuf& b, size_t used, size_t need) {
+  if (need <= b.cap) return FX_OK;
+  DevBuf nb;
+  FX_TRY(nb.ensure(need));
+  if (used) FX_CUDA(cudaMemcpyAsync(nb.p, b.p, used, cudaMemcpyDeviceToDevice, ctx->stream));
+  FX_CUDA(cudaStreamSynchronize(ctx->stream));
+  b.release();
+  b = nb;
+  return FX_OK;
+}
+
+// Distance columns of a range-search batch: at most this much scratch (or one column), whatever n_q x N is.
+constexpr size_t RANGE_COL_BYTES = size_t(256) << 20;
+
+// Hits of the listed queries by the exact scan: the distance columns of a batch of queries at a time, then the unmasked
+// rows within the radius become keys in each query's segment of ctx->d_hits, appended at *used. seg / hits: host
+// arrays over every query of the search.
+static int range_scan(fx_corpus* c, const float* d_q, int64_t n_q, const std::vector<int>& list, int metric, float radius,
+                      const uint8_t* d_mask, std::vector<int64_t>& seg, std::vector<int64_t>& hits, size_t* used) {
+  fx_ctx* ctx = c->ctx;
+  const size_t per_q = size_t(c->pitch) * 8 + 8 + 8 + 8 + 2 * 8 + 4;   // exact_scan_kernel's shared memory, column mode
+  const int qb = int(std::min<size_t>(fx::SCAN_MAX_QB, (200 * 1024) / per_q));
+  if (qb < 1) return fail(FX_EUNSUP, "fx_search_range: dim %d too large for the exact scan", c->dim);
+  const int batch = int(std::max<int64_t>(1, std::min<int64_t>(4096, int64_t(RANGE_COL_BYTES / (size_t(c->n) * 4)))));
+  const int nb_max = int(std::min<size_t>(size_t(batch), list.size()));
+  FX_TRY(ctx->d_col.ensure(size_t(nb_max) * c->n * 4));
+  FX_TRY(ctx->d_rbatch.ensure(size_t(nb_max) * 24));   // per slot: list entry, count, fill (int) and segment (int64)
+  FX_TRY(ctx->h_flags.ensure(size_t(nb_max) * sizeof(int)));
+  float* col = static_cast<float*>(ctx->d_col.p);
+  int64_t* d_seg = static_cast<int64_t*>(ctx->d_rbatch.p);
+  int* d_list = reinterpret_cast<int*>(d_seg + nb_max);
+  int* d_cnt = d_list + nb_max;
+  int* d_fill = d_cnt + nb_max;
+  int* h_cnt = static_cast<int*>(ctx->h_flags.p);
+  std::vector<int64_t> seg_b(nb_max);
+  const int64_t tiles = (c->n + fx::SCAN_THREADS - 1) / fx::SCAN_THREADS;
+  const int cblocks = int(std::min<int64_t>((c->n + 255) / 256, 256));
+  for (size_t b0 = 0; b0 < list.size(); b0 += size_t(batch)) {
+    const int nb = int(std::min<size_t>(size_t(batch), list.size() - b0));
+    FX_CUDA(cudaMemcpyAsync(d_list, list.data() + b0, size_t(nb) * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+    FX_CUDA(cudaMemsetAsync(d_cnt, 0, size_t(2 * nb_max) * sizeof(int), ctx->stream));   // counts and fills
+    fx::ScanParams p{};
+    p.X = c->X; p.n_rows = c->n; p.pitch = c->pitch; p.dim = c->dim; p.Q = d_q; p.n_q = int(n_q); p.metric = metric;
+    p.mask = nullptr; p.q_list = d_list; p.n_list = nb; p.k = 0; p.buf = 2; p.qb = std::min(qb, nb); p.floor = nullptr;
+    p.partial = nullptr; p.dist_out = col;
+    const int groups = (nb + p.qb - 1) / p.qb;
+    const int W = int(std::min<int64_t>(tiles, std::max<int64_t>(1, (8 * int64_t(ctx->sm_count) + groups - 1) / groups)));
+    fx::exact_scan_kernel<<<dim3(W, groups), fx::SCAN_THREADS, per_q * p.qb + 16, ctx->stream>>>(p);
+    FX_CUDA(cudaGetLastError());
+    fx::range_col_count_kernel<<<dim3(cblocks, nb), 256, 0, ctx->stream>>>(col, c->n, d_mask, radius, d_cnt);
+    FX_CUDA(cudaGetLastError());
+    FX_CUDA(cudaMemcpyAsync(h_cnt, d_cnt, size_t(nb) * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    FX_CUDA(cudaStreamSynchronize(ctx->stream));
+    const size_t before = *used;
+    for (int i = 0; i < nb; ++i) {
+      const int q = list[b0 + i];
+      seg[q] = seg_b[i] = int64_t(*used);
+      hits[q] = h_cnt[i];
+      *used += size_t(h_cnt[i]);
+    }
+    FX_TRY(grow_keep(ctx, ctx->d_hits, before * 8, std::max<size_t>(*used, 1) * 8));
+    FX_CUDA(cudaMemcpyAsync(d_seg, seg_b.data(), size_t(nb) * sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream));
+    fx::range_col_compact_kernel<<<dim3(cblocks, nb), 256, 0, ctx->stream>>>(col, c->n, d_mask, radius, d_seg, d_fill,
+                                                                             static_cast<uint64_t*>(ctx->d_hits.p));
+    FX_CUDA(cudaGetLastError());
+    ctx->launches += 3; c->stats.kernel_launches += 3;
+  }
+  return FX_OK;
+}
+
+extern "C" int fx_search_range(fx_corpus* c, const float* queries, int64_t n_q, int32_t metric, float radius,
+                               int32_t precision, const uint8_t* row_mask, int64_t capacity, int64_t* out_offsets,
+                               int64_t* out_rows, float* out_dist) {
+  FX_LEASE(c, "fx_search_range");
+  NvtxRange nvtx("fenix:search_range");
+  if (!c->finalized) return fail(FX_ESTATE, "fx_search_range: corpus is not finalized");
+  if (n_q < 0 || capacity < 0) return fail(FX_EINVAL, "fx_search_range: negative query count or capacity");
+  if (!out_offsets || (n_q > 0 && !queries) || (capacity > 0 && (!out_rows || !out_dist)))
+    return fail(FX_EINVAL, "fx_search_range: NULL buffer");
+  if (n_q > int64_t(1) << 24) return fail(FX_EUNSUP, "fx_search_range: at most 2^24 queries per call");
+  if (metric < 0 || metric > 2) return fail(FX_EINVAL, "fx_search_range: unknown metric %d", metric);
+  if (radius != radius) return fail(FX_EINVAL, "fx_search_range: radius is NaN");
+  if (precision == FX_PREC_TF32 || precision == FX_PREC_BF16)
+    return fail(FX_EUNSUP, "fx_search_range: range search is exact only (FX_PREC_FP32 or FX_PREC_EXACT_SCAN)");
+  if (precision != FX_PREC_FP32 && precision != FX_PREC_EXACT_SCAN)
+    return fail(FX_EINVAL, "fx_search_range: unknown precision mode %d", precision);
+  std::fill(out_offsets, out_offsets + n_q + 1, int64_t(0));
+  if (n_q == 0 || c->n == 0) return FX_OK;
+  fx_ctx* ctx = c->ctx;
+  std::lock_guard<std::mutex> lock(ctx->mu);
+  FX_TRY(bind(ctx));
+  const size_t q_bytes = size_t(n_q) * c->dim * sizeof(float);
+  FX_TRY(ctx->d_q.ensure(q_bytes));
+  FX_TRY(ctx->h_q.ensure(q_bytes));
+  std::memcpy(ctx->h_q.p, queries, q_bytes);
+  FX_CUDA(cudaEventRecord(ctx->ev_start, ctx->stream));
+  FX_CUDA(cudaMemcpyAsync(ctx->d_q.p, ctx->h_q.p, q_bytes, cudaMemcpyHostToDevice, ctx->stream));
+  const float* d_q = static_cast<const float*>(ctx->d_q.p);
+  const uint8_t* d_mask = nullptr;
+  if (row_mask) {
+    FX_TRY(ctx->d_mask.ensure(size_t(c->n)));
+    FX_CUDA(cudaMemcpyAsync(ctx->d_mask.p, row_mask, size_t(c->n), cudaMemcpyHostToDevice, ctx->stream));
+    d_mask = static_cast<const uint8_t*>(ctx->d_mask.p);
+  }
+  // per-query device arrays: segment start, candidate count, segment end (int64), output offsets [n_q + 1],
+  // preset threshold, hit count
+  size_t off = 0;
+  auto take = [&](size_t bytes) { size_t o = off; off = (off + bytes + 255) & ~size_t(255); return o; };
+  const size_t o_seg = take(size_t(n_q) * 8), o_cand = take(size_t(n_q) * 8), o_end = take(size_t(n_q) * 8);
+  const size_t o_off = take(size_t(n_q + 1) * 8), o_tau = take(size_t(n_q) * 4), o_hits = take(size_t(n_q) * 4);
+  FX_TRY(ctx->d_rmeta.ensure(off));
+  char* rm = static_cast<char*>(ctx->d_rmeta.p);
+  int64_t* d_seg = reinterpret_cast<int64_t*>(rm + o_seg);
+  int64_t* d_cand = reinterpret_cast<int64_t*>(rm + o_cand);
+  int64_t* d_end = reinterpret_cast<int64_t*>(rm + o_end);
+  int64_t* d_off = reinterpret_cast<int64_t*>(rm + o_off);
+  uint32_t* d_tau = reinterpret_cast<uint32_t*>(rm + o_tau);
+  int* d_hitcnt = reinterpret_cast<int*>(rm + o_hits);
+  FX_TRY(ctx->h_rows.ensure(size_t(n_q + 1) * 8));
+  int64_t* h_i64 = static_cast<int64_t*>(ctx->h_rows.p);
+
+  std::vector<int64_t> seg(n_q, 0), hits(n_q, 0);
+  std::vector<int> scan_list;
+  size_t used = 0;
+  SearchRun run;
+  run.n_q = n_q;
+  // tensor-core path: the operand an exact k = 1 search would filter with, thresholds from the radius, no selection
+  const bool want_tc = precision == FX_PREC_FP32 && fx::tc_supported(&ctx->tc, &c->tc, c->n, c->dim, 1, int(n_q));
+  if (want_tc) {
+    fx::TcSearch s{};
+    s.X = c->X; s.hx = c->hx; s.rx = c->rx; s.n_rows = c->n; s.dim = c->dim; s.pitch = c->pitch;
+    s.row_base = c->row_base; s.max_norm = c->max_norm; s.Q = d_q; s.n_q = int(n_q); s.metric = metric; s.k = 1;
+    s.certify = true; s.out_rows = nullptr; s.out_dist = nullptr;
+    s.stream = ctx->stream; s.ev_k0 = ctx->ev_k0; s.ev_k1 = ctx->ev_k1; s.ev_flags = cudaEventRecordDefault; s.dbg = nullptr;
+    s.tau_fixed = d_tau; s.no_prepass = 1; s.full_lists = 1; s.no_finish = 1;
+    const bool have_i8 = int8_wanted(c, metric, 1, FX_PREC_FP32) && ensure_i8_shadow(c);
+    const bool have_shadow = !have_i8 && !ctx->tc.knobs.fp32_filter_tf32 &&
+                             ((metric == 1 && ensure_norm_shadow(c)) || ensure_plain_shadow(c));
+    const int kind = have_i8 ? 2 : (have_shadow ? 1 : 0);
+    FX_TRY(configure_filter(c, metric, kind, d_mask, &s));
+    double c_err = 0.0, c_add = 0.0;
+    fx::tc_cert_consts(s, &c_err, &c_add);
+    fx::range_prep_kernel<<<int((n_q + 3) / 4), 128, 0, ctx->stream>>>(d_q, int(n_q), c->dim, metric, radius, c->max_norm,
+                                                                       c_err, c_add, kind == 2 ? 1 : 0, d_tau);
+    FX_CUDA(cudaGetLastError());
+    const fx::TcLaunch L = fx::tc_prepare(&ctx->tc, s);
+    FX_TRY(ctx->d_tc.ensure(L.scratch_bytes));
+    std::string err;
+    int launched = 0, variant = 0;
+    if (!fx::tc_search(&ctx->tc, &c->tc, s, L, ctx->d_tc.p, &launched, &err, &variant)) return fail(FX_ECUDA, "fx_search_range: %s", err.c_str());
+    const fx::FinishParams f = fx::tc_finish_params(s, L.pl, ctx->d_tc.p);
+    fx::range_count_kernel<<<int((n_q + 7) / 8), 256, 0, ctx->stream>>>(f, d_cand);
+    FX_CUDA(cudaGetLastError());
+    FX_CUDA(cudaMemcpyAsync(h_i64, d_cand, size_t(n_q) * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    FX_CUDA(cudaStreamSynchronize(ctx->stream));
+    for (int64_t q = 0; q < n_q; ++q) {
+      if (h_i64[q] < 0) { scan_list.push_back(int(q)); continue; }   // a candidate list overflowed
+      seg[q] = int64_t(used);
+      used += size_t(h_i64[q]);
+    }
+    FX_TRY(ctx->d_hits.ensure(std::max<size_t>(used, 1) * 8));
+    FX_CUDA(cudaMemcpyAsync(d_seg, seg.data(), size_t(n_q) * 8, cudaMemcpyHostToDevice, ctx->stream));
+    fx::range_finish_kernel<<<int(n_q), 256, size_t(c->pitch) * 4 + 16, ctx->stream>>>(f, radius, d_seg,
+                                                                                      static_cast<uint64_t*>(ctx->d_hits.p), d_hitcnt);
+    FX_CUDA(cudaGetLastError());
+    ctx->launches += launched + 3; c->stats.kernel_launches += launched + 3;   // (+ prep, count, finish)
+    run.tc = true; run.path = kind == 0 ? 1 : 2; run.operand = kind;
+    set_variant(c, variant);
+    c->stats.fallback_queries += int64_t(scan_list.size());
+  } else {
+    scan_list.resize(size_t(n_q));
+    for (int64_t q = 0; q < n_q; ++q) scan_list[size_t(q)] = int(q);
+    FX_CUDA(cudaEventRecord(ctx->ev_k0, ctx->stream));
+  }
+  if (want_tc) {
+    // hit counts of the tensor-core queries (the scan's own are counted on the host)
+    FX_CUDA(cudaMemcpyAsync(h_i64, d_hitcnt, size_t(n_q) * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    FX_CUDA(cudaStreamSynchronize(ctx->stream));
+    const int* h_hits = reinterpret_cast<const int*>(h_i64);
+    for (int64_t q = 0; q < n_q; ++q) hits[q] = h_hits[q];
+  }
+  if (!scan_list.empty()) FX_TRY(range_scan(c, d_q, n_q, scan_list, metric, radius, d_mask, seg, hits, &used));
+  if (!want_tc) FX_CUDA(cudaEventRecord(ctx->ev_k1, ctx->stream));
+  for (int64_t q = 0; q < n_q; ++q) out_offsets[q + 1] = out_offsets[q] + hits[q];
+  const int64_t total = out_offsets[n_q];
+  if (total > capacity || total == 0) {
+    FX_CUDA(cudaEventRecord(ctx->ev_stop, ctx->stream));
+    FX_CUDA(cudaStreamSynchronize(ctx->stream));
+    search_account(c, run);
+    if (total > capacity)
+      return fail(FX_ETRUNC, "fx_search_range: %lld hits exceed the capacity of %lld (out_offsets holds the sizes needed)",
+                  (long long)total, (long long)capacity);
+    return FX_OK;
+  }
+  if (used > size_t(INT32_MAX)) return fail(FX_EUNSUP, "fx_search_range: %zu candidates exceed 2^31 - 1 (split the query batch)", used);
+  // sort every query's segment by (distance, row), then write rows and distances at its output offset
+  {
+    std::vector<int64_t> end(n_q);
+    for (int64_t q = 0; q < n_q; ++q) end[q] = seg[q] + hits[q];
+    FX_CUDA(cudaMemcpyAsync(d_seg, seg.data(), size_t(n_q) * 8, cudaMemcpyHostToDevice, ctx->stream));
+    FX_CUDA(cudaMemcpyAsync(d_end, end.data(), size_t(n_q) * 8, cudaMemcpyHostToDevice, ctx->stream));
+    FX_CUDA(cudaMemcpyAsync(d_off, out_offsets, size_t(n_q + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
+    FX_TRY(ctx->d_hits2.ensure(used * 8));
+    const uint64_t* keys = static_cast<const uint64_t*>(ctx->d_hits.p);
+    uint64_t* sorted = static_cast<uint64_t*>(ctx->d_hits2.p);
+    size_t tmp_bytes = 0;
+    FX_CUDA(cub::DeviceSegmentedSort::SortKeys(nullptr, tmp_bytes, keys, sorted, int(used), int(n_q), d_seg, d_end, ctx->stream));
+    FX_TRY(ctx->d_cub.ensure(std::max<size_t>(tmp_bytes, 1)));
+    FX_CUDA(cub::DeviceSegmentedSort::SortKeys(ctx->d_cub.p, tmp_bytes, keys, sorted, int(used), int(n_q), d_seg, d_end, ctx->stream));
+    FX_TRY(ctx->d_rows.ensure(size_t(total) * 8));
+    FX_TRY(ctx->d_dist.ensure(size_t(total) * 4));
+    fx::range_gather_kernel<<<int(n_q), 256, 0, ctx->stream>>>(sorted, d_seg, d_off, c->row_base,
+                                                              static_cast<int64_t*>(ctx->d_rows.p), static_cast<float*>(ctx->d_dist.p));
+    FX_CUDA(cudaGetLastError());
+    ctx->launches += 2; c->stats.kernel_launches += 2;   // (the sort: counted as one)
+  }
+  FX_CUDA(cudaEventRecord(ctx->ev_stop, ctx->stream));
+  FX_TRY(ctx->h_rows.ensure(size_t(total) * 8));
+  FX_TRY(ctx->h_dist.ensure(size_t(total) * 4));
+  FX_CUDA(cudaMemcpyAsync(ctx->h_rows.p, ctx->d_rows.p, size_t(total) * 8, cudaMemcpyDeviceToHost, ctx->stream));
+  FX_CUDA(cudaMemcpyAsync(ctx->h_dist.p, ctx->d_dist.p, size_t(total) * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  FX_CUDA(cudaStreamSynchronize(ctx->stream));
+  std::memcpy(out_rows, ctx->h_rows.p, size_t(total) * 8);
+  std::memcpy(out_dist, ctx->h_dist.p, size_t(total) * 4);
+  search_account(c, run);
   return FX_OK;
 }
 

@@ -266,6 +266,7 @@ struct TcSearch {
   int seeded;                // set by tc_prepare: this main pass starts from the sample prepass's thresholds (list quotas >= k, see tc_plan)
   int full_lists;            // 1: every candidate list keeps K' entries (re-run of starved queries: when a query's neighbours sit in
                              // ONE list - clustered rows in row order - a list that keeps fewer than k can never supply them)
+  int no_finish;             // 1: the filter only; the caller reads the candidate lists itself (range search, tc_finish_params)
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -1480,6 +1481,49 @@ struct FinishParams {
   int unit_q;       // 1: scores are cosine upper bounds of the NORMALISED query (int8 filter), not scaled by |q|
 };
 
+// Candidate list l of query tile qt, tile row r (the query's slot) - the layout every filter kernel writes: with the
+// resident-query kernel one list per slice (its unit holds two query tiles), else list l = (slice, half), the buffer of
+// thread slot half*128 + r of unit slice*n_qt + qt (or qt*n_slices + slice, query-tile-major order). count: its entries.
+__device__ __forceinline__ const uint2* fin_list(const FinishParams& p, int qt, int r, int l, int& count) {
+  size_t unit_slot;
+  if (p.rq) {
+    unit_slot = (size_t(l) * p.n_qp + (qt >> 1)) * TC_SLOTS + (qt & 1) * TC_BM + r;
+  } else {
+    const int slice = l / TC_SPLIT, half = l % TC_SPLIT;
+    const size_t unit = p.qt_major ? size_t(qt) * p.n_slices + slice : size_t(slice) * p.n_qt + qt;
+    unit_slot = unit * TC_SLOTS + half * TC_BM + r;
+  }
+  count = p.wcnt[unit_slot];
+  return p.wbuf + unit_slot * p.cap;
+}
+
+// THE summation order of every exact distance this library reports from 8-lane groups (the finish kernels here and
+// direct_scan.cuh, bit for bit): per lane one accumulator per float4 component over j = sub, sub + 8, ...; lane
+// total = (x + y) + (z + w); then the xor tree over the 8 lanes. Four independent chains per sum: the fp64 pipe's
+// latency, not its rate, bounded the single-chain form. Every lane of the warp calls it (the shuffles); xx = |x|^2 and
+// qx = <q, x> of the group's row come back in every lane of the group.
+__device__ __forceinline__ void rerank8(const float* X, int pitch, uint32_t row, bool live, const float* qs, int sub,
+                                        double& xx, double& qx) {
+  const float4* xp = reinterpret_cast<const float4*>(X + size_t(row) * pitch);
+  const int n4 = pitch >> 2;
+  double xa[4] = {0.0, 0.0, 0.0, 0.0}, qa[4] = {0.0, 0.0, 0.0, 0.0};
+#pragma unroll 4
+  for (int j = sub; j < n4; j += 8) {
+    const float4 xv = live ? __ldg(xp + j) : make_float4(0.f, 0.f, 0.f, 0.f);
+    const float4 qv = *reinterpret_cast<const float4*>(qs + 4 * j);
+    xa[0] = fma(double(xv.x), double(xv.x), xa[0]); qa[0] = fma(double(xv.x), double(qv.x), qa[0]);
+    xa[1] = fma(double(xv.y), double(xv.y), xa[1]); qa[1] = fma(double(xv.y), double(qv.y), qa[1]);
+    xa[2] = fma(double(xv.z), double(xv.z), xa[2]); qa[2] = fma(double(xv.z), double(qv.z), qa[2]);
+    xa[3] = fma(double(xv.w), double(xv.w), xa[3]); qa[3] = fma(double(xv.w), double(qv.w), qa[3]);
+  }
+  xx = (xa[0] + xa[1]) + (xa[2] + xa[3]); qx = (qa[0] + qa[1]) + (qa[2] + qa[3]);
+#pragma unroll
+  for (int o = 4; o > 0; o >>= 1) {
+    xx += __shfl_xor_sync(0xffffffffu, xx, o);
+    qx += __shfl_xor_sync(0xffffffffu, qx, o);
+  }
+}
+
 // One CTA per query. The query's candidates live in 2 * n_slices buffers (one per unit-half).
 //  1. block-wide radix select (4 passes of 8 bits over the ordered score bits) finds the K'-th best
 //     approximate score among the entries above the final shared threshold;
@@ -1518,19 +1562,7 @@ knn_tc_finish_kernel(FinishParams p) {
   const uint32_t tg = p.tau_g[q];
   const bool overflowed = p.flags[q] != 0;   // set by the filter kernel in refinement mode
 
-  // list l = (slice, half): buffer of thread slot half*128 + r of unit slice*n_qt + qt
-  auto list_ptr = [&](int l, int& count) -> const uint2* {
-    size_t unit_slot;
-    if (p.rq) {   // one list per slice; the unit holds two query tiles
-      unit_slot = (size_t(l) * p.n_qp + (qt >> 1)) * TC_SLOTS + (qt & 1) * TC_BM + r;
-    } else {
-      const int slice = l / TC_SPLIT, half = l % TC_SPLIT;
-      const size_t unit = p.qt_major ? size_t(qt) * p.n_slices + slice : size_t(slice) * p.n_qt + qt;
-      unit_slot = unit * TC_SLOTS + half * TC_BM + r;
-    }
-    count = p.wcnt[unit_slot];
-    return p.wbuf + unit_slot * p.cap;
-  };
+  auto list_ptr = [&](int l, int& count) -> const uint2* { return fin_list(p, qt, r, l, count); };
 
   // ---- 0. gather: one pass over the query's lists copies every entry at or above the final threshold into a
   // shared-memory pool, so the selection passes below never touch global memory again (with hundreds of short
@@ -1654,32 +1686,12 @@ knn_tc_finish_kernel(FinishParams p) {
   const double qq = s_qq;
   {
     const int sub = lane & 7, grp = lane >> 3;
-    const int n4 = p.pitch >> 2;
     for (int c0 = warp * 4; c0 < p.sort2; c0 += n_warps * 4) {
       const int c = c0 + grp;
       const bool live = c < n_gt || (!keep_all && c >= p.kp - n_tie_kept && c < p.kp);
       const uint32_t row = live ? cand[c] : 0u;
-      const float4* xp = reinterpret_cast<const float4*>(p.X + size_t(row) * p.pitch);
-      // THE summation order of every exact distance this library reports from 8-lane groups (here and in
-      // direct_scan.cuh, bit for bit): per lane one accumulator per float4 component over j = sub, sub + 8, ...; lane
-      // total = (x + y) + (z + w); then the xor tree over the 8 lanes. Four independent chains per sum: the fp64 pipe's
-      // latency, not its rate, bounded the single-chain form.
-      double xa[4] = {0.0, 0.0, 0.0, 0.0}, qa[4] = {0.0, 0.0, 0.0, 0.0};
-#pragma unroll 4
-      for (int j = sub; j < n4; j += 8) {
-        const float4 xv = live ? __ldg(xp + j) : make_float4(0.f, 0.f, 0.f, 0.f);
-        const float4 qv = *reinterpret_cast<const float4*>(qs + 4 * j);
-        xa[0] = fma(double(xv.x), double(xv.x), xa[0]); qa[0] = fma(double(xv.x), double(qv.x), qa[0]);
-        xa[1] = fma(double(xv.y), double(xv.y), xa[1]); qa[1] = fma(double(xv.y), double(qv.y), qa[1]);
-        xa[2] = fma(double(xv.z), double(xv.z), xa[2]); qa[2] = fma(double(xv.z), double(qv.z), qa[2]);
-        xa[3] = fma(double(xv.w), double(xv.w), xa[3]); qa[3] = fma(double(xv.w), double(qv.w), qa[3]);
-      }
-      double xx = (xa[0] + xa[1]) + (xa[2] + xa[3]), qx = (qa[0] + qa[1]) + (qa[2] + qa[3]);
-#pragma unroll
-      for (int o = 4; o > 0; o >>= 1) {
-        xx += __shfl_xor_sync(0xffffffffu, xx, o);
-        qx += __shfl_xor_sync(0xffffffffu, qx, o);
-      }
+      double xx, qx;
+      rerank8(p.X, p.pitch, row, live, qs, sub, xx, qx);
       if (sub == 0 && c < p.sort2) keys2[c] = live ? make_key(finish_distance(p.metric, qq, xx, qx), row) : KEY_PAD;
     }
   }
@@ -1775,6 +1787,30 @@ knn_tc_tau0_kernel(const float* __restrict__ pre_max, int n_q, int n_rec, int m,
   if (live && sub == 0) tau_g[q] = v > ORD_NEG_INF ? v : ORD_NEG_INF;
 }
 
+// Preset admission threshold (ordered encoding) for the rows at distance <= dk of a query with |q|^2 = qq: every such
+// row has exact score >= s(dk), hence filter score >= s(dk) - E (E: the error bound of the operand in use; unit_q: see
+// FinishParams). dk = +inf (or a non-finite result) admits everything.
+__device__ __forceinline__ uint32_t admission_threshold(int metric, double qq, double dk, float max_norm, double c_err,
+                                                        double c_add, int unit_q) {
+  const double nq = unit_q ? 1.0 : sqrt(qq), xm = double(max_norm);
+  dk = dk + 1e-6 * fabs(dk) + 1e-37;            // a row at distance <= dk (after fp32 rounding) must survive
+  double score, e_abs;
+  if (metric == 0) {
+    e_abs = c_err * nq * xm + c_add * (0.5 * xm * xm + nq * xm);
+    score = 0.5 * (qq - dk * dk);
+  } else if (metric == 1) {
+    e_abs = nq * (c_err + 1e-6);
+    score = (1.0 - 2.0 * dk) * (nq > 1e-12 ? nq : 1e-12);
+  } else {
+    e_abs = c_err * nq * xm;
+    score = -dk;
+  }
+  double t = score - e_abs;
+  t = t - 1e-6 * fabs(t) - 1e-30;
+  float tf = __double2float_rd(t);
+  return (t == t && dk < 1e300) ? f2ord(tf) : ORD_NEG_INF;
+}
+
 // Refinement of flagged queries. One block per flagged query i (original index qlist[i]): gathers the query
 // into Qr[i] and derives the preset admission threshold from the k-th distance d_k of the first pass:
 // every row that can still beat d_k has exact score > s(d_k), hence filter score > s(d_k) - E.
@@ -1796,26 +1832,22 @@ refine_prep_kernel(const float* __restrict__ Q, const int* __restrict__ qlist, i
   __syncthreads();
   if (threadIdx.x == 0) {
     const double qq = part[0] + part[1] + part[2] + part[3];
-    const double nq = unit_q ? 1.0 : sqrt(qq), xm = double(max_norm);   // unit_q: see FinishParams
-    double dk = double(dist[size_t(q) * k + (k - 1)]);
-    dk = dk + 1e-6 * fabs(dk) + 1e-37;            // a row at distance <= dk (after fp32 rounding) must survive
-    double score, e_abs;
-    if (metric == 0) {
-      e_abs = c_err * nq * xm + c_add * (0.5 * xm * xm + nq * xm);
-      score = 0.5 * (qq - dk * dk);
-    } else if (metric == 1) {
-      e_abs = nq * (c_err + 1e-6);
-      score = (1.0 - 2.0 * dk) * (nq > 1e-12 ? nq : 1e-12);
-    } else {
-      e_abs = c_err * nq * xm;
-      score = -dk;
-    }
-    double t = score - e_abs;
-    t = t - 1e-6 * fabs(t) - 1e-30;
-    float tf = __double2float_rd(t);
-    // fewer than k candidates in the first pass (dk = inf) or non-finite input: admit everything
-    tau_fixed[i] = (t == t && dk < 1e300) ? f2ord(tf) : ORD_NEG_INF;
+    tau_fixed[i] = admission_threshold(metric, qq, double(dist[size_t(q) * k + (k - 1)]), max_norm, c_err, c_add, unit_q);
   }
+}
+
+// Preset thresholds of a range search (fx_search_range): the same derivation from the radius, for every query.
+// One warp per query; the queries stay where they are.
+__global__ void __launch_bounds__(128)
+range_prep_kernel(const float* __restrict__ Q, int n_q, int dim, int metric, float radius, float max_norm, double c_err,
+                  double c_add, int unit_q, uint32_t* __restrict__ tau_fixed) {
+  const int q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+  if (q >= n_q) return;
+  double s = 0.0;
+  for (int d = lane; d < dim; d += 32) { const double v = double(Q[size_t(q) * dim + d]); s = fma(v, v, s); }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+  if (lane == 0) tau_fixed[q] = admission_threshold(metric, s, double(radius), max_norm, c_err, c_add, unit_q);
 }
 
 // Copy refined results of the queries whose certificate now holds back to their slots.
@@ -2344,11 +2376,28 @@ inline bool tc_prepass_config(const TcState* st, const TcSearch& s, const TcPlan
   return true;
 }
 
+// Where a pass over the plan `pl` left its padded queries, thresholds, flags and candidate lists in `scratch`, and what
+// the finish kernel does with them.
+inline FinishParams tc_finish_params(const TcSearch& s, const TcPlan& pl, void* scratch) {
+  char* base = static_cast<char*>(scratch);
+  FinishParams f{};
+  f.X = s.X; f.pitch = s.pitch; f.dim = s.dim; f.row_base = s.row_base; f.Qp = reinterpret_cast<float*>(base + pl.off_qp);
+  f.n_q = s.n_q; f.n_qt = pl.n_qt_lists;
+  f.n_flagged = reinterpret_cast<int*>(base);
+  f.n_slices = pl.n_slices; f.cap = pl.cap; f.metric = s.metric; f.k = s.k; f.kp = pl.kp;
+  int sort2 = 2; while (sort2 < pl.kp) sort2 <<= 1;
+  f.sort2 = sort2; f.tau_g = reinterpret_cast<uint32_t*>(base + pl.off_tau); f.wbuf = reinterpret_cast<uint2*>(base + pl.off_wbuf);
+  f.wcnt = reinterpret_cast<int*>(base + pl.off_wcnt); f.qt_major = pl.qt_major; f.rq = pl.rq; f.n_qp = pl.n_qp;
+  f.flags = reinterpret_cast<int*>(base + pl.off_flags); f.certify = s.certify ? 1 : 0;
+  f.max_norm = s.max_norm; tc_cert_consts(s, &f.c_err, &f.c_add); f.out_rows = s.out_rows; f.out_dist = s.out_dist;
+  f.unit_q = s.kind == 2 ? 1 : 0;
+  return f;
+}
+
 // One filter launch (+ finish) over the plan of `s`; queries / state have been prepared in `scratch` already.
 inline bool tc_run_pass(TcState* st, TcCorpus* tc, const TcSearch& s, const TcPlan& pl, void* scratch, const CUtensorMap& map_q,
                         std::string* err) {
   char* base = static_cast<char*>(scratch);
-  float* qp = reinterpret_cast<float*>(base + pl.off_qp);
   uint32_t* tau_g = reinterpret_cast<uint32_t*>(base + pl.off_tau);
   int* flags = reinterpret_cast<int*>(base + pl.off_flags);
   int* wcnt = reinterpret_cast<int*>(base + pl.off_wcnt);
@@ -2452,14 +2501,9 @@ inline bool tc_run_pass(TcState* st, TcCorpus* tc, const TcSearch& s, const TcPl
     return true;
   }
 
-  FinishParams f{};
-  f.X = s.X; f.pitch = s.pitch; f.dim = s.dim; f.row_base = s.row_base; f.Qp = qp; f.n_q = s.n_q; f.n_qt = pl.n_qt_lists;
-  f.n_flagged = reinterpret_cast<int*>(base);
-  f.n_slices = pl.n_slices; f.cap = pl.cap; f.metric = s.metric; f.k = s.k; f.kp = pl.kp;
-  int sort2 = 2; while (sort2 < pl.kp) sort2 <<= 1;
-  f.sort2 = sort2; f.tau_g = tau_g; f.wbuf = wbuf; f.wcnt = wcnt; f.qt_major = pl.qt_major; f.rq = pl.rq; f.n_qp = pl.n_qp; f.flags = flags; f.certify = s.certify ? 1 : 0;
-  f.max_norm = s.max_norm; tc_cert_consts(s, &f.c_err, &f.c_add); f.out_rows = s.out_rows; f.out_dist = s.out_dist;
-  f.unit_q = s.kind == 2 ? 1 : 0;
+  if (s.no_finish) return true;
+  const FinishParams f = tc_finish_params(s, pl, scratch);
+  const int sort2 = f.sort2;
   const size_t fin_smem = size_t(sort2) * 12 + size_t(s.pitch) * 4 + size_t(FIN_POOL) * 8 + 16;
   // many short lists per query (small batches split over all SMs): more warps sweep them in parallel
   // few lists, many candidates to rerank (K' >= 128: k = 100): 128-thread CTAs - more of them per SM cover the scattered

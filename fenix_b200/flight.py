@@ -189,10 +189,25 @@ class Flight:
                select: Sequence[str] | None = None, filter: pc.Expression | None = None,
                maxval: int | None = None, probes: int | None = None) -> pa.Table:
         assert metric in METRICS
-        command = pickle.dumps({
+        return self._exchange(target, {
             "coding": coding, "source": source, "column": column, "metric": metric, "select": select,
             "filter": pickle.dumps(filter), "maxval": maxval, "probes": probes,
         })
+
+    def search_range(self, target, source: str | Sequence[str], column: str, metric: str, radius: float,
+                     select: Sequence[str] | None = None, filter: pc.Expression | None = None,
+                     maxval: int | None = None) -> pa.Table:
+        """Every row within `radius` of the target (distance <= radius), ordered by (distance, row); with `maxval`, at
+        most that many, nearest first. The command is `search`'s plus a "radius" key, so requests without one stay
+        byte-identical to the reference client's."""
+        assert metric in METRICS
+        return self._exchange(target, {
+            "coding": None, "source": source, "column": column, "metric": metric, "select": select,
+            "filter": pickle.dumps(filter), "maxval": maxval, "probes": None, "radius": float(radius),
+        })
+
+    def _exchange(self, target, config: dict) -> pa.Table:
+        command = pickle.dumps(config)
         if type(target).__module__.startswith("torch"):
             target = target.numpy()
         if isinstance(target, np.ndarray):

@@ -176,9 +176,18 @@ def call(
     maxval: int | None = None,
     probes: int | None = None,
     precision: int = knn.PREC_FP32,
+    radius: float | None = None,
 ) -> pa.Table:
+    """`radius` (this build's extension): every row within that distance of the target, ordered by (distance, row); with
+    `maxval` as well, at most maxval of them (the exact k-NN, rows beyond the radius dropped)."""
     if metric is not None:
         knn.metric_code(metric)  # ValueError on unknown names, as coder.py:50
+    if radius is not None:
+        radius = float(radius)
+        if radius != radius:
+            raise ValueError("radius is NaN")
+        if coding is not None or probes is not None:
+            raise NotImplementedError("range search (radius) over an IVF coding is not supported")
     if isinstance(source, pa.Table):
         data = source
         shard = _shards.from_chunks(data.column(column))
@@ -207,6 +216,8 @@ def call(
 
         out_cols = [*select] if select is not None else data.column_names
         mask = _row_mask(data, column, filter) if filter is not None else None
+        if radius is not None:
+            return _range(shard, data, out_cols, typ, queries, batched, metric, radius, maxval, mask, precision)
 
         if probe_codes is not None and batched:
             # Batched IVF: every query has its own probe cells, i.e. its own row mask (index.py:113-126 per query).
@@ -296,6 +307,31 @@ def call(
             shard.close()
         else:
             shard.release()   # the lease taken by shards.get
+
+
+def _range(shard, data: pa.Table, out_cols, typ, queries: np.ndarray, batched: bool, metric: str, radius: float, maxval,
+           mask, precision) -> pa.Table:
+    """Rows within `radius` of each query, ordered by (distance, row): the range search, or with `maxval` the exact k-NN
+    (k = min(maxval, surviving rows)) cut at the radius."""
+    n_q = queries.shape[0]
+    if maxval is None:
+        offsets, rows, dist = shard.search_range(queries, metric, radius, precision, mask)
+        qid = np.repeat(np.arange(n_q, dtype=np.int32), np.diff(offsets))
+    else:
+        n_live = int(mask.sum()) if mask is not None else data.num_rows
+        k = min(int(maxval), n_live)
+        if k < 1:
+            rows, dist, qid = np.zeros(0, np.int64), np.zeros(0, np.float32), np.zeros(0, np.int32)
+        else:
+            r, d = shard.search(queries, metric, k, precision, mask)
+            keep = (r >= 0) & (d <= np.float32(radius))   # the radius as the library sees it (one float32)
+            rows, dist = r[keep], d[keep]
+            qid = np.repeat(np.arange(n_q, dtype=np.int32), k).reshape(n_q, k)[keep]
+    out = take_rows(data, out_cols, rows)
+    out = out.append_column(DIST_COL, _distance_array(dist, typ.value_type))
+    if batched:
+        out = out.append_column(QUERY_COL, pa.array(qid, type=pa.int32()))
+    return out.combine_chunks()
 
 
 def _cells_key(root: str, coding: str, source, column: str) -> tuple:

@@ -144,6 +144,26 @@ class ShardSet:
         # inside the library), the k x W candidates are all-gathered over NVLink and merged on the device
         return self.group.search(self.corpora, queries, metric, k, precision, row_mask)
 
+    def search_range(self, queries: np.ndarray, metric: str, radius: float, precision: int = knn.PREC_FP32,
+                     row_mask: Optional[np.ndarray] = None) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """Every row within `radius` of each query: (offsets[Q + 1], rows, dist) in CSR form, each query's hits ordered
+        by (distance, row). Several devices: each shard in turn (as `distances`), the lists merged on the host."""
+        if len(self.corpora) == 1:
+            return self.corpora[0].search_range(queries, metric, radius, precision, row_mask)
+        n_q = np.atleast_2d(np.asarray(queries)).shape[0]
+        qids, rows, dists = [], [], []
+        for c, base in zip(self.corpora, self.bases):
+            part_mask = None if row_mask is None else row_mask[base: base + c.n_rows]
+            off, r, d = c.search_range(queries, metric, radius, precision, part_mask)
+            qids.append(np.repeat(np.arange(n_q, dtype=np.int64), np.diff(off)))
+            rows.append(r)
+            dists.append(d)
+        qid, row, dist = np.concatenate(qids), np.concatenate(rows), np.concatenate(dists)
+        order = np.lexsort((row, dist, qid))
+        offsets = np.zeros(n_q + 1, dtype=np.int64)
+        np.cumsum(np.bincount(qid, minlength=n_q), out=offsets[1:])
+        return offsets, row[order], dist[order]
+
     def distances(self, query: np.ndarray, metric: str) -> np.ndarray:
         parts = [c.distances(query, metric) for c in self.corpora]
         return parts[0] if len(parts) == 1 else np.concatenate(parts)

@@ -25,10 +25,11 @@ __all__ = [
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB_NAME = "libfenix_knn.so"
 COMM_ID_BYTES = 128
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 FX_OK = 0
 FX_EINVAL, FX_ECUDA, FX_ENOMEM, FX_ESTATE, FX_EUNSUP = -1, -2, -3, -4, -5
+FX_ETRUNC = -6   # fx_search_range: output capacity too small, out_offsets holds the sizes needed
 PREC_FP32, PREC_TF32, PREC_BF16, PREC_EXACT_SCAN = 0, 1, 2, 3
 
 # the five names accepted by the reference (flight.py:254, coder.py:39,42,47) -> 3 forms
@@ -41,7 +42,7 @@ ABI_SYMBOLS = (
     "fx_merge_topk", "fx_get_stats", "fx_debug_scores", "fx_last_error", "fx_abi_version", "fx_set_option",
     "fx_comm_unique_id", "fx_comm_init_rank", "fx_comm_destroy", "fx_search_sharded", "fx_search_sharded_device",
     "fx_group_create", "fx_group_size", "fx_group_ctx", "fx_group_search", "fx_group_destroy",
-    "fx_corpus_set_cells", "fx_search_cells",
+    "fx_corpus_set_cells", "fx_search_cells", "fx_search_range",
 )
 
 
@@ -143,6 +144,7 @@ def load_library() -> ctypes.CDLL:
         lib.fx_group_destroy.argtypes = [vp]
         lib.fx_corpus_set_cells.argtypes = [vp, vp, i64, vp, i64]
         lib.fx_search_cells.argtypes = [vp, vp, i64, i32, i32, vp, i32, vp, vp, vp]
+        lib.fx_search_range.argtypes = [vp, vp, i64, i32, ctypes.c_float, i32, vp, i64, vp, vp, vp]
         for name in ABI_SYMBOLS:
             fn = getattr(lib, name)
             if name not in ("fx_last_error", "fx_group_ctx"):
@@ -306,6 +308,47 @@ class Corpus:
         _check(self._lib, self._lib.fx_search(self._h, q.ctypes.data, n_q, m, k, int(precision), mask_ptr,
                                               out_rows.ctypes.data, out_dist.ctypes.data))
         return out_rows, out_dist
+
+    def search_range(self, queries: np.ndarray, metric: str | int, radius: float, precision: int = PREC_FP32,
+                     row_mask: Optional[np.ndarray] = None,
+                     capacity: Optional[int] = None) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """Every row within `radius` of each query (distance <= radius, inclusive). Returns (offsets[int64, Q + 1],
+        rows[int64], dist[float32]) in CSR form: query q's hits are rows[offsets[q]:offsets[q + 1]], ordered by
+        (distance, row). `precision` is PREC_FP32 or PREC_EXACT_SCAN (the result is exact either way).
+
+        The result size is unknown before the search: the first call uses `capacity` (default: 64 hits per query) and,
+        when the hits do not fit, the library reports the sizes needed and the search runs a SECOND time into buffers
+        of that size."""
+        m = metric if isinstance(metric, int) else metric_code(metric)
+        radius = float(radius)
+        if radius != radius:
+            raise ValueError("radius is NaN")
+        q = np.asarray(queries)
+        if q.ndim == 1:
+            q = q.reshape(1, -1)
+        if q.ndim != 2 or q.shape[1] != self.dim:
+            raise ValueError(f"expected queries of shape (*, {self.dim}), got {q.shape}")
+        q = np.ascontiguousarray(q, dtype=np.float32)
+        n_q = q.shape[0]
+        mask_ptr = None
+        if row_mask is not None:
+            row_mask = np.ascontiguousarray(row_mask, dtype=np.uint8)
+            if row_mask.shape != (self.n_rows,):
+                raise ValueError(f"row_mask must have shape ({self.n_rows},), got {row_mask.shape}")
+            mask_ptr = row_mask.ctypes.data
+        offsets = np.zeros(n_q + 1, dtype=np.int64)
+        cap = 64 * n_q if capacity is None else int(capacity)
+        for attempt in range(2):
+            rows = np.empty(cap, dtype=np.int64)
+            dist = np.empty(cap, dtype=np.float32)
+            code = self._lib.fx_search_range(self._h, q.ctypes.data, n_q, m, radius, int(precision), mask_ptr, cap,
+                                             offsets.ctypes.data, rows.ctypes.data, dist.ctypes.data)
+            if code != FX_ETRUNC or attempt == 1:
+                break
+            cap = int(offsets[-1])   # the sizes the first search reported
+        _check(self._lib, code)
+        total = int(offsets[-1])
+        return offsets, rows[:total], dist[:total]
 
     def search_raw(self, q_ptr: int, n_q: int, metric: int, k: int, precision: int,
                    out_rows_ptr: int, out_dist_ptr: int, mask_ptr: Optional[int] = None) -> None:

@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define FX_ABI_VERSION 5
+#define FX_ABI_VERSION 6
 
 /* error codes */
 #define FX_OK 0
@@ -42,6 +42,7 @@ extern "C" {
 #define FX_ENOMEM (-3)   /* host or device allocation failed */
 #define FX_ESTATE (-4)   /* call not valid in this state (append after finalize, search before) */
 #define FX_EUNSUP (-5)   /* valid request this build does not support (dtype, huge dim) */
+#define FX_ETRUNC (-6)   /* output capacity too small: out_offsets holds the sizes needed (fx_search_range) */
 
 /* metrics: the five reference names map to three arithmetic forms (coder.py:39,42,47) */
 #define FX_METRIC_L2 0     /* "l2", "euclidean" */
@@ -176,6 +177,21 @@ int fx_search_cells(fx_corpus* c, const float* queries, int64_t n_q, int32_t met
  * out_dist[n_rows]). This is the `maxval is None or len(data) <= maxval` branch of
  * index.py:162-165, where the reference returns all rows with __DISTANCE__ attached. */
 int fx_distances(fx_corpus* c, const float* query, int32_t metric, float* out_dist);
+
+/* Range search: every shard row r (after row_mask) with distance d(q, r) <= radius, for each of `n_q` queries (HOST,
+ * row-major n_q x dim floats). d is the distance fx_distances reports for the row; the comparison is inclusive; a
+ * query's hits are ordered by (distance, row), rows global (row_base + local). radius: one float per call, NaN is
+ * FX_EINVAL, negative values are valid (inner-product distances can be negative), +inf admits every unmasked row.
+ * Output in CSR form (HOST): query q's hits are out_rows / out_dist [out_offsets[q], out_offsets[q + 1]).
+ * out_offsets [n_q + 1] is always written; when out_offsets[n_q] > capacity the call returns FX_ETRUNC and leaves
+ * out_rows / out_dist untouched, so the caller can size its buffers and call again (a second search).
+ * precision: FX_PREC_FP32 (the tensor-core filter with thresholds preset from the radius, every candidate reranked in
+ * fp64; queries whose candidate lists overflow, and shards the tensor-core path does not take, run on the exact scan) or
+ * FX_PREC_EXACT_SCAN; TF32 / BF16 are FX_EUNSUP. fx_stats: last_path / last_operand name the filter that ran,
+ * fallback_queries counts the queries whose candidate lists overflowed and the scan settled, last_search_ms is the
+ * device time of the search. */
+int fx_search_range(fx_corpus* c, const float* queries, int64_t n_q, int32_t metric, float radius, int32_t precision,
+                    const uint8_t* row_mask, int64_t capacity, int64_t* out_offsets, int64_t* out_rows, float* out_dist);
 
 /* Merge `n_lists` per-shard results (DEVICE, each [n_q*k], laid out list-major:
  * rows[l*n_q*k + q*k + j]) into the global top-k ordered by (distance, row).
