@@ -918,10 +918,11 @@ static int search_settle(fx_corpus* c, SearchRun* run, bool* changed) {
     int64_t* rows2 = reinterpret_cast<int64_t*>(rb + o_rows);
     float* dist2 = reinterpret_cast<float*>(rb + o_dist);
     // gathers the flagged queries (and derives the preset thresholds tier 1 uses)
-    double c_err = 0.0, c_add = 0.0;
-    fx::tc_cert_consts(s, &c_err, &c_add);
+    double c_err = 0.0, c_add = 0.0, c_abs = 0.0;
+    fx::tc_cert_consts(s, &c_err, &c_add, &c_abs);
     fx::refine_prep_kernel<<<n_f, 128, 0, ctx->stream>>>(d_q, static_cast<const int*>(ctx->d_qlist.p), c->dim, metric, k,
-                                                        d_out_dist, c->max_norm, c_err, c_add, q_r, tau_fixed, s.kind == 2 ? 1 : 0);
+                                                        d_out_dist, c->max_norm, c_err, c_add, c_abs, q_r, tau_fixed,
+                                                        s.kind == 2 ? 1 : 0);
     FX_CUDA(cudaGetLastError());
     fx::TcSearch s2 = s;
     s2.Q = q_r; s2.n_q = n_f; s2.out_rows = rows2; s2.out_dist = dist2; s2.certify = true;
@@ -1518,10 +1519,10 @@ extern "C" int fx_search_range(fx_corpus* c, const float* queries, int64_t n_q, 
                              ((metric == 1 && ensure_norm_shadow(c)) || ensure_plain_shadow(c));
     const int kind = have_i8 ? 2 : (have_shadow ? 1 : 0);
     FX_TRY(configure_filter(c, metric, kind, d_mask, &s));
-    double c_err = 0.0, c_add = 0.0;
-    fx::tc_cert_consts(s, &c_err, &c_add);
+    double c_err = 0.0, c_add = 0.0, c_abs = 0.0;
+    fx::tc_cert_consts(s, &c_err, &c_add, &c_abs);
     fx::range_prep_kernel<<<int((n_q + 3) / 4), 128, 0, ctx->stream>>>(d_q, int(n_q), c->dim, metric, radius, c->max_norm,
-                                                                       c_err, c_add, kind == 2 ? 1 : 0, d_tau);
+                                                                       c_err, c_add, c_abs, kind == 2 ? 1 : 0, d_tau);
     FX_CUDA(cudaGetLastError());
     const fx::TcLaunch L = fx::tc_prepare(&ctx->tc, s);
     FX_TRY(ctx->d_tc.ensure(L.scratch_bytes));

@@ -17,7 +17,7 @@
 namespace fx {
 
 // Candidate count of every query (one warp each): the sum of its lists' entry counts, or -1 when a list overflowed
-// (the filter flagged the query; the scan settles it).
+// (the filter flagged the query) or its threshold is ORD_SCAN (the filter's scores are not bounded): the scan settles it.
 __global__ void __launch_bounds__(256)
 range_count_kernel(FinishParams p, int64_t* __restrict__ cand) {
   const int q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
@@ -29,12 +29,12 @@ range_count_kernel(FinishParams p, int64_t* __restrict__ cand) {
   for (int l = lane; l < n_lists; l += 32) { int count; fin_list(p, qt, r, l, count); s += count; }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-  if (lane == 0) cand[q] = p.flags[q] != 0 ? int64_t(-1) : s;
+  if (lane == 0) cand[q] = (p.flags[q] != 0 || p.tau_g[q] == ORD_SCAN) ? int64_t(-1) : s;
 }
 
 // One CTA per query: every candidate of its lists is reranked exactly (8 lanes per candidate, as the k-NN finish kernel)
 // and kept when its distance is <= radius. keys[seg[q] ...]: the hits in no particular order; hits[q]: their number.
-// Flagged queries (overflowed lists) are skipped.
+// Queries the count kernel sent to the scan are skipped.
 __global__ void __launch_bounds__(256)
 range_finish_kernel(FinishParams p, float radius, const int64_t* __restrict__ seg, uint64_t* __restrict__ keys,
                     int* __restrict__ hits) {
@@ -44,7 +44,7 @@ range_finish_kernel(FinishParams p, float radius, const int64_t* __restrict__ se
   __shared__ double s_qq;
   const int q = blockIdx.x;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, n_warps = blockDim.x >> 5;
-  if (p.flags[q] != 0) {
+  if (p.flags[q] != 0 || p.tau_g[q] == ORD_SCAN) {
     if (tid == 0) hits[q] = 0;
     return;
   }

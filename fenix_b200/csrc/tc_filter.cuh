@@ -81,6 +81,9 @@ static_assert(TC3_FIXED_BYTES + 9 * TC_A_BYTES + TC3_MIN_STAGES * TC2_B_BYTES <=
 constexpr size_t TC_HDR_BYTES = 256;        // scratch header (word 0: flagged-query counter of the last finish launch)
 constexpr int TC_MAX_WAVES = 4;            // units per CTA at most (bounds the candidate-buffer scratch)
 constexpr uint32_t ORD_NEG_INF = 0x007fffffu;  // f2ord(-inf)
+// Preset threshold of a query the filter cannot settle (admission_threshold): below every ordered float (a NaN as a
+// float, so the float epilogues admit nothing); the range search sends such queries to the exact scan.
+constexpr uint32_t ORD_SCAN = 0u;
 
 // Geometry of a bf16 shadow of a [n][dim] shard (see to_bf16_tiled_kernel). The four augmented columns - three terms
 // of -|x|^2/2 and the row's error weight |x| - sit right after the data when the last 64-column k-block has room for
@@ -1475,7 +1478,7 @@ struct FinishParams {
   const float* X; int pitch; int dim; int64_t row_base;
   const float* Qp; int n_q; int n_qt; int n_slices; int cap; int metric; int k; int kp; int sort2;  // sort2: pow2 >= kp
   const uint32_t* tau_g; const uint2* wbuf; const int* wcnt; int qt_major; int rq; int n_qp;
-  int* flags; int certify; float max_norm; double c_err; double c_add;
+  int* flags; int certify; float max_norm; double c_err; double c_add; double c_abs;
   int64_t* out_rows; float* out_dist;
   int* n_flagged;   // counts the queries this launch flags (read back by the host together with the results)
   int unit_q;       // 1: scores are cosine upper bounds of the NORMALISED query (int8 filter), not scaled by |q|
@@ -1522,6 +1525,27 @@ __device__ __forceinline__ void rerank8(const float* X, int pitch, uint32_t row,
     xx += __shfl_xor_sync(0xffffffffu, xx, o);
     qx += __shfl_xor_sync(0xffffffffu, qx, o);
   }
+}
+
+// Error bound E of a query's filter scores (score units; nq = |q|, or 1 with unit_q; xm = the shard's max |x|), shared by
+// the certificate and the preset thresholds. c_err / c_add: the relative bounds (0 where the score already is an upper
+// bound); c_abs: products and partial sums below FLT_MIN, which the tensor cores may lose (tc_c_abs), multiplied for
+// cosine by the epilogue's row factor 1/max(|x|, 1e-12) <= 1e12. NaN when a product or partial sum of the filter could
+// overflow fp32 (|q| |x| + |x|^2/2 near FLT_MAX): its score may then be +-inf or NaN, which no threshold bounds.
+__device__ __forceinline__ double score_error(int metric, double nq, double xm, double c_err, double c_add, double c_abs,
+                                              int unit_q) {
+  double e_abs, span;
+  if (metric == 0) {
+    e_abs = c_err * nq * xm + c_add * (0.5 * xm * xm + nq * xm) + c_abs;
+    span = nq * xm + 0.5 * xm * xm;
+  } else if (metric == 1) {
+    e_abs = nq * (c_err + 1e-6) + c_abs * 1e12;
+    span = nq * fmax(xm, 1.0);
+  } else {
+    e_abs = c_err * nq * xm + c_abs;
+    span = nq * xm;
+  }
+  return (unit_q || span < 0x1p126) ? e_abs : __longlong_as_double(0x7ff8000000000000ll);
 }
 
 // One CTA per query. The query's candidates live in 2 * n_slices buffers (one per unit-half).
@@ -1721,17 +1745,14 @@ knn_tc_finish_kernel(FinishParams p) {
       // every row that is not a candidate has approximate score <= T
       const float t_score = ord2f(pivot);
       const double nq = p.unit_q ? 1.0 : sqrt(qq);
-      const double xm = double(p.max_norm);
-      double e_abs, lb;
+      const double e_abs = score_error(p.metric, nq, double(p.max_norm), p.c_err, p.c_add, p.c_abs, p.unit_q);
+      double lb;
       if (p.metric == 0) {
-        e_abs = p.c_err * nq * xm + p.c_add * (0.5 * xm * xm + nq * xm);
         double d2 = qq - 2.0 * (double(t_score) + e_abs);
-        lb = sqrt(d2 > 0.0 ? d2 : 0.0);
+        lb = sqrt(d2 > 0.0 ? d2 : 0.0);   // (a NaN bound clamps to 0: no distance is below it)
       } else if (p.metric == 1) {
-        e_abs = nq * (p.c_err + 1e-6);
         lb = 0.5 - 0.5 * (double(t_score) + e_abs) / (nq > 1e-12 ? nq : 1e-12);
       } else {
-        e_abs = p.c_err * nq * xm;
         lb = -(double(t_score) + e_abs);
       }
       lb = lb - 1e-6 * fabs(lb) - 1e-37;
@@ -1788,27 +1809,21 @@ knn_tc_tau0_kernel(const float* __restrict__ pre_max, int n_q, int n_rec, int m,
 }
 
 // Preset admission threshold (ordered encoding) for the rows at distance <= dk of a query with |q|^2 = qq: every such
-// row has exact score >= s(dk), hence filter score >= s(dk) - E (E: the error bound of the operand in use; unit_q: see
-// FinishParams). dk = +inf (or a non-finite result) admits everything.
+// row has exact score >= s(dk), hence filter score >= s(dk) - E (E: score_error of the operand in use; unit_q: see
+// FinishParams). dk = +inf admits everything; ORD_SCAN when E is undefined (the filter's sums could overflow).
 __device__ __forceinline__ uint32_t admission_threshold(int metric, double qq, double dk, float max_norm, double c_err,
-                                                        double c_add, int unit_q) {
-  const double nq = unit_q ? 1.0 : sqrt(qq), xm = double(max_norm);
+                                                        double c_add, double c_abs, int unit_q) {
+  const double nq = unit_q ? 1.0 : sqrt(qq);
+  const double e_abs = score_error(metric, nq, double(max_norm), c_err, c_add, c_abs, unit_q);
   dk = dk + 1e-6 * fabs(dk) + 1e-37;            // a row at distance <= dk (after fp32 rounding) must survive
-  double score, e_abs;
-  if (metric == 0) {
-    e_abs = c_err * nq * xm + c_add * (0.5 * xm * xm + nq * xm);
-    score = 0.5 * (qq - dk * dk);
-  } else if (metric == 1) {
-    e_abs = nq * (c_err + 1e-6);
-    score = (1.0 - 2.0 * dk) * (nq > 1e-12 ? nq : 1e-12);
-  } else {
-    e_abs = c_err * nq * xm;
-    score = -dk;
-  }
+  double score;
+  if (metric == 0) score = 0.5 * (qq - dk * dk);
+  else if (metric == 1) score = (1.0 - 2.0 * dk) * (nq > 1e-12 ? nq : 1e-12);
+  else score = -dk;
   double t = score - e_abs;
   t = t - 1e-6 * fabs(t) - 1e-30;
   float tf = __double2float_rd(t);
-  return (t == t && dk < 1e300) ? f2ord(tf) : ORD_NEG_INF;
+  return t != t ? ORD_SCAN : (dk < 1e300 ? f2ord(tf) : ORD_NEG_INF);
 }
 
 // Refinement of flagged queries. One block per flagged query i (original index qlist[i]): gathers the query
@@ -1816,7 +1831,7 @@ __device__ __forceinline__ uint32_t admission_threshold(int metric, double qq, d
 // every row that can still beat d_k has exact score > s(d_k), hence filter score > s(d_k) - E.
 __global__ void __launch_bounds__(128)
 refine_prep_kernel(const float* __restrict__ Q, const int* __restrict__ qlist, int dim, int metric, int k,
-                   const float* __restrict__ dist, float max_norm, double c_err, double c_add,
+                   const float* __restrict__ dist, float max_norm, double c_err, double c_add, double c_abs,
                    float* __restrict__ Qr, uint32_t* __restrict__ tau_fixed, int unit_q) {
   __shared__ double part[4];
   const int i = blockIdx.x, q = qlist[i];
@@ -1832,7 +1847,7 @@ refine_prep_kernel(const float* __restrict__ Q, const int* __restrict__ qlist, i
   __syncthreads();
   if (threadIdx.x == 0) {
     const double qq = part[0] + part[1] + part[2] + part[3];
-    tau_fixed[i] = admission_threshold(metric, qq, double(dist[size_t(q) * k + (k - 1)]), max_norm, c_err, c_add, unit_q);
+    tau_fixed[i] = admission_threshold(metric, qq, double(dist[size_t(q) * k + (k - 1)]), max_norm, c_err, c_add, c_abs, unit_q);
   }
 }
 
@@ -1840,14 +1855,14 @@ refine_prep_kernel(const float* __restrict__ Q, const int* __restrict__ qlist, i
 // One warp per query; the queries stay where they are.
 __global__ void __launch_bounds__(128)
 range_prep_kernel(const float* __restrict__ Q, int n_q, int dim, int metric, float radius, float max_norm, double c_err,
-                  double c_add, int unit_q, uint32_t* __restrict__ tau_fixed) {
+                  double c_add, double c_abs, int unit_q, uint32_t* __restrict__ tau_fixed) {
   const int q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (q >= n_q) return;
   double s = 0.0;
   for (int d = lane; d < dim; d += 32) { const double v = double(Q[size_t(q) * dim + d]); s = fma(v, v, s); }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-  if (lane == 0) tau_fixed[q] = admission_threshold(metric, s, double(radius), max_norm, c_err, c_add, unit_q);
+  if (lane == 0) tau_fixed[q] = admission_threshold(metric, s, double(radius), max_norm, c_err, c_add, c_abs, unit_q);
 }
 
 // Copy refined results of the queries whose certificate now holds back to their slots.
@@ -2103,8 +2118,9 @@ inline bool tc_bind_corpus(TcState* st, TcCorpus* tc, const float* X, int64_t n_
 // K' (candidates kept by each selection) and the buffer capacity that goes with it
 constexpr int TC_KP_I8 = 256;   // int8 filter, k <= 16: rows above the k-th exact cosine that the bound lets through (K' sweep)
 inline int tc_kp(int k, bool certify, int kind = 0) {
-  // slack so that the certificate holds for (nearly) every query in one pass: the bf16 bound is ~1.8x looser than
-  // the TF32 one (measured on C3: K' = 32 flags 25 of 4096 queries per batch with bf16, K' = 64 none); the int8 bound
+  // slack so that the certificate holds for (nearly) every query in one pass: the bf16 bound is ~3.5x looser than
+  // the TF32 one (2^-7 against 1.25 2^-9 per product; K' was measured on C3 when the bf16 constant was half its present,
+  // correct value: K' = 32 flagged 25 of 4096 queries per batch with bf16, K' = 64 none); the int8 bound
   // (~0.02 in cosine units at D = 768) needs a few hundred rows, see TC_KP_I8
   if (kind == 2) return certify ? std::max(TC_KP_I8, (k + k / 2 + 31) & ~31) : ((k + 31) & ~31);
   int kp = certify ? k + std::max(kind == 1 ? 48 : 16, k / 2) : k;
@@ -2302,12 +2318,13 @@ inline const int* tc_flag_count(void* scratch) { return static_cast<const int*>(
 // rigorous bound constant of the TF32 dot product: |acc - <q,x>| <= c * |q| * |x|
 // (operands truncated to 10 mantissa bits: 2^-10 each -> 2^-9 on the product, 25% margin;
 //  fp32 accumulation of D terms: D * 2^-21)
-// bf16 operands are rounded to nearest (2^-9 each -> 2^-8 on the product, 10% margin).
+// bf16 operands are rounded to nearest: 8 significant bits, so up to 2^-8 relative each -> 2^-7 on the product, 10%
+// margin (tests/test_gpu_exactness_edges.py plants rows that reach 0.9 of it).
 // L2 only: rounding of the -|x|^2/2 term and of its addition, relative to |x|^2/2 + |q||x|. When the term rides
 // through the MMA (augmented shadow) every one of the tile's accumulation steps may round it again.
 inline double tc_c_add(int dim, bool aug) { return 4.8e-7 + (aug ? double((dim + TC_AUG_COLS + 15) / 16) * 1.2e-7 : 0.0); }
 inline double tc_c_err(int dim, int kind = 0) {
-  const double prod = kind == 0 ? 1.25 * std::ldexp(1.0, -9) : 1.10 * std::ldexp(1.0, -8);
+  const double prod = kind == 0 ? 1.25 * std::ldexp(1.0, -9) : 1.10 * std::ldexp(1.0, -7);
   return prod + double(dim) * std::ldexp(1.0, -21);
 }
 
@@ -2315,7 +2332,13 @@ inline double tc_c_err(int dim, int kind = 0) {
 // score already carries c |q| |x| per row plus the folded |x|^2/2 allowance - it IS an upper bound of the exact score -
 // so nothing is added on top and the certificate no longer depends on the largest norm of the shard: one 100x-norm
 // outlier (or clustered rows far from the origin) inflates only its own row's score.
-inline void tc_cert_consts(const TcSearch& s, double* c_err, double* c_add) {
+// Absolute term of the TF32 / bf16 bounds: every product and every partial sum of the MMA (data and augmented columns)
+// that falls below FLT_MIN loses less than 2^-126, whether the tensor cores keep subnormals or flush them, and the
+// relative terms above do not cover that loss on rows of tiny magnitude (tests/test_gpu_exactness_edges.py).
+inline double tc_c_abs(int dim) { return 2.0 * double(dim + TC_AUG_COLS + 4) * std::ldexp(1.0, -126); }
+// The int8 filter's scores are exact integer sums, converted once and rounded up: no absolute term.
+inline void tc_cert_consts(const TcSearch& s, double* c_err, double* c_add, double* c_abs) {
+  *c_abs = s.kind == 2 ? 0.0 : tc_c_abs(s.dim);
   if ((s.kind == 1 && s.aug != 0) || s.kind == 2) { *c_err = 0.0; *c_add = 0.0; return; }
   *c_err = tc_c_err(s.dim, s.kind);
   *c_add = tc_c_add(s.dim, false);
@@ -2389,7 +2412,7 @@ inline FinishParams tc_finish_params(const TcSearch& s, const TcPlan& pl, void* 
   f.sort2 = sort2; f.tau_g = reinterpret_cast<uint32_t*>(base + pl.off_tau); f.wbuf = reinterpret_cast<uint2*>(base + pl.off_wbuf);
   f.wcnt = reinterpret_cast<int*>(base + pl.off_wcnt); f.qt_major = pl.qt_major; f.rq = pl.rq; f.n_qp = pl.n_qp;
   f.flags = reinterpret_cast<int*>(base + pl.off_flags); f.certify = s.certify ? 1 : 0;
-  f.max_norm = s.max_norm; tc_cert_consts(s, &f.c_err, &f.c_add); f.out_rows = s.out_rows; f.out_dist = s.out_dist;
+  f.max_norm = s.max_norm; tc_cert_consts(s, &f.c_err, &f.c_add, &f.c_abs); f.out_rows = s.out_rows; f.out_dist = s.out_dist;
   f.unit_q = s.kind == 2 ? 1 : 0;
   return f;
 }

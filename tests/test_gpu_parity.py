@@ -865,7 +865,7 @@ def test_tf32_error_bound_of_the_certificate(ctx, dim):
 @pytest.mark.parametrize("dim", [64, 768])
 def test_bf16_shadow_filter_is_exact_in_fp32_mode(ctx, dim, monkeypatch):
     """With a bf16 shadow the exact mode filters with kind::f16 MMAs; results must not change, and the bf16
-    error bound c = 1.1 * 2^-8 + D * 2^-21 must hold for the raw scores."""
+    error bound c = 1.1 * 2^-7 + D * 2^-21 must hold for the raw scores (Gaussian rows use less than 0.3 of it)."""
     monkeypatch.setenv("FENIX_BF16_SHADOW", "1")
     rng = np.random.default_rng(dim + 5)
     corpus = rng.standard_normal((20000, dim), dtype=np.float32)
@@ -877,8 +877,8 @@ def test_bf16_shadow_filter_is_exact_in_fp32_mode(ctx, dim, monkeypatch):
     finally:
         ctx.set_option("FENIX_DEBUG_BF16", None)
     q, x = queries[:128].astype(np.float64), corpus[:256].astype(np.float64)
-    bound = (1.1 * 2.0 ** -8 + dim * 2.0 ** -21) * np.linalg.norm(q, axis=1)[:, None] * np.linalg.norm(x, axis=1)[None, :]
-    assert (np.abs(s - q @ x.T) / bound).max() < 0.6
+    bound = (1.1 * 2.0 ** -7 + dim * 2.0 ** -21) * np.linalg.norm(q, axis=1)[:, None] * np.linalg.norm(x, axis=1)[None, :]
+    assert (np.abs(s - q @ x.T) / bound).max() < 0.3
     for metric in ("l2", "cosine", "dot"):
         rows, dist = c.search(queries, metric, 10, knn.PREC_FP32)
         assert c.stats().last_path == 2   # bf16 filter
