@@ -17,7 +17,7 @@ PKG = os.path.dirname(HERE)
 ROOT = os.path.dirname(PKG)
 OUT = os.environ.get("FENIX_BUILD_OUT") or os.path.join(PKG, "libfenix_knn.so")   # FENIX_BUILD_OUT: tuning variants
 SOURCES = ["fenix_knn.cu"]
-DEPS = ["fenix_knn.cu", "common.cuh", "exact_scan.cuh", "direct_scan.cuh", "tc_filter.cuh", "range_search.cuh",
+DEPS = ["fenix_knn.cu", "common.cuh", "exact_scan.cuh", "direct_scan.cuh", "tc_filter.cuh", "range_search.cuh", "kmeans.cuh",
         os.path.join(ROOT, "include", "fenix_knn.h")]
 
 NVCC_FLAGS = [

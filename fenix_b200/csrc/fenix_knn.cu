@@ -33,6 +33,7 @@
 #include "direct_scan.cuh"
 #include "tc_filter.cuh"
 #include "range_search.cuh"
+#include "kmeans.cuh"
 
 #include <cub/device/device_segmented_sort.cuh>
 
@@ -1604,6 +1605,227 @@ extern "C" int fx_search_range(fx_corpus* c, const float* queries, int64_t n_q, 
   std::memcpy(out_rows, ctx->h_rows.p, size_t(total) * 8);
   std::memcpy(out_dist, ctx->h_dist.p, size_t(total) * 4);
   search_account(c, run);
+  return FX_OK;
+}
+
+// ----------------------------------------------------------------------------------------
+// codebook training: one epoch of mini-batch k-means per call (DESIGN.md §4.11; csrc/kmeans.cuh)
+// ----------------------------------------------------------------------------------------
+// Staging buffer on the training device when the rows span several devices (two of them, filled alternately).
+constexpr size_t TRAIN_STAGE_BYTES = size_t(256) << 20;
+
+namespace {
+// Per-call device memory and events of fx_train_codebooks, released on every return path after the streams drain.
+struct TrainScratch {
+  struct Alloc { int device; void* p; };
+  struct Event { int device; cudaEvent_t e; };
+  std::vector<Alloc> allocs;
+  std::vector<Event> events;
+  std::vector<std::pair<int, cudaStream_t>> streams;
+  ~TrainScratch() {
+    for (auto& s : streams) { cudaSetDevice(s.first); cudaStreamSynchronize(s.second); }
+    for (auto& a : allocs) { cudaSetDevice(a.device); cudaFree(a.p); }
+    for (auto& e : events) { cudaSetDevice(e.device); cudaEventDestroy(e.e); }
+    cudaGetLastError();
+  }
+  template <typename T>
+  int alloc(int device, size_t count, T** out) {
+    void* p = nullptr;
+    cudaError_t e = cudaMalloc(&p, std::max<size_t>(count, 1) * sizeof(T));
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      return fail(FX_ENOMEM, "fx_train_codebooks: cudaMalloc(%zu) on device %d failed: %s", count * sizeof(T), device,
+                  cudaGetErrorString(e));
+    }
+    allocs.push_back({device, p});
+    *out = static_cast<T*>(p);
+    return FX_OK;
+  }
+  int event(int device, cudaEvent_t* out) {
+    FX_CUDA(cudaEventCreateWithFlags(out, cudaEventDisableTiming));
+    events.push_back({device, *out});
+    return FX_OK;
+  }
+};
+}  // namespace
+
+extern "C" int fx_train_codebooks(fx_corpus* const* shards, int32_t n_shards, int32_t metric, int32_t n_books, int32_t k,
+                                  int32_t batch, const int64_t* positions, int64_t n_steps, float* books) {
+  if (!shards || !books || (n_steps > 0 && !positions)) return fail(FX_EINVAL, "fx_train_codebooks: NULL argument");
+  if (n_shards < 1 || n_books < 1 || k < 1 || batch < 1 || n_steps < 0)
+    return fail(FX_EINVAL, "fx_train_codebooks: n_shards, n_books, k and batch must be >= 1 and n_steps >= 0");
+  if (metric < 0 || metric > 2) return fail(FX_EINVAL, "fx_train_codebooks: unknown metric %d", metric);
+  if (n_books > 65535) return fail(FX_EUNSUP, "fx_train_codebooks: at most 65535 codebooks");
+  std::vector<std::unique_ptr<Lease>> leases;
+  for (int i = 0; i < n_shards; ++i) {
+    leases.emplace_back(new Lease(shards[i]));
+    if (!leases.back()->ok) return fail(FX_EINVAL, "fx_train_codebooks: shard %d is not a live corpus handle", i);
+    if (!shards[i]->finalized) return fail(FX_ESTATE, "fx_train_codebooks: shard %d is not finalized", i);
+    if (shards[i]->dim != shards[0]->dim)
+      return fail(FX_EINVAL, "fx_train_codebooks: shard %d has dim %d, shard 0 has %d", i, shards[i]->dim, shards[0]->dim);
+    if (i > 0 && shards[i]->row_base != shards[i - 1]->row_base + shards[i - 1]->n)
+      return fail(FX_EINVAL, "fx_train_codebooks: shards must hold contiguous row ranges in order (shard %d starts at %lld, expected %lld)",
+                  i, (long long)shards[i]->row_base, (long long)(shards[i - 1]->row_base + shards[i - 1]->n));
+  }
+  const int dim = shards[0]->dim;
+  const int64_t pitch = shards[0]->pitch;
+  const int64_t lo = shards[0]->row_base, hi = shards[n_shards - 1]->row_base + shards[n_shards - 1]->n;
+  const int64_t per_step = int64_t(n_books) * batch;
+  if (per_step > (int64_t(1) << 30) || int64_t(k) * dim > (int64_t(1) << 40))
+    return fail(FX_EUNSUP, "fx_train_codebooks: n_books * batch or k * dim too large");
+  for (int64_t s = 0; s < n_steps; ++s) {
+    const int64_t* ps = positions + s * per_step;
+    for (int64_t t = 0; t < per_step; ++t) {
+      if (ps[t] < lo || ps[t] >= hi)
+        return fail(FX_EINVAL, "fx_train_codebooks: position %lld of step %lld is outside the shards' rows [%lld, %lld)",
+                    (long long)ps[t], (long long)s, (long long)lo, (long long)hi);
+      if (t > 0 && ps[t] < ps[t - 1])
+        return fail(FX_EINVAL, "fx_train_codebooks: positions of step %lld are not ascending", (long long)s);
+    }
+  }
+  if (n_steps == 0) return FX_OK;
+
+  // every distinct context locked once, in address order (two shards may share a context)
+  std::vector<fx_ctx*> ctxs;
+  for (int i = 0; i < n_shards; ++i) ctxs.push_back(shards[i]->ctx);
+  std::sort(ctxs.begin(), ctxs.end());
+  ctxs.erase(std::unique(ctxs.begin(), ctxs.end()), ctxs.end());
+  std::vector<std::unique_lock<std::mutex>> locks;
+  for (fx_ctx* x : ctxs) locks.emplace_back(x->mu);
+
+  fx_corpus* c0 = shards[0];
+  fx_ctx* ctx = c0->ctx;
+  TrainScratch scratch;
+  int64_t launches = 0;
+  const size_t book_floats = size_t(n_books) * k * dim;
+  FX_TRY(bind(ctx));
+  scratch.streams.push_back({ctx->device, ctx->stream});
+  fx::KmParams p{};
+  FX_TRY(scratch.alloc(ctx->device, book_floats, &p.books));
+  FX_TRY(scratch.alloc(ctx->device, size_t(per_step), &p.keys));
+  FX_TRY(scratch.alloc(ctx->device, size_t(per_step), &p.xx));
+  FX_TRY(scratch.alloc(ctx->device, size_t(n_books) * (k + 1), &p.off));
+  FX_TRY(scratch.alloc(ctx->device, size_t(n_books) * k, &p.cur));
+  FX_TRY(scratch.alloc(ctx->device, size_t(per_step), &p.order));
+  int64_t* d_idx = nullptr;
+  FX_TRY(scratch.alloc(ctx->device, size_t(n_steps * per_step), &d_idx));
+  const size_t upd_smem = size_t(dim) * sizeof(double);
+  FX_CUDA(cudaFuncSetAttribute(fx::km_update_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(upd_smem)));
+  FX_CUDA(cudaMemcpyAsync(p.books, books, book_floats * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+  FX_CUDA(cudaMemsetAsync(p.keys, 0xff, size_t(per_step) * sizeof(unsigned long long), ctx->stream));
+  p.pitch = pitch; p.dim = dim; p.k = k; p.batch = batch; p.metric = metric;
+
+  // assignment grid: row tiles x codeword ranges x codebooks, codeword ranges split until the grid fills the device
+  const int row_tiles = (batch + fx::KM_TR - 1) / fx::KM_TR, cw_tiles = (k + fx::KM_TC - 1) / fx::KM_TC;
+  const int64_t rows_blocks = int64_t(row_tiles) * n_books;
+  const int splits = int(std::min<int64_t>(cw_tiles, std::max<int64_t>(1, (2 * int64_t(ctx->sm_count) + rows_blocks - 1) / rows_blocks)));
+  p.cw_per_block = ((cw_tiles + splits - 1) / splits) * fx::KM_TC;
+  const dim3 assign_grid(row_tiles, (k + p.cw_per_block - 1) / p.cw_per_block, n_books);
+  auto run_steps = [&](int64_t s0, int64_t s1, const float* X) -> int {
+    p.X = X;
+    for (int64_t s = s0; s < s1; ++s) {
+      p.idx = d_idx + s * per_step;
+      fx::km_assign_kernel<<<assign_grid, fx::KM_THREADS, 0, ctx->stream>>>(p);
+      fx::km_bucket_kernel<<<n_books, fx::KM_BUCKET_THREADS, 0, ctx->stream>>>(p);
+      fx::km_update_kernel<<<dim3(k, n_books), fx::KM_UPDATE_THREADS, upd_smem, ctx->stream>>>(p);
+      FX_CUDA(cudaGetLastError());
+      launches += 3;
+    }
+    return FX_OK;
+  };
+
+  std::vector<int64_t> idx(size_t(n_steps * per_step));
+  if (n_shards == 1) {
+    // one shard: the steps read the sample rows straight from its rows
+    for (size_t t = 0; t < idx.size(); ++t) idx[t] = positions[t] - lo;
+    FX_CUDA(cudaMemcpyAsync(d_idx, idx.data(), idx.size() * sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream));
+    FX_TRY(run_steps(0, n_steps, c0->X));
+  } else {
+    // several shards: per chunk of steps, every shard gathers its part of the chunk's sample rows (in position order)
+    // and copies it into one of two staging buffers on shard 0's device; the steps read the rows from there
+    const int64_t chunk = std::max<int64_t>(1, int64_t(TRAIN_STAGE_BYTES / (size_t(per_step) * pitch * sizeof(float))));
+    const int64_t n_chunks = (n_steps + chunk - 1) / chunk;
+    std::vector<std::vector<int64_t>> rows(n_shards);          // local rows each shard gathers, chunk after chunk
+    std::vector<int64_t> cnt(size_t(n_chunks) * n_shards, 0);  // rows of shard i in chunk q
+    std::vector<int64_t> at(n_shards);
+    auto shard_of = [&](int64_t pos) {
+      int i = 0;
+      while (i + 1 < n_shards && pos >= shards[i + 1]->row_base) ++i;
+      return i;
+    };
+    for (int64_t q = 0; q < n_chunks; ++q) {
+      const int64_t t0 = q * chunk * per_step, t1 = std::min(n_steps, (q + 1) * chunk) * per_step;
+      int64_t* cq = cnt.data() + q * n_shards;
+      for (int64_t t = t0; t < t1; ++t) cq[shard_of(positions[t])]++;
+      for (int i = 0, o = 0; i < n_shards; o += int(cq[i]), ++i) at[i] = o;
+      for (int64_t t = t0; t < t1; ++t) {   // idx: the row's slot in the chunk's staging buffer, shard after shard
+        const int i = shard_of(positions[t]);
+        idx[size_t(t)] = at[i]++;
+        rows[i].push_back(positions[t] - shards[i]->row_base);
+      }
+    }
+    float* stage[2] = {nullptr, nullptr};
+    const size_t stage_rows = size_t(std::min(chunk, n_steps) * per_step);
+    FX_TRY(scratch.alloc(ctx->device, stage_rows * pitch, &stage[0]));
+    FX_TRY(scratch.alloc(ctx->device, n_chunks > 1 ? stage_rows * pitch : 0, &stage[1]));
+    cudaEvent_t consumed[2];
+    FX_TRY(scratch.event(ctx->device, &consumed[0]));
+    FX_TRY(scratch.event(ctx->device, &consumed[1]));
+    std::vector<int64_t*> d_rows(n_shards, nullptr);
+    std::vector<float*> gbuf(n_shards, nullptr);
+    std::vector<cudaEvent_t> copied(n_shards, nullptr);
+    for (int i = 0; i < n_shards; ++i) {
+      fx_ctx* xi = shards[i]->ctx;
+      int64_t most = 0;
+      for (int64_t q = 0; q < n_chunks; ++q) most = std::max(most, cnt[size_t(q * n_shards + i)]);
+      FX_TRY(bind(xi));
+      scratch.streams.push_back({xi->device, xi->stream});
+      FX_TRY(scratch.alloc(xi->device, rows[i].size(), &d_rows[i]));
+      FX_CUDA(cudaMemcpyAsync(d_rows[i], rows[i].data(), rows[i].size() * sizeof(int64_t), cudaMemcpyHostToDevice, xi->stream));
+      if (i > 0) {
+        FX_TRY(scratch.alloc(xi->device, size_t(most) * pitch, &gbuf[i]));
+        FX_TRY(scratch.event(xi->device, &copied[i]));
+      }
+    }
+    FX_TRY(bind(ctx));
+    FX_CUDA(cudaMemcpyAsync(d_idx, idx.data(), idx.size() * sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream));
+    std::vector<int64_t> done(n_shards, 0);   // rows of shard i gathered so far
+    for (int64_t q = 0; q < n_chunks; ++q) {
+      const int b = int(q & 1);
+      int64_t slot = 0;
+      for (int i = 0; i < n_shards; ++i) {
+        const int64_t m = cnt[size_t(q * n_shards + i)];
+        if (m == 0) continue;
+        fx_ctx* xi = shards[i]->ctx;
+        FX_TRY(bind(xi));
+        const int blocks = int(std::min<int64_t>(m, 4 * int64_t(xi->sm_count)));
+        if (i == 0) {
+          fx::km_gather_kernel<<<blocks, 256, 0, xi->stream>>>(shards[i]->X, pitch, d_rows[i] + done[i], m,
+                                                               stage[b] + slot * pitch);
+          FX_CUDA(cudaGetLastError());
+        } else {
+          if (q >= 2) FX_CUDA(cudaStreamWaitEvent(xi->stream, consumed[b], 0));
+          fx::km_gather_kernel<<<blocks, 256, 0, xi->stream>>>(shards[i]->X, pitch, d_rows[i] + done[i], m, gbuf[i]);
+          FX_CUDA(cudaGetLastError());
+          FX_CUDA(cudaMemcpyPeerAsync(stage[b] + slot * pitch, ctx->device, gbuf[i], xi->device,
+                                      size_t(m) * pitch * sizeof(float), xi->stream));
+          FX_CUDA(cudaEventRecord(copied[i], xi->stream));
+          FX_TRY(bind(ctx));
+          FX_CUDA(cudaStreamWaitEvent(ctx->stream, copied[i], 0));
+        }
+        launches++;
+        done[i] += m;
+        slot += m;
+      }
+      FX_TRY(bind(ctx));
+      FX_TRY(run_steps(q * chunk, std::min(n_steps, (q + 1) * chunk), stage[b]));
+      FX_CUDA(cudaEventRecord(consumed[b], ctx->stream));
+    }
+  }
+  FX_CUDA(cudaMemcpyAsync(books, p.books, book_floats * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+  FX_CUDA(cudaStreamSynchronize(ctx->stream));
+  ctx->launches += launches;
+  c0->stats.kernel_launches += launches;
   return FX_OK;
 }
 

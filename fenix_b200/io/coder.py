@@ -9,8 +9,8 @@ combination in the k^n product space, codebook 0 most significant (coder.py:171-
 Where the arithmetic runs: every vector-to-codeword distance (`distance`, the probe ranking of `call`, the code
 assignment behind `io.index.make`) is computed by libfenix_knn on the device against a small resident shard
 holding the codewords; the host only adds n distances per composite code and ranks k^n sums (coder.py:171-186).
-Codebook TRAINING (`make`, coder.py:93-127: mini-batch k-means, unseeded) is ingest-time host code here as it
-is in the reference (SURVEY.md section 8f rank 4) - it is not on the search path.
+Codebook TRAINING (`make`, coder.py:93-127: mini-batch k-means) runs on the device too: the host draws the seeds and
+the per-epoch permutations, and every epoch is one `fx_train_codebooks` call over the column's resident shards.
 """
 from __future__ import annotations
 
@@ -23,7 +23,6 @@ import pyarrow as pa
 
 from .. import knn
 from . import shards as _shards
-from . import table as _table
 
 LOCATION: str = "codings"
 
@@ -205,54 +204,46 @@ def assign(root: str, name: str, vectors: np.ndarray) -> np.ndarray:
     return code
 
 
-def _normalize(x: np.ndarray) -> np.ndarray:
-    return x / np.maximum(np.linalg.norm(x, axis=-1, keepdims=True), 1e-12)
+def _seed_rows(column: pa.ChunkedArray, sel: np.ndarray) -> np.ndarray:
+    """Rows at the ascending global positions `sel` of a vector column, read from its chunks."""
+    bounds = np.cumsum([0] + [len(c) for c in column.chunks])
+    which = np.searchsorted(bounds, sel, side="right") - 1
+    out = np.empty((len(sel), column.type.list_size), dtype=np.float32)
+    for w in np.unique(which):
+        hit = which == w
+        out[hit] = _shards.chunk_rows(column.chunks[w])[sel[hit] - bounds[w]]
+    return out
 
 
-def _host_distance(u: np.ndarray, v: np.ndarray, metric: str) -> np.ndarray:
-    if metric in ("euclidean", "l2"):
-        d2 = (u * u).sum(-1)[:, None] - 2.0 * (u @ v.T) + (v * v).sum(-1)[None, :]
-        return np.sqrt(np.maximum(d2, 0.0))
-    if metric == "cosine":
-        return 0.5 - 0.5 * (_normalize(u) @ _normalize(v).T)
-    if metric in ("dot", "inner_product"):
-        return -(u @ v.T)
-    raise ValueError(f"unknown metric {metric!r}")
-
-
-def make(root: str, name: str, source, column: str, config: Config) -> Coding:
+def make(root: str, name: str, source, column: str, config: Config, rng: Optional[np.random.Generator] = None) -> Coding:
     """Train codebook `name` on `column` of `source` (coder.py:93-127): n codebooks of k codewords seeded with
     random rows, then `num_epochs` passes of mini-batch k-means in which every codeword moves to the mean of itself
     and the batch vectors assigned to it (coder.py:53-65, `index_reduce(.., "mean")` counts the old codeword).
-    Ingest-time host arithmetic, unseeded like the reference's."""
+
+    The host draws the seeds and every epoch's permutation from `rng` (default: unseeded, like the reference's); the
+    epochs run on the device against the column's resident shards (`knn.train_codebooks`, one call per epoch)."""
     import torch
 
     knn.metric_code(config["metric"])
-    data = _table.load(root, source)
+    data = _shards.load_table(root, source)
     n, k, bs = int(config["num_codebooks"]), int(config["codebook_size"]), int(config["batch_size"])
-    rows = np.concatenate([_shards.chunk_rows(c) for c in data.column(column).chunks]) if data.num_rows else np.empty((0, 0), np.float32)
-    if len(rows) < n * k:
-        raise ValueError(f"{len(rows)} rows cannot seed {n} codebooks of {k} codewords")
-    rng = np.random.default_rng()
-    books = rows[np.sort(rng.permutation(len(rows))[: n * k])].reshape(n, k, -1).astype(np.float32)
-    cosine = config["metric"] == "cosine"
-    for _ in range(int(config["num_epochs"])):
-        perm = rng.permutation(len(rows))
-        step = n * bs
-        for lo in range(0, len(perm) // step * step, step):
-            sample = rows[np.sort(perm[lo: lo + step])].reshape(n, bs, -1)
-            for j in range(n):
-                q, v = (_normalize(books[j]), _normalize(sample[j])) if cosine else (books[j], sample[j])
-                nearest = np.argmin(_host_distance(v, q, config["metric"]), axis=-1)
-                total, count = q.copy(), np.ones(k, dtype=np.float32)
-                np.add.at(total, nearest, v)
-                np.add.at(count, nearest, 1.0)
-                q = total / count[:, None]
-                books[j] = _normalize(q) if cosine else q
+    total = data.num_rows
+    if total < n * k:
+        raise ValueError(f"{total} rows cannot seed {n} codebooks of {k} codewords")
+    rng = np.random.default_rng() if rng is None else rng
+    vectors = data.column(column)
+    books = _seed_rows(vectors, np.sort(rng.permutation(total)[: n * k])).reshape(n, k, -1)
+    step = n * bs
+    with _shards.get(root, source, column, data) as shard:
+        for _ in range(int(config["num_epochs"])):
+            perm = rng.permutation(total)
+            steps = total // step
+            positions = np.sort(perm[: steps * step].reshape(steps, step), axis=1)
+            books = knn.train_codebooks(shard.corpora, config["metric"], books, bs, positions)
     path = path_of(root, name)
     os.makedirs(os.path.dirname(path), exist_ok=True)
     with open(path, "wb") as f:
-        torch.save({"tensor": torch.from_numpy(np.ascontiguousarray(books)), "column": data.column(column).type,
+        torch.save({"tensor": torch.from_numpy(np.ascontiguousarray(books)), "column": vectors.type,
                     "config": dict(config)}, f)
     return load(root, name)
 

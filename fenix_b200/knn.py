@@ -20,6 +20,7 @@ import numpy as np
 __all__ = [
     "FenixKnnError", "Context", "Corpus", "Comm", "Group", "Stats", "METRICS", "metric_code",
     "PREC_FP32", "PREC_TF32", "PREC_BF16", "PREC_EXACT_SCAN", "load_library", "library_path", "COMM_ID_BYTES",
+    "train_codebooks",
 ]
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -42,7 +43,7 @@ ABI_SYMBOLS = (
     "fx_merge_topk", "fx_get_stats", "fx_debug_scores", "fx_last_error", "fx_abi_version", "fx_set_option",
     "fx_comm_unique_id", "fx_comm_init_rank", "fx_comm_destroy", "fx_search_sharded", "fx_search_sharded_device",
     "fx_group_create", "fx_group_size", "fx_group_ctx", "fx_group_search", "fx_group_destroy",
-    "fx_corpus_set_cells", "fx_search_cells", "fx_search_range",
+    "fx_corpus_set_cells", "fx_search_cells", "fx_search_range", "fx_train_codebooks",
 )
 
 
@@ -145,6 +146,7 @@ def load_library() -> ctypes.CDLL:
         lib.fx_corpus_set_cells.argtypes = [vp, vp, i64, vp, i64]
         lib.fx_search_cells.argtypes = [vp, vp, i64, i32, i32, vp, i32, vp, vp, vp]
         lib.fx_search_range.argtypes = [vp, vp, i64, i32, ctypes.c_float, i32, vp, i64, vp, vp, vp]
+        lib.fx_train_codebooks.argtypes = [ctypes.POINTER(vp), i32, i32, i32, i32, i32, vp, i64, vp]
         for name in ABI_SYMBOLS:
             fn = getattr(lib, name)
             if name not in ("fx_last_error", "fx_group_ctx"):
@@ -243,6 +245,30 @@ def cells_csr(cell_of_row: np.ndarray) -> tuple[np.ndarray, np.ndarray]:
     if n_cells:
         np.cumsum(np.bincount(cells, minlength=n_cells), out=off[1:])
     return inv, off
+
+
+def train_codebooks(shards: "list[Corpus]", metric: str | int, books: np.ndarray, batch: int,
+                    positions: np.ndarray) -> np.ndarray:
+    """One epoch of mini-batch k-means on the device (fx_train_codebooks): `books` (n, k, D) float32 codewords, trained
+    on the rows of the contiguous row shards `shards` (shard 0's device trains). `positions` (n_steps, n * batch) holds
+    global row positions, ascending within a step; step s trains codebook j on positions[s, j*batch:(j+1)*batch].
+    Returns the trained codewords (a new array)."""
+    m = metric if isinstance(metric, int) else metric_code(metric)
+    out = np.array(books, dtype=np.float32, order="C", copy=True)
+    if out.ndim != 3:
+        raise ValueError(f"books must be (n_books, k, dim), got shape {out.shape}")
+    pos = np.ascontiguousarray(positions, dtype=np.int64)
+    if pos.ndim != 2 or pos.shape[1] != out.shape[0] * int(batch):
+        raise ValueError(f"positions must be (n_steps, {out.shape[0]} * batch), got shape {pos.shape}")
+    if not shards:
+        raise ValueError("no shards")
+    if any(c.dim != out.shape[2] for c in shards):
+        raise ValueError(f"codewords have {out.shape[2]} coordinates, the shards {[c.dim for c in shards]}")
+    lib = shards[0]._lib
+    handles = (ctypes.c_void_p * len(shards))(*[c._h for c in shards])
+    _check(lib, lib.fx_train_codebooks(handles, len(shards), m, out.shape[0], out.shape[1], int(batch), pos.ctypes.data,
+                                       pos.shape[0], out.ctypes.data))
+    return out
 
 
 class Corpus:

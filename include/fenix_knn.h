@@ -193,6 +193,20 @@ int fx_distances(fx_corpus* c, const float* query, int32_t metric, float* out_di
 int fx_search_range(fx_corpus* c, const float* queries, int64_t n_q, int32_t metric, float radius, int32_t precision,
                     const uint8_t* row_mask, int64_t capacity, int64_t* out_offsets, int64_t* out_rows, float* out_dist);
 
+/* ---- IVF codebook training ------------------------------------------------------------------------------------------
+ * One epoch of mini-batch k-means over the rows of `n_shards` contiguous row shards (shard i's rows start at its
+ * row_base; all shards share dim). books [n_books][k][dim] HOST, in: current codewords, out: trained.
+ * positions [n_steps][n_books * batch] HOST, global row positions, ascending within a step; step s trains codebook j
+ * on positions[s][j*batch .. (j+1)*batch). metric as fx_search. Runs on shard 0's device; rows of other shards are
+ * gathered on their devices and copied there in bounded chunks. n_steps = 0 leaves `books` untouched.
+ * Per step and codebook: every sample row takes the codeword with the smallest fp32 distance (fx_search's distance,
+ * fp64 sums in ascending coordinate order; ties to the lowest codeword), then every codeword becomes
+ * (old + sum of its rows) / (1 + count), summed in fp64 in sample order and rounded once to fp32. Cosine: the old
+ * codeword and the rows are normalised (x / max(|x|, 1e-12), fp64) before the sum and the mean after it. The result
+ * is deterministic: the same call gives the same bits. */
+int fx_train_codebooks(fx_corpus* const* shards, int32_t n_shards, int32_t metric, int32_t n_books, int32_t k,
+                       int32_t batch, const int64_t* positions, int64_t n_steps, float* books);
+
 /* Merge `n_lists` per-shard results (DEVICE, each [n_q*k], laid out list-major:
  * rows[l*n_q*k + q*k + j]) into the global top-k ordered by (distance, row).
  * The step after the all-gather of the k*world candidates (fx_search_sharded does both itself). Any lists * k. */
