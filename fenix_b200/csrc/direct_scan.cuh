@@ -126,10 +126,8 @@ __device__ __forceinline__ unsigned long long ds_now() {
   return t;
 }
 
-// QREG (one query, rows of <= 128 floats): the lane's sixteen query values live in registers, the multiply loop reads
-// no shared memory at all.
 // LISTS (batched IVF): one query per CTA column (blockIdx.y), rows come from the query's probed posting lists.
-template <int NQ, int R, bool QREG, bool LISTS = false>
+template <int NQ, int R, bool LISTS = false>
 __global__ void __launch_bounds__(DS_THREADS, 1)
 knn_direct_kernel(DirectParams p) {
   static_assert(!LISTS || NQ == 1, "LISTS mode scans one query per CTA");
@@ -203,14 +201,6 @@ knn_direct_kernel(DirectParams p) {
   double xa[4] = {0.0, 0.0, 0.0, 0.0}, qa[NQ][4];
 #pragma unroll
   for (int q = 0; q < NQ; ++q) { qa[q][0] = 0.0; qa[q][1] = 0.0; qa[q][2] = 0.0; qa[q][3] = 0.0; }
-  double qreg[QREG ? 16 : 1];
-  if constexpr (QREG) {
-#pragma unroll
-    for (int u = 0; u < 4; ++u) {
-#pragma unroll
-      for (int e = 0; e < 4; ++e) qreg[4 * u + e] = qs[4 * (sub + 8 * u) + e];
-    }
-  }
 
   auto item_of = [&](int st) { return (int64_t(blockIdx.x) + int64_t(st) * gridDim.x) * DS_ROWS_PER_STEP + warp * 4 + grp; };
   // the shard row behind an item: the item itself, or (LISTS) entry `item` of the query's concatenated posting lists
@@ -276,17 +266,12 @@ knn_direct_kernel(DirectParams p) {
         const int j = ch * 32 + sub + 8 * u;           // (j >= n4: x is zero, the query row is zero-padded to whole chunks)
         const double a0 = x[u].x, a1 = x[u].y, a2 = x[u].z, a3 = x[u].w;
         xa[0] = fma(a0, a0, xa[0]); xa[1] = fma(a1, a1, xa[1]); xa[2] = fma(a2, a2, xa[2]); xa[3] = fma(a3, a3, xa[3]);
-        if constexpr (QREG) {
-          qa[0][0] = fma(a0, qreg[4 * u], qa[0][0]); qa[0][1] = fma(a1, qreg[4 * u + 1], qa[0][1]);
-          qa[0][2] = fma(a2, qreg[4 * u + 2], qa[0][2]); qa[0][3] = fma(a3, qreg[4 * u + 3], qa[0][3]);
-        } else {
 #pragma unroll
-          for (int q = 0; q < NQ; ++q) {
-            const double2* qp = reinterpret_cast<const double2*>(qs + size_t(q) * pitch_q + 4 * j);
-            const double2 v0 = qp[0], v1 = qp[1];
-            qa[q][0] = fma(a0, v0.x, qa[q][0]); qa[q][1] = fma(a1, v0.y, qa[q][1]);
-            qa[q][2] = fma(a2, v1.x, qa[q][2]); qa[q][3] = fma(a3, v1.y, qa[q][3]);
-          }
+        for (int q = 0; q < NQ; ++q) {
+          const double2* qp = reinterpret_cast<const double2*>(qs + size_t(q) * pitch_q + 4 * j);
+          const double2 v0 = qp[0], v1 = qp[1];
+          qa[q][0] = fma(a0, v0.x, qa[q][0]); qa[q][1] = fma(a1, v0.y, qa[q][1]);
+          qa[q][2] = fma(a2, v1.x, qa[q][2]); qa[q][3] = fma(a3, v1.y, qa[q][3]);
         }
       }
     }
@@ -413,7 +398,7 @@ knn_direct_kernel(DirectParams p) {
 }
 
 // ---- host side ----
-struct DirectPlan { bool ok = false; bool qreg = true; int nq_t = 0; int r = 0; int grid = 0; int cap_steps = 0; size_t smem = 0; size_t partial_bytes = 0; };
+struct DirectPlan { bool ok = false; int nq_t = 0; int r = 0; int grid = 0; int cap_steps = 0; size_t smem = 0; size_t partial_bytes = 0; };
 
 // Shapes the kernel takes: a handful of queries, k <= 128, queries + the warps' lists + at least one step of parked
 // sums within shared memory.
@@ -437,24 +422,20 @@ inline DirectPlan direct_plan(int64_t n_rows, int pitch, int64_t n_q, int k, int
 }
 
 // More than 48 KB of dynamic shared memory needs the opt-in attribute; it is set at the launch that needs it (wide rows,
-// several queries with k > 64) rather than for all 24 instantiations at fx_init, which cost a second of module loading.
+// several queries with k > 64) rather than for all 12 instantiations at fx_init, which cost a second of module loading.
 template <typename K>
 inline void ds_launch(K kernel, dim3 grid, size_t smem, cudaStream_t stream, const DirectParams& p) {
   if (smem > size_t(48) * 1024) cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
   kernel<<<grid, DS_THREADS, smem, stream>>>(p);
 }
 
-template <int NQ, int R>
-inline void direct_launch_qr(const DirectPlan& pl, const DirectParams& p, cudaStream_t stream) {
-  if (NQ == 1 && p.pitch <= 128 && pl.qreg) ds_launch(knn_direct_kernel<1, R, true, false>, dim3(pl.grid), pl.smem, stream, p);
-  else ds_launch(knn_direct_kernel<NQ, R, false, false>, dim3(pl.grid), pl.smem, stream, p);
-}
 template <int NQ>
 inline void direct_launch_q(const DirectPlan& pl, const DirectParams& p, cudaStream_t stream) {
+  const dim3 grid(pl.grid);
   switch (pl.r) {
-    case 1: direct_launch_qr<NQ, 1>(pl, p, stream); break;
-    case 2: direct_launch_qr<NQ, 2>(pl, p, stream); break;
-    default: direct_launch_qr<NQ, 4>(pl, p, stream); break;
+    case 1: ds_launch(knn_direct_kernel<NQ, 1>, grid, pl.smem, stream, p); break;
+    case 2: ds_launch(knn_direct_kernel<NQ, 2>, grid, pl.smem, stream, p); break;
+    default: ds_launch(knn_direct_kernel<NQ, 4>, grid, pl.smem, stream, p); break;
   }
 }
 inline cudaError_t direct_launch(const DirectPlan& pl, const DirectParams& p, cudaStream_t stream) {
@@ -492,7 +473,7 @@ inline CellsPlan cells_plan(int pitch, int64_t n_q, int k, int n_probe, int64_t 
 template <int R>
 inline void cells_launch_r(const CellsPlan& pl, const DirectParams& p, int n_q, cudaStream_t stream) {
   const dim3 grid(pl.ctas, n_q);
-  ds_launch(knn_direct_kernel<1, R, false, true>, grid, pl.smem, stream, p);
+  ds_launch(knn_direct_kernel<1, R, true>, grid, pl.smem, stream, p);
 }
 inline cudaError_t cells_launch(const CellsPlan& pl, const DirectParams& p, int n_q, cudaStream_t stream) {
   switch (pl.r) {

@@ -706,18 +706,15 @@ static bool int8_wanted(const fx_corpus* c, int metric, int k, int precision) {
 static int configure_filter(fx_corpus* c, int metric, int kind, const uint8_t* d_mask, fx::TcSearch* s) {
   fx_ctx* ctx = c->ctx;
   s->kind = kind; s->pitch_b = c->pitch_b; s->shadow = 0; s->aug = 0; s->epi = metric;
-  s->hx = c->hx; s->rx = c->rx; s->Xb = c->Xb; s->Xn = c->Xn; s->X8 = c->X8; s->i8_tile = c->x8_tile;
+  s->hx = c->hx; s->rx = c->rx; s->i8_tile = c->x8_tile;
   if (kind == 2) {   // cosine over the int8 normalised shadow: upper bounds straight out of the MMA and the tile constants
     s->epi = 2; s->pitch_b = fx::I8_KB * fx::i8_n_kb(c->dim);
   } else if (kind == 1) {
-    const int errcol = ctx->tc.knobs.errcol;
     if (metric == 0) { s->aug = 1; s->epi = 2; }                       // -|x|^2/2 and the row's error weight ride in the shadow's extra columns
-    else if (metric == 1) { if (ensure_norm_shadow(c)) { s->shadow = 1; s->epi = 2; s->Xn = c->Xn; } else ensure_plain_shadow(c); }
-    else if (errcol == 1 || (errcol < 0 && c->max_norm > 2.0f * c->mean_norm)) s->aug = 2;   // inner product over rows whose norms spread:
+    else if (metric == 1) { if (ensure_norm_shadow(c)) { s->shadow = 1; s->epi = 2; } else ensure_plain_shadow(c); }
+    else if (c->max_norm > 2.0f * c->mean_norm) s->aug = 2;           // inner product over rows whose norms spread:
                                                                        // per-row error weights instead of c |q| max|x| for every row
-    if (s->aug != 0 && errcol == 0) { s->aug = metric == 0 ? 1 : 0; }
     s->c_pair = s->aug != 0 ? fx::tc_c_pair(c->dim, s->aug) : 0.0;
-    s->Xb = c->Xb; s->Xn = c->Xn;   // (a shadow may just have been built)
   }
   if (d_mask) {
     const int64_t n_alloc = ((c->n + 255) / 256) * 256;
@@ -809,8 +806,7 @@ static int search_enqueue(fx_corpus* c, const float* d_q, int64_t n_q, int metri
     }
     for (int64_t q0 = 0; q0 < n_q; q0 += fx::DS_LAUNCH_Q) {
       const int64_t nq_l = std::min<int64_t>(fx::DS_LAUNCH_Q, n_q - q0);
-      fx::DirectPlan pl = fx::direct_plan(c->n, c->pitch, nq_l, k, ctx->sm_count);
-      pl.qreg = ctx->tc.knobs.direct_qreg != 0;
+      const fx::DirectPlan pl = fx::direct_plan(c->n, c->pitch, nq_l, k, ctx->sm_count);
       fx::DirectParams p{};
       p.X = c->X; p.n_rows = c->n; p.pitch = c->pitch; p.dim = c->dim; p.row_base = c->row_base;
       p.Q = d_q + q0 * c->dim; p.n_q = int(nq_l); p.metric = metric; p.k = k; p.mask = d_mask;
@@ -884,11 +880,6 @@ static int search_settle(fx_corpus* c, SearchRun* run, bool* changed) {
   FX_CUDA(cudaStreamSynchronize(ctx->stream));
   std::vector<int> bad, starved;
   for (int64_t i = 0; i < n_q; ++i) { if (h_flags[i] == 2) starved.push_back(int(i)); else if (h_flags[i]) bad.push_back(int(i)); }
-  const bool trace = ctx->tc.knobs.debug_tiers != 0;
-  auto now_ms = [] { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
-  double t_mark = now_ms();
-  if (trace) fprintf(stderr, "[fenix tiers] main pass: %zu certificate failures, %zu starved (of %lld queries, prepass %d)\n",
-                     bad.size(), starved.size(), (long long)n_q, int(run->L.with_pre));
   // Flagged queries are settled by further filter passes over their own (small) batch:
   //  tier 0 (queries left with fewer than k candidates - there is no k-th distance to refine from): the search again with
   //         FULL candidate lists (K' entries each). Stage a keeps the sample prepass: the small batch draws its own sample
@@ -901,7 +892,7 @@ static int search_settle(fx_corpus* c, SearchRun* run, bool* changed) {
   std::vector<int> to_refine;
   to_refine.swap(bad);                 // certificate failures of the main pass: tier 1
   bool adaptive_done = false;
-  for (int stage = starved.empty() ? 2 : 0; stage <= 2 && !ctx->tc.knobs.no_refine; ++stage) {
+  for (int stage = starved.empty() ? 2 : 0; stage <= 2; ++stage) {
     if (stage == 1 && adaptive_done) continue;
     std::vector<int>& in = stage == 2 ? to_refine : starved;
     if (in.empty()) continue;
@@ -952,42 +943,17 @@ static int search_settle(fx_corpus* c, SearchRun* run, bool* changed) {
       else still.push_back(in[i]);
     }
     c->stats.refined_queries += int64_t(n_f - int(still.size()) - int(still_starved.size()));
-    if (trace) {
-      const double t = now_ms();
-      fprintf(stderr, "[fenix tiers] tier %s: %d queries in, %zu still flagged, %.3f ms\n",
-              stage == 0 ? (L2.with_pre ? "0a (sample thresholds, full lists)" : "0 (adaptive, full lists)") : stage == 1 ? "0b (adaptive, full lists)" : "1 (refinement)",
-              n_f, still.size() + still_starved.size(), t - t_mark);
-      t_mark = t;
-    }
     if (stage < 2) { starved.swap(still_starved); to_refine.insert(to_refine.end(), still.begin(), still.end()); }
     else bad.swap(still);
   }
-  if (ctx->tc.knobs.no_refine) { bad.swap(to_refine); bad.insert(bad.end(), starved.begin(), starved.end()); }
   if (!bad.empty()) {
     // tier 2: the certificate-free fp64 scan
-    std::vector<int64_t> before_rows; std::vector<float> before_dist;
-    if (trace) {   // what the tiers had for the first still-flagged query, to compare with the scan's answer
-      before_rows.resize(k); before_dist.resize(k);
-      cudaMemcpy(before_rows.data(), d_out_rows + size_t(bad[0]) * k, size_t(k) * 8, cudaMemcpyDeviceToHost);
-      cudaMemcpy(before_dist.data(), d_out_dist + size_t(bad[0]) * k, size_t(k) * 4, cudaMemcpyDeviceToHost);
-    }
     FX_TRY(ctx->d_qlist.ensure(bad.size() * sizeof(int)));
     FX_CUDA(cudaMemcpyAsync(ctx->d_qlist.p, bad.data(), bad.size() * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
     FX_TRY(run_exact_scan(c, d_q, int(n_q), static_cast<int*>(ctx->d_qlist.p), int(bad.size()), metric, k,
                           run->d_mask, d_out_rows, d_out_dist));
     FX_CUDA(cudaStreamSynchronize(ctx->stream));  // `bad` must outlive the H2D copy
-    if (trace) {
-      std::vector<int64_t> after_rows(k); std::vector<float> after_dist(k);
-      cudaMemcpy(after_rows.data(), d_out_rows + size_t(bad[0]) * k, size_t(k) * 8, cudaMemcpyDeviceToHost);
-      cudaMemcpy(after_dist.data(), d_out_dist + size_t(bad[0]) * k, size_t(k) * 4, cudaMemcpyDeviceToHost);
-      int differ = 0;
-      for (int i = 0; i < k; ++i) differ += before_rows[i] != after_rows[i];
-      fprintf(stderr, "[fenix tiers] query %d: tiers vs scan: %d of %d ranks differ; tiers d[0]=%.7g d[k-1]=%.7g rows %lld..%lld | scan d[0]=%.7g d[k-1]=%.7g rows %lld..%lld\n",
-              bad[0], differ, k, before_dist[0], before_dist[k - 1], (long long)before_rows[0], (long long)before_rows[k - 1],
-              after_dist[0], after_dist[k - 1], (long long)after_rows[0], (long long)after_rows[k - 1]);
-    }
     c->stats.fallback_queries += int64_t(bad.size());
-    if (trace) fprintf(stderr, "[fenix tiers] tier 2 (fp64 scan): %zu queries, %.3f ms\n", bad.size(), now_ms() - t_mark);
   }
   FX_CUDA(cudaEventRecord(ctx->ev_stop, ctx->stream));   // the search now ends here
   return FX_OK;
@@ -1111,7 +1077,7 @@ extern "C" int fx_search(fx_corpus* c, const float* queries, int64_t n_q, int32_
     FX_TRY(ctx->h_rows.ensure(r_bytes));
     FX_TRY(ctx->h_dist.ensure(d_bytes));
     SearchRun run;
-    run.spin = ctx->tc.knobs.direct_spin != 0 && !ctx->tc.knobs.debug_direct;
+    run.spin = !ctx->tc.knobs.debug_direct;   // (the timeline's stamps land after the completion word)
     if (n_q * int64_t(c->dim) <= fx::DS_INLINE_FLOATS) {
       run.inline_q = queries;
     } else {
@@ -1874,9 +1840,8 @@ static int enqueue_merge(fx_ctx* ctx, const int64_t* d_rows, const float* d_dist
                          int64_t rows_stride, int64_t dist_stride, int64_t* d_out_rows, float* d_out_dist) {
   const int64_t total = int64_t(n_lists) * k;
   // the lists arrive sorted: ranking every entry by binary searches over the other lists beats re-sorting them in shared
-  // memory from ~128 candidates per query on (C4's exchange, 8 x 100 per query: 0.59 -> 0.35 ms; scripts/ubench/merge_bench.py)
-  const int rank_min = ctx->tc.knobs.merge_rank_min > 0 ? ctx->tc.knobs.merge_rank_min : 128;
-  if (total < rank_min && total <= 8192) {
+  // memory from ~128 candidates per query on (C4's exchange, 8 x 100 per query: 0.59 -> 0.35 ms)
+  if (total < 128) {
     const int n_sort = next_pow2(std::max(int(total), 2));
     fx::merge_pairs_kernel<<<unsigned(n_q), 256, size_t(n_sort) * 12, ctx->stream>>>(
         d_rows, d_dist, n_lists, n_q, k, n_sort, rows_stride, dist_stride, d_out_rows, d_out_dist);

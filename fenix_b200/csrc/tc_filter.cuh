@@ -26,6 +26,7 @@
 #include <cuda_runtime.h>
 
 #include <cstdlib>
+#include <cstring>
 #include <string>
 
 #include "common.cuh"
@@ -42,10 +43,7 @@ constexpr int TC_UMMA_K = 8;               // kind::tf32: 32 bytes of K per inst
 constexpr int TC_STAGES = 4;
 constexpr int TC_ACC_STAGES = 2;           // 2 x 256 TMEM columns = all 512
 constexpr int TC_SPLIT = 2;                // two epilogue warps per TMEM lane quadrant, 128 accumulator columns each
-#ifndef FENIX_EPI_UNROLL
-#define FENIX_EPI_UNROLL 2                 // unroll factor of the epilogue's chunk-pair loop (1 = rolled, 2 = all four chunks)
-#endif
-constexpr int TC_EPI_UNROLL = FENIX_EPI_UNROLL;
+constexpr int TC_EPI_UNROLL = 2;          // unroll factor of the epilogue's chunk-pair loop (1 = rolled, 2 = all four chunks)
 constexpr int TC_EPI_WARPS = 4 * TC_SPLIT; // 4 warps cover the 128 TMEM lanes; TC_SPLIT groups split the columns
 constexpr int TC_THREADS = 32 * (4 + TC_EPI_WARPS);
 constexpr int TC_EPI_FIRST_WARP = 4;
@@ -133,100 +131,67 @@ __device__ __forceinline__ int i8_threshold(float tau, double ss, double ae) {
   return x >= 2147483647.0 ? 0x7fffffff : (x > double(I8_FLOOR) ? int(floor(x)) : I8_FLOOR);
 }
 
-// Tuning knobs. Read from the environment ONCE per context (fx_init) - the search path never calls getenv - and
-// settable per context afterwards through fx_set_option (same names).
+// Tuning options. Read from the environment ONCE per context (fx_init) - the search path never calls getenv - and
+// settable per context afterwards through fx_set_option, under the names of TC_KNOB_TABLE below.
 struct TcKnobs {
-  int kp = 0;              // FENIX_TC_KP          force K' (candidates reranked per query)
-  int fullk = 0;           // FENIX_TC_FULLK       multiply the zero padding of the last k-block too
-  int no_rq = 0;           // FENIX_TC_NO_RQ       never take the resident-query kernel
-  int slices = 0;          // FENIX_TC_SLICES      force the corpus slice count
-  int max_waves = 0;       // FENIX_TC_MAX_WAVES   units per worker at most (bounds the slice count and the candidate-list scratch)
-  int order = -1;          // FENIX_TC_ORDER       unit order of the one-CTA streaming kernel (1 = query-tile major)
-  int kp_list = 0;         // FENIX_TC_KP_LIST     candidates each (query, list) keeps at a selection
-  int pre_wide = 1;        // FENIX_TC_PRE_WIDE    sample prepass also for wide rows at large batches (0: off)
-  int pre = -1;            // FENIX_TC_PRE         0: no sample prepass
-  int pre_small = 1;       // FENIX_TC_PRE_SMALL   0: no sample prepass for one query tile over < 2048 tiles
-  double pre_safety = 0.0; // FENIX_TC_PRE_SAFETY
-  double pre_m = 0.0;      // FENIX_TC_PRE_M
-  int pf = 0;              // FENIX_TC_PF          L2 prefetch distance in tiles
-  int rq_stages = 0;       // FENIX_RQ_STAGES
-  int fin_threads = 0;     // FENIX_FIN_THREADS
-  int warm = 0;            // FENIX_TC_WARM        keep thresholds of the previous search (experiments only)
-  int pair = -1;           // FENIX_TC_PAIR        CTA-pair streaming kernel: 0 never, 1 whenever possible, -1 auto
-  int errcol = -1;         // FENIX_TC_ERRCOL      certified upper-bound scores (row error weight in the shadow): -1 auto (L2 always,
-                           //                      inner product when the shard's norms spread), 0 never, 1 always
-  int fp32_filter_tf32 = 0;// FENIX_FP32_FILTER_TF32  exact mode filters with TF32 over the fp32 rows even when a shadow exists
-  int no_refine = 0;       // FENIX_NO_REFINE      flagged queries go straight to the fp64 scan
-  int no_norm_shadow = 0;  // FENIX_NO_NORM_SHADOW cosine keeps the plain shadow + multiplicative epilogue
-  int debug_bf16 = 0;      // FENIX_DEBUG_BF16     fx_debug_scores dumps the bf16 filter's scores
-  int graph = 1;           // FENIX_GRAPH          small searches (<= 64 queries, no mask) replay a captured CUDA graph from their second
-                           //                      identical call on (0: always launch kernel by kernel)
-  int debug_tiers = 0;     // FENIX_DEBUG_TIERS    stderr trace of the certificate-failure tiers (counts, host-clock times)
-  int direct = 1;          // FENIX_DIRECT         0: never take the single-launch direct scan (direct_scan.cuh: <= 8 queries, small shards)
-  int direct_mb = 256;     // FENIX_DIRECT_MAX_MB  largest shard (MB of fp32 rows) the direct scan takes
-  int direct_spin = 1;     // FENIX_DIRECT_SPIN    fx_search waits for a direct scan by spinning on the kernel's completion word in mapped
-                           //                      host memory (0: cudaStreamSynchronize, events around the launch)
-  int direct_qreg = 0;     // FENIX_DIRECT_QREG    1: the direct scan keeps a single narrow query in registers instead of shared memory (measured
-                           //                      slower: the 32 extra registers spill)
-  int merge_rank_min = 0;  // FENIX_MERGE_RANK_MIN candidates per query (lists x k) from which the exchange merges by rank (binary searches
-                           //                      over the sorted lists) instead of a shared-memory sort; 0: built-in default
-  int debug_direct = 0;    // FENIX_DEBUG_DIRECT   stderr timeline (globaltimer stamps) of every direct scan launched by fx_search
-  int int8 = -1;           // FENIX_INT8           exact cosine filters with int8 MMAs over the int8 normalised shadow: -1 auto (rows
-                           //                      wider than 192 columns, k <= 16), 0 never, 1 whenever the metric and precision allow
-  int resident = -1;       // FENIX_TC_RESIDENT    int8 CTA-pair kernel with the query tiles resident in shared memory: -1 auto (wherever
-                           //                      the CTA-pair kernel runs and the tile fits), 0 never, 1 whenever it fits
+  int kp = 0;              // force K' (candidates reranked per query)
+  int no_rq = 0;           // never take the resident-query kernel
+  int slices = 0;          // force the corpus slice count
+  int pre = -1;            // 0: no sample prepass
+  double pre_safety = 0.0; // sample prepass: rows the initial threshold passes, in units of K' (0: the planner's choice)
+  double pre_m = 0.0;      // sample prepass: rank of the sample statistic (0: the planner's choice)
+  int pair = -1;           // CTA-pair streaming kernel: 0 never, 1 whenever possible, -1 auto
+  int resident = -1;       // int8 CTA-pair kernel with the query tiles resident in shared memory: -1 auto (wherever the CTA-pair
+                           // kernel runs and the tile fits), 0 never, 1 whenever it fits
+  int int8 = -1;           // exact cosine filters with int8 MMAs over the int8 normalised shadow: -1 auto (rows wider than 192
+                           // columns, k <= 16), 0 never, 1 whenever the metric and precision allow
+  int fp32_filter_tf32 = 0;// exact mode filters with TF32 over the fp32 rows even when a shadow exists
+  int no_norm_shadow = 0;  // cosine keeps the plain shadow + multiplicative epilogue
+  int debug_bf16 = 0;      // fx_debug_scores dumps the bf16 filter's scores
+  int graph = 1;           // small searches (<= 64 queries, no mask) replay a captured CUDA graph from their second identical
+                           // call on (0: always launch kernel by kernel)
+  int direct = 1;          // 0: never take the single-launch direct scan (direct_scan.cuh: <= 8 queries, small shards)
+  int direct_mb = 256;     // largest shard (MB of fp32 rows) the direct scan takes
+  int debug_direct = 0;    // stderr timeline (globaltimer stamps) of every direct scan launched by fx_search. Kept although
+                           // it is a debug aid: without its stamps ptxas (CUDA 12.9) spills in knn_direct_kernel<2, 4>
+                           // (16 B) and gives two other instances 2 more registers
 };
-// name = the environment variable's name; value = its text, or null to restore the default. False: unknown name.
+// Every option once: its name (the environment variable's) and the member it sets, an integer (atoi) or a real (atof).
+using TcKnobInt = int TcKnobs::*;
+using TcKnobReal = double TcKnobs::*;
+struct TcKnobDef { const char* name; TcKnobInt i; TcKnobReal r; };
+inline const TcKnobDef TC_KNOB_TABLE[] = {
+    {"FENIX_TC_KP", &TcKnobs::kp, nullptr},
+    {"FENIX_TC_NO_RQ", &TcKnobs::no_rq, nullptr},
+    {"FENIX_TC_SLICES", &TcKnobs::slices, nullptr},
+    {"FENIX_TC_PRE", &TcKnobs::pre, nullptr},
+    {"FENIX_TC_PRE_SAFETY", nullptr, &TcKnobs::pre_safety},
+    {"FENIX_TC_PRE_M", nullptr, &TcKnobs::pre_m},
+    {"FENIX_TC_PAIR", &TcKnobs::pair, nullptr},
+    {"FENIX_TC_RESIDENT", &TcKnobs::resident, nullptr},
+    {"FENIX_INT8", &TcKnobs::int8, nullptr},
+    {"FENIX_FP32_FILTER_TF32", &TcKnobs::fp32_filter_tf32, nullptr},
+    {"FENIX_NO_NORM_SHADOW", &TcKnobs::no_norm_shadow, nullptr},
+    {"FENIX_DEBUG_BF16", &TcKnobs::debug_bf16, nullptr},
+    {"FENIX_GRAPH", &TcKnobs::graph, nullptr},
+    {"FENIX_DIRECT", &TcKnobs::direct, nullptr},
+    {"FENIX_DIRECT_MAX_MB", &TcKnobs::direct_mb, nullptr},
+    {"FENIX_DEBUG_DIRECT", &TcKnobs::debug_direct, nullptr},
+};
+// value = the option's text, or null to restore the default. False: unknown name.
 inline bool tc_set_knob(TcKnobs* k, const char* name, const char* value) {
-  const std::string n(name ? name : "");
   const TcKnobs d{};
-  auto as_int = [&](int dflt) { return value ? std::atoi(value) : dflt; };
-  auto as_flag = [&]() { return (value && std::atoi(value) != 0) ? 1 : 0; };   // switches: a non-zero integer sets them
-  auto as_dbl = [&]() { return value ? std::atof(value) : 0.0; };
-  if (n == "FENIX_TC_KP") k->kp = as_int(d.kp);
-  else if (n == "FENIX_TC_FULLK") k->fullk = as_flag();
-  else if (n == "FENIX_TC_NO_RQ") k->no_rq = as_flag();
-  else if (n == "FENIX_TC_SLICES") k->slices = as_int(d.slices);
-  else if (n == "FENIX_TC_MAX_WAVES") k->max_waves = as_int(d.max_waves);
-  else if (n == "FENIX_TC_ORDER") k->order = as_int(d.order);
-  else if (n == "FENIX_TC_KP_LIST") k->kp_list = as_int(d.kp_list);
-  else if (n == "FENIX_TC_PRE_WIDE") k->pre_wide = as_int(d.pre_wide);
-  else if (n == "FENIX_TC_PRE") k->pre = as_int(d.pre);
-  else if (n == "FENIX_TC_PRE_SMALL") k->pre_small = as_int(d.pre_small);
-  else if (n == "FENIX_TC_PRE_SAFETY") k->pre_safety = as_dbl();
-  else if (n == "FENIX_TC_PRE_M") k->pre_m = as_dbl();
-  else if (n == "FENIX_TC_PF") k->pf = as_int(d.pf);
-  else if (n == "FENIX_RQ_STAGES") k->rq_stages = as_int(d.rq_stages);
-  else if (n == "FENIX_FIN_THREADS") k->fin_threads = as_int(d.fin_threads);
-  else if (n == "FENIX_TC_WARM") k->warm = as_flag();
-  else if (n == "FENIX_TC_PAIR") k->pair = as_int(d.pair);
-  else if (n == "FENIX_TC_ERRCOL") k->errcol = as_int(d.errcol);
-  else if (n == "FENIX_FP32_FILTER_TF32") k->fp32_filter_tf32 = as_flag();
-  else if (n == "FENIX_NO_REFINE") k->no_refine = as_flag();
-  else if (n == "FENIX_NO_NORM_SHADOW") k->no_norm_shadow = as_flag();
-  else if (n == "FENIX_DEBUG_BF16") k->debug_bf16 = as_flag();
-  else if (n == "FENIX_DEBUG_TIERS") k->debug_tiers = as_flag();
-  else if (n == "FENIX_GRAPH") k->graph = as_int(d.graph);
-  else if (n == "FENIX_DIRECT") k->direct = as_int(d.direct);
-  else if (n == "FENIX_DIRECT_MAX_MB") k->direct_mb = as_int(d.direct_mb);
-  else if (n == "FENIX_DEBUG_DIRECT") k->debug_direct = as_flag();
-  else if (n == "FENIX_DIRECT_SPIN") k->direct_spin = as_int(d.direct_spin);
-  else if (n == "FENIX_DIRECT_QREG") k->direct_qreg = as_int(d.direct_qreg);
-  else if (n == "FENIX_MERGE_RANK_MIN") k->merge_rank_min = as_int(d.merge_rank_min);
-  else if (n == "FENIX_INT8") k->int8 = as_int(d.int8);
-  else if (n == "FENIX_TC_RESIDENT") k->resident = as_int(d.resident);
-  else return false;
-  return true;
+  for (const TcKnobDef& o : TC_KNOB_TABLE) {
+    if (!name || std::strcmp(name, o.name) != 0) continue;
+    if (o.i) k->*o.i = value ? std::atoi(value) : d.*o.i;
+    else k->*o.r = value ? std::atof(value) : d.*o.r;
+    return true;
+  }
+  return false;
 }
 inline void tc_knobs_from_env(TcKnobs* k) {
-  static const char* const names[] = {
-      "FENIX_TC_KP", "FENIX_TC_FULLK", "FENIX_TC_NO_RQ", "FENIX_TC_SLICES", "FENIX_TC_MAX_WAVES", "FENIX_TC_ORDER", "FENIX_TC_KP_LIST",
-      "FENIX_TC_PRE_WIDE", "FENIX_TC_PRE", "FENIX_TC_PRE_SMALL", "FENIX_TC_PRE_SAFETY", "FENIX_TC_PRE_M", "FENIX_TC_PF", "FENIX_RQ_STAGES",
-      "FENIX_FIN_THREADS", "FENIX_TC_WARM", "FENIX_TC_PAIR", "FENIX_TC_ERRCOL", "FENIX_FP32_FILTER_TF32", "FENIX_NO_REFINE",
-      "FENIX_NO_NORM_SHADOW", "FENIX_DEBUG_BF16", "FENIX_DEBUG_TIERS", "FENIX_GRAPH", "FENIX_DIRECT", "FENIX_DIRECT_MAX_MB", "FENIX_DEBUG_DIRECT", "FENIX_DIRECT_SPIN", "FENIX_DIRECT_QREG", "FENIX_MERGE_RANK_MIN", "FENIX_INT8", "FENIX_TC_RESIDENT"};
-  for (const char* name : names) {
-    if (const char* v = std::getenv(name)) tc_set_knob(k, name, v);
-  }
+  for (const TcKnobDef& o : TC_KNOB_TABLE)
+    if (const char* v = std::getenv(o.name)) tc_set_knob(k, o.name, v);
 }
 
 struct TcState {
@@ -258,7 +223,6 @@ struct TcSearch {
   const uint32_t* tau_fixed; // refinement pass: preset per-query admission thresholds (ordered encoding) or null
   int epi;                   // epilogue form: 0 score = acc + hx[row], 1 score = acc * rx[row], 2 score = acc
   int shadow;                // kind 1: 0 = plain shadow (+ augmented columns), 1 = normalised shadow
-  const void* Xb; const void* Xn; const void* X8;   // device addresses of the shadows (L2 prefetch)
   int aug;                   // kind 1: the query's augmented columns. 1 (L2): [1, 1, 1, u] pick up the shadow's -|x|^2/2 terms
                              // and the row's error weight; 2 (inner product, rows of very different norm): [0, 0, 0, u];
                              // u = c |q| rounded up, so that the filter score is a certified UPPER bound of the exact score
@@ -337,10 +301,6 @@ __device__ __forceinline__ void bulk_load_1d(void* dst, const void* src, uint32_
   asm volatile(
       "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
       ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(src)), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-// Pull `bytes` (multiple of 16) at a global address into L2 without occupying shared memory.
-__device__ __forceinline__ void prefetch_l2(const void* src, uint32_t bytes) {
-  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(reinterpret_cast<uint64_t>(src)), "r"(bytes) : "memory");
 }
 __device__ __forceinline__ void prefetch_tmap(const CUtensorMap* map) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(map)) : "memory");
@@ -527,8 +487,6 @@ struct TcParams {
   int n_kb_data;          // data k-blocks per tile (the tile stride of the tiled shadow)
   int nk_last;            // MMA instructions (32 B of K each) of the last data block: only columns that hold data are multiplied
   int aug_line0;          // first 128-byte line of the separate augmented region of the shadow (one block per tile)
-  const unsigned char* xb; // base of the tiled bf16 shadow in use (L2 prefetch), or null
-  int pf_tiles;           // L2 prefetch distance in tiles (0: off): the TMA ring only covers ~2 tiles, far less than a DRAM miss
   int rq_stages;          // resident-query kernels (rq, CTA pair with resident query tiles): depth of the corpus-block ring
   uint32_t sleep_ns;      // producer / MMA polling loops sleep this long between polls (0: spin). Sleeping keeps their
                           // spin loops out of the epilogue warps' issue slots where the epilogue binds (narrow rows);
@@ -540,7 +498,6 @@ struct TcParams {
   uint2* wbuf;            // [units][256][cap] candidate buffers (score bits, row), one per (unit, epilogue thread)
   int* wcnt;              // [units][256] entries left in each buffer when its unit finished
   uint32_t* tau_g;        // [n_q] shared per-query threshold, ordered-uint encoding
-  int qt_major;           // unit order: 1 = all slices of a query tile adjacent, 0 = all query tiles of a slice adjacent
   int fixed;              // refinement pass: thresholds are preset in tau_g, no selection; buffer overflow sets flags[q]
   int* flags;             // [n_q]
   float* dbg;             // diagnostics: raw scores of (query tile 0) x (corpus tile 0), [128][256], or null
@@ -933,7 +890,7 @@ knn_tc_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
   // worker unit u -> (query tile of THIS CTA, corpus slice, index of this CTA's candidate-list block)
   auto decode = [&](int u, int& qt, int& slice, int& cu) {
     if (PAIR) { const int qp = u % n_qp; slice = u / n_qp; qt = 2 * qp + int(rank); cu = slice * (2 * n_qp) + qt; }
-    else { qt = p.qt_major ? u / p.n_slices : u % p.n_qt; slice = p.qt_major ? u % p.n_slices : u / p.n_qt; cu = u; }
+    else { slice = u / p.n_qt; qt = u - slice * p.n_qt; cu = u; }
   };
 
   if (warp == 0) {
@@ -986,13 +943,6 @@ knn_tc_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
               if (KIND == 0) tma_load_2d(&map_x, &full_bar[stage], a_dst + TC_A_BYTES, kb * kElemsPerBlock, t * TC_BN);
               else {
                 tma_load_2d(&map_x, &full_bar[stage], a_dst + TC_A_BYTES, 0, line);
-#ifndef FENIX_NO_PFCODE
-                if (p.pf_tiles > 0 && tv + p.pf_tiles < t1) {
-                  const int tp = (tv + p.pf_tiles) * p.tile_stride;
-                  const int64_t linep = kb < p.n_kb_data ? (int64_t(tp) * p.n_kb_data + kb) * TC_BN : int64_t(p.aug_line0) + int64_t(tp) * TC_BN;
-                  prefetch_l2(p.xb + linep * 128, TC_B_BYTES);
-                }
-#endif
               }
             }
             if (++stage == n_stages) { stage = 0; phase ^= 1; }
@@ -1263,11 +1213,6 @@ knn_rq_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
             mbar_expect_tx(&full_bar[stage], RQ_BLOCK_BYTES);
             const int line = (kb < p.n_kb_data ? (blk * p.n_kb_data + kb) * TC_BN : p.aug_line0 + blk * TC_BN) + hrow;
             tma_load_2d(&map_x, &full_bar[stage], b_ring + stage * RQ_BLOCK_BYTES, 0, line);
-            if (p.pf_tiles > 0 && tv + p.pf_tiles < t1) {
-              const int tp = (tv + p.pf_tiles) * p.tile_stride, blkp = tp >> 1;
-              const int64_t linep = (kb < p.n_kb_data ? (int64_t(blkp) * p.n_kb_data + kb) * TC_BN : int64_t(p.aug_line0) + int64_t(blkp) * TC_BN) + (tp & 1) * RQ_BN;
-              prefetch_l2(p.xb + linep * 128, RQ_BLOCK_BYTES);
-            }
             if (++stage == n_stages) { stage = 0; phase ^= 1; }
           }
           if (++acc == 2) { acc = 0; acc_phase ^= 1; }
@@ -1393,7 +1338,7 @@ knn_qerr_kernel(const float* __restrict__ Q, int n_q, int dim, double c, float* 
 __global__ void knn_prep_kernel(const float* __restrict__ Q, int n_q, int n_rows_p, int dim, int pitch, float* __restrict__ Qp,
                                 uint32_t* __restrict__ tau_g, int* __restrict__ flags,
                                 __nv_bfloat16* __restrict__ Qb, int pitch_b,
-                                const uint32_t* __restrict__ tau_fixed, int keep_tau, int aug_col, int* __restrict__ n_flagged,
+                                const uint32_t* __restrict__ tau_fixed, int aug_col, int* __restrict__ n_flagged,
                                 int aug_mode, const float* __restrict__ qerr) {
   if (blockIdx.x == 0 && threadIdx.x == 0) *n_flagged = 0;
   // Rows are written in TILE order: row qt*128 + j holds query qt*128 + (j % 32) * 4 + j / 32 (zeros past the last
@@ -1422,7 +1367,7 @@ __global__ void knn_prep_kernel(const float* __restrict__ Q, int n_q, int n_rows
     }
   }
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n_q; i += gridDim.x * blockDim.x) {
-    if (!keep_tau) tau_g[i] = tau_fixed ? tau_fixed[i] : ORD_NEG_INF;
+    tau_g[i] = tau_fixed ? tau_fixed[i] : ORD_NEG_INF;
     flags[i] = 0;
   }
 }
@@ -1477,7 +1422,7 @@ constexpr int FIN_POOL = 2048;   // candidates the finish kernel can hold in sha
 struct FinishParams {
   const float* X; int pitch; int dim; int64_t row_base;
   const float* Qp; int n_q; int n_qt; int n_slices; int cap; int metric; int k; int kp; int sort2;  // sort2: pow2 >= kp
-  const uint32_t* tau_g; const uint2* wbuf; const int* wcnt; int qt_major; int rq; int n_qp;
+  const uint32_t* tau_g; const uint2* wbuf; const int* wcnt; int rq; int n_qp;
   int* flags; int certify; float max_norm; double c_err; double c_add; double c_abs;
   int64_t* out_rows; float* out_dist;
   int* n_flagged;   // counts the queries this launch flags (read back by the host together with the results)
@@ -1486,15 +1431,14 @@ struct FinishParams {
 
 // Candidate list l of query tile qt, tile row r (the query's slot) - the layout every filter kernel writes: with the
 // resident-query kernel one list per slice (its unit holds two query tiles), else list l = (slice, half), the buffer of
-// thread slot half*128 + r of unit slice*n_qt + qt (or qt*n_slices + slice, query-tile-major order). count: its entries.
+// thread slot half*128 + r of unit slice*n_qt + qt. count: its entries.
 __device__ __forceinline__ const uint2* fin_list(const FinishParams& p, int qt, int r, int l, int& count) {
   size_t unit_slot;
   if (p.rq) {
     unit_slot = (size_t(l) * p.n_qp + (qt >> 1)) * TC_SLOTS + (qt & 1) * TC_BM + r;
   } else {
     const int slice = l / TC_SPLIT, half = l % TC_SPLIT;
-    const size_t unit = p.qt_major ? size_t(qt) * p.n_slices + slice : size_t(slice) * p.n_qt + qt;
-    unit_slot = unit * TC_SLOTS + half * TC_BM + r;
+    unit_slot = size_t(slice * p.n_qt + qt) * TC_SLOTS + half * TC_BM + r;
   }
   count = p.wcnt[unit_slot];
   return p.wbuf + unit_slot * p.cap;
@@ -2141,7 +2085,6 @@ inline bool tc_supported(const TcState* st, const TcCorpus* tc, int64_t n_rows, 
 struct TcPlan {
   int n_qt, n_tiles, n_slices, tiles_per_slice, grid, units, kp, cap, n_kblocks, n_kb_data, nk_last, aug_line0, aug_col;
   int n_vtiles, tile_stride;
-  int qt_major;
   int rq;        // 1: resident-query kernel (units = query pairs x slices of 128-row tiles, one list per unit and query)
   int pair;      // 1: CTA-pair streaming kernel (units = query pairs x slices; candidate lists per CTA as in the one-CTA kernel)
   int resident;  // 1: the CTA-pair kernel with resident query tiles (int8 shadow; same units and candidate lists as pair)
@@ -2183,7 +2126,6 @@ inline TcPlan tc_plan(const TcState* st, const TcSearch& s) {
     pl.aug_line0 = pl.n_tiles * g.n_kb_data * TC_BN;
     pl.aug_col = g.aug_col;
   }
-  if (kn.fullk) pl.nk_last = TC_BK / TC_UMMA_K;   // tuning knob: multiply the zero padding too
   pl.kb_bf16 = s.kind == 2 ? (s.dim + 63) / 64 : pl.n_kblocks;
   // narrow rows and at least two query tiles: the resident-query kernel (operand traffic, not the tensor pipe, binds
   // the streaming kernel there); its tiles are 128 corpus rows, its units pair two query tiles
@@ -2211,15 +2153,15 @@ inline TcPlan tc_plan(const TcState* st, const TcSearch& s) {
   const int n_tiles_u = (n_tiles_full + pl.tile_stride - 1) / pl.tile_stride;          // tiles the units iterate over
   pl.n_vtiles = n_tiles_u;
   const int n_qu = (pl.rq || pl.pair) ? pl.n_qp : pl.n_qt;                          // query blocks per slice
-  // Slices: units = n_qt * n_slices (query-tile major, so all slices of a query tile run at the same time and
-  // share thresholds) are dealt round-robin to min(units, #SM) persistent CTAs.
+  // Slices: units = n_qt * n_slices, slice major (all query tiles of a slice adjacent; query-tile-major order, which
+  // runs all slices of a query tile at the same time, was measured slower on C3 - 112 vs 94 ms, profiles/r01_c3_sweep.txt -
+  // and removed), are dealt round-robin to min(units, #SM) persistent CTAs.
   // Maximise SM utilisation units / (G * ceil(units / G)); few slices are preferred (longer units give
   // tighter thresholds and fewer candidate lists), and every unit should span enough tiles for its
   // threshold to become selective.
   const int sms = pl.pair ? st->sm_count / 2 : st->sm_count;   // persistent workers: CTAs, or CTA pairs
   const int min_tiles = pre ? 4 : std::max(4, (8 * pl.kp + TC_BN - 1) / TC_BN) * (pl.rq ? 2 : 1);
-  const int max_waves = kn.max_waves > 0 ? kn.max_waves : TC_MAX_WAVES;
-  const int s_cap = std::max(1, (max_waves * sms) / n_qu);
+  const int s_cap = std::max(1, (TC_MAX_WAVES * sms) / n_qu);
   const int s_max = std::max(1, std::min(n_tiles_u / min_tiles, s_cap));
   double best = -1.0; int best_s = 1;
   for (int sl = 1; sl <= s_max; ++sl) {
@@ -2238,12 +2180,9 @@ inline TcPlan tc_plan(const TcState* st, const TcSearch& s) {
       best_s = (n_tiles_u + tps - 1) / tps;
     }
   }
-  pl.qt_major = 0;   // measured on C3: slice-major 94 ms vs query-tile-major 112 ms (profiles/r01_c3_sweep.txt)
-  if (kn.order >= 0) pl.qt_major = kn.order != 0;
   pl.n_slices = best_s;
   pl.tiles_per_slice = (n_tiles_u + best_s - 1) / best_s;
   pl.units = pl.n_slices * n_qu;
-  if (pl.rq || pl.pair) pl.qt_major = 0;
   // Each query's candidates are spread over L = TC_SPLIT * n_slices lists. A list does not need to keep K'
   // entries: the global top-k lands ~k/L per list, so keeping 2k/L + 16 (>= 32) per list gives much tighter
   // local thresholds (fewer appends and selections). If a query's neighbours are concentrated in few lists
@@ -2258,7 +2197,6 @@ inline TcPlan tc_plan(const TcState* st, const TcSearch& s) {
     // query's global threshold vouches for m candidates only): with quotas of k rounded up the reference tests' clustered
     // rows at C2 scale lose their 800 starved queries per batch (4.5 -> 3.3 ms per step; Gaussian rows unchanged).
     if (s.seeded && !pre && !s.full_lists && !s.tau_fixed) pl.kp_list = std::min(pl.kp, std::max(pl.kp_list, (s.k + 31) & ~31));
-    if (!pre && !s.full_lists && kn.kp_list >= 32) pl.kp_list = std::min(pl.kp, (kn.kp_list + 31) & ~31);
     pl.cap = (s.tau_fixed || pre) ? pl.cap : tc_cap(pl.kp_list);
   }
   pl.grid = int(std::min<long>(pl.units, sms)) * (pl.pair ? 2 : 1);
@@ -2363,9 +2301,8 @@ inline bool tc_prepass_config(const TcState* st, const TcSearch& s, const TcPlan
   // but units get SHORT when the corpus is sharded (1.25M rows per GPU: 132 tiles per unit) and per-list thresholds - each
   // list keeps its own 32 best, ~2400 admitted rows per query over 74 lists - stay loose for most of a unit: measured on
   // one 8-GPU shard of C3 the filter kernel takes 6.35 ms without and 5.09 ms with the sample's GLOBAL thresholds
-  // (0.76 -> 0.95 of the burst bf16 peak, profiles/r02_sweep_prepass.txt). On by default; FENIX_TC_PRE_WIDE=0 disables.
+  // (0.76 -> 0.95 of the burst bf16 peak, profiles/r02_sweep_prepass.txt).
   const bool wide = main_pl.kb_bf16 > 4;
-  if (wide && main_pl.n_qt > 3 && !kn.pre_wide) return false;
   if (s.epi != 2) return false;                            // a row mask (predicate / IVF cells) of unknown selectivity: the
                                                            // sample says nothing about how many LIVE rows pass a threshold
   if (kn.pre == 0) return false;
@@ -2382,8 +2319,6 @@ inline bool tc_prepass_config(const TcState* st, const TcSearch& s, const TcPlan
   int stride = int(double(main_pl.kp) * safety / target_m);         // S = N / stride, m = safety K' S / N
   const int64_t n_tiles_full = (s.n_rows + tile_rows - 1) / tile_rows;
   if (stride < 4 || n_tiles_full / stride < 32) return false;       // shard too small for a sample to pay off
-  // FENIX_TC_PRE_SMALL=0: no sample for one query tile over a small shard (single-query searches of a 100k-row table)
-  if (main_pl.n_qt == 1 && n_tiles_full < 2048 && kn.pre_small == 0) return false;
   const int rec_per_tile = main_pl.rq ? 1 : TC_SPLIT;
   // at most 4096 records per query (they are held in registers by the tau0 kernel) and 256 MB of records in all
   const int64_t max_rec = std::min<int64_t>(4096, std::max<int64_t>(64, (int64_t(1) << 26) / std::max(s.n_q, 1)));
@@ -2410,7 +2345,7 @@ inline FinishParams tc_finish_params(const TcSearch& s, const TcPlan& pl, void* 
   f.n_slices = pl.n_slices; f.cap = pl.cap; f.metric = s.metric; f.k = s.k; f.kp = pl.kp;
   int sort2 = 2; while (sort2 < pl.kp) sort2 <<= 1;
   f.sort2 = sort2; f.tau_g = reinterpret_cast<uint32_t*>(base + pl.off_tau); f.wbuf = reinterpret_cast<uint2*>(base + pl.off_wbuf);
-  f.wcnt = reinterpret_cast<int*>(base + pl.off_wcnt); f.qt_major = pl.qt_major; f.rq = pl.rq; f.n_qp = pl.n_qp;
+  f.wcnt = reinterpret_cast<int*>(base + pl.off_wcnt); f.rq = pl.rq; f.n_qp = pl.n_qp;
   f.flags = reinterpret_cast<int*>(base + pl.off_flags); f.certify = s.certify ? 1 : 0;
   f.max_norm = s.max_norm; tc_cert_consts(s, &f.c_err, &f.c_add, &f.c_abs); f.out_rows = s.out_rows; f.out_dist = s.out_dist;
   f.unit_q = s.kind == 2 ? 1 : 0;
@@ -2418,7 +2353,7 @@ inline FinishParams tc_finish_params(const TcSearch& s, const TcPlan& pl, void* 
 }
 
 // One filter launch (+ finish) over the plan of `s`; queries / state have been prepared in `scratch` already.
-inline bool tc_run_pass(TcState* st, TcCorpus* tc, const TcSearch& s, const TcPlan& pl, void* scratch, const CUtensorMap& map_q,
+inline bool tc_run_pass(TcCorpus* tc, const TcSearch& s, const TcPlan& pl, void* scratch, const CUtensorMap& map_q,
                         std::string* err) {
   char* base = static_cast<char*>(scratch);
   uint32_t* tau_g = reinterpret_cast<uint32_t*>(base + pl.off_tau);
@@ -2433,15 +2368,11 @@ inline bool tc_run_pass(TcState* st, TcCorpus* tc, const TcSearch& s, const TcPl
   p.tiles_per_slice = pl.tiles_per_slice; p.n_vtiles = pl.n_vtiles; p.tile_stride = pl.tile_stride;
   p.n_kblocks = pl.n_kblocks; p.n_kb_data = pl.n_kb_data; p.nk_last = pl.nk_last;
   p.aug_line0 = pl.aug_line0;
-  p.xb = s.kind == 1 ? static_cast<const unsigned char*>(s.shadow == 1 ? s.Xn : s.Xb)
-                     : (s.kind == 2 ? static_cast<const unsigned char*>(s.X8) : nullptr);
   p.i8_tile = s.i8_tile; p.i8_q = reinterpret_cast<const float4*>(base + pl.off_qerr);
-  p.pf_tiles = 0;   // off: measured neutral where operands come from L2 (C2, C4) and 1.9x slower where HBM binds (C5)
-  if (st->knobs.pf > 0 && p.xb) p.pf_tiles = st->knobs.pf;
   p.kp = pl.kp_list; p.cap = pl.cap;
   p.sleep_ns = pl.n_kblocks >= 6 ? 0u : 64u;
   p.hx = s.hx; p.rx = s.rx; p.dbg = s.dbg; p.wbuf = wbuf; p.wcnt = wcnt; p.tau_g = tau_g;
-  p.qt_major = pl.qt_major; p.fixed = s.tau_fixed ? 1 : 0; p.flags = flags;
+  p.fixed = s.tau_fixed ? 1 : 0; p.flags = flags;
   if (s.ev_k0) cudaEventRecordWithFlags(s.ev_k0, s.stream, s.ev_flags);
   const int epi = s.epi;   // epilogue form: 0 add, 1 multiply, 2 none
   // dispatch on (epilogue form, operand kind, mode: filter / diagnostics dump / prepass, CTA pairs)
@@ -2459,7 +2390,6 @@ inline bool tc_run_pass(TcState* st, TcCorpus* tc, const TcSearch& s, const TcPl
   if (pl.rq) {
     const CUtensorMap& map_h = s.shadow == 1 ? tc->map_xn_h : tc->map_xb_h;
     p.rq_stages = rq_stages(pl.n_kblocks);
-    if (st->knobs.rq_stages >= 2 && st->knobs.rq_stages <= p.rq_stages) p.rq_stages = st->knobs.rq_stages;
     const uint32_t rq_smem = rq_smem_bytes(pl.n_kblocks);
     if (pre) {
       if (epi == 0) launch(knn_rq_filter_kernel<0, 2>, map_h, rq_smem, 1);
@@ -2531,8 +2461,7 @@ inline bool tc_run_pass(TcState* st, TcCorpus* tc, const TcSearch& s, const TcPl
   // many short lists per query (small batches split over all SMs): more warps sweep them in parallel
   // few lists, many candidates to rerank (K' >= 128: k = 100): 128-thread CTAs - more of them per SM cover the scattered
   // exact-row reads better (C2: 2.87 -> 2.78 ms per step; 512 threads: 3.04)
-  int fin_threads = (pl.rq ? 1 : TC_SPLIT) * pl.n_slices > 32 ? 1024 : (pl.kp >= 128 && pl.kp <= 512 ? 128 : 256);   // (refinement passes rerank up to 1024 survivors: 256)
-  { const int ft = st->knobs.fin_threads; if (ft == 128 || ft == 256 || ft == 512 || ft == 1024) fin_threads = ft; }
+  const int fin_threads = (pl.rq ? 1 : TC_SPLIT) * pl.n_slices > 32 ? 1024 : (pl.kp >= 128 && pl.kp <= 512 ? 128 : 256);   // (refinement passes rerank up to 1024 survivors: 256)
   knn_tc_finish_kernel<<<s.n_q, fin_threads, fin_smem, s.stream>>>(f);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) { *err = std::string("tensor-core path launch failed: ") + cudaGetErrorString(e); return false; }
@@ -2569,7 +2498,6 @@ inline bool tc_search(TcState* st, TcCorpus* tc, const TcSearch& s, const TcLaun
     *launched += 1;
   }
   knn_prep_kernel<<<std::max(prep_blocks, 1), 256, 0, s.stream>>>(s.Q, s.n_q, n_rows_p, s.dim, s.pitch, qp, tau_g, flags, qb, s.pitch_b, s.tau_fixed,
-                                                                  (!s.tau_fixed && st->knobs.warm) ? 1 : 0,
                                                                   aug ? pl.aug_col : 0, reinterpret_cast<int*>(base), s.aug, qerr);
   if (s.kind == 2) {
     knn_qprep_i8_kernel<<<(n_rows_p + 7) / 8, 256, 0, s.stream>>>(s.Q, s.n_q, n_rows_p, s.dim, s.pitch_b,
@@ -2579,10 +2507,10 @@ inline bool tc_search(TcState* st, TcCorpus* tc, const TcSearch& s, const TcLaun
   // threshold prepass over a strided sample (the padded queries and tau_g sit at the same scratch offsets in both plans)
   if (variant) *variant = (pl.rq ? 1 : 0) | (L.with_pre ? 2 : 0) | (pl.pair ? 4 : 0) | (pl.resident ? 8 : 0);
   if (L.with_pre) {
-    if (!tc_run_pass(st, tc, L.pre, L.ppl, scratch, map_q, err)) return false;
+    if (!tc_run_pass(tc, L.pre, L.ppl, scratch, map_q, err)) return false;
     *launched += 2;
   }
-  return tc_run_pass(st, tc, s, pl, scratch, map_q, err);
+  return tc_run_pass(tc, s, pl, scratch, map_q, err);
 }
 
 }  // namespace fx

@@ -134,8 +134,9 @@ int fx_corpus_finalize(fx_corpus* c);
 int fx_corpus_destroy(fx_corpus* c);
 
 /* Tuning knob of the context, by the name of the environment variable that provides its default (FENIX_TC_PRE,
- * FENIX_TC_NO_RQ, FENIX_TC_PAIR, ...; see fenix_b200/csrc/tc_filter.cuh TcKnobs). The environment is read ONCE, at
- * fx_init; the search path never calls getenv. value = NULL restores the built-in default. */
+ * FENIX_TC_NO_RQ, FENIX_TC_PAIR, ...; every name is listed once, in TC_KNOB_TABLE of fenix_b200/csrc/tc_filter.cuh).
+ * The environment is read ONCE, at fx_init; the search path never calls getenv. value = NULL restores the built-in
+ * default; an unknown name fails with FX_EINVAL. */
 int fx_set_option(fx_ctx* ctx, const char* name, const char* value);
 
 /* ---- search ---------------------------------------------------------------------------- */

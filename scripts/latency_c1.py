@@ -53,9 +53,6 @@ for b in (2, 4, 8):
     o_r = np.empty((b, K), np.int64); o_d = np.empty((b, K), np.float32)
     print(f"fx_search, {b} queries        ", timeit(lambda i: c.search_raw(qs[i % 290:].ctypes.data, b, m, K, knn.PREC_FP32, o_r.ctypes.data, o_d.ctypes.data), 500),
           f" device {c.stats().last_search_ms * 1e3:.1f} us path {c.stats().last_path}")
-c.ctx.set_option("FENIX_DIRECT_SPIN", 0)
-print("fx_search, FENIX_DIRECT_SPIN=0 (events + cudaStreamSynchronize)", timeit(raw, 1000), f" device {c.stats().last_search_ms * 1e3:.1f} us")
-c.ctx.set_option("FENIX_DIRECT_SPIN", None)
 c.ctx.set_option("FENIX_DIRECT", 0)
 for graph in (1, 0):
     c.ctx.set_option("FENIX_GRAPH", graph)

@@ -25,7 +25,7 @@ for k, lines in kernels.items():
                     ops[key] += 1
     short = k if len(k) < 150 else k[:147] + "..."
     out.append(f"{short}\n    {len(lines)} instructions; " + ", ".join(f"{a} x{b}" for a, b in ops.items()) + "\n")
-for pat, n in (("knn_tc_filter_kernel<2, 1, 0, 1>", 70), ("knn_tc_filter_kernel<2, 2, 0, 1>", 70), ("knn_rq_filter_kernel<2, 0>", 50), ("knn_direct_kernel<1, 1, false, false>", 60)):
+for pat, n in (("knn_tc_filter_kernel<2, 1, 0, 1>", 70), ("knn_tc_filter_kernel<2, 2, 0, 1>", 70), ("knn_rq_filter_kernel<2, 0>", 50), ("knn_direct_kernel<1, 1, false>", 60)):
     for k, lines in kernels.items():
         if pat in k.replace("(int)", "").replace("(bool)", ""):
             mma = [i for i, l in enumerate(lines) if "UTCHMMA" in l or "UTCIMMA" in l or "DFMA" in l]

@@ -107,6 +107,65 @@ def test_null_arguments_are_einval(built_library):
     assert lib.fx_get_stats(None, None) == knn.FX_EINVAL
 
 
+# Every name fx_set_option accepts (and fx_init reads from the environment), and names it no longer accepts.
+OPTIONS = ("FENIX_TC_KP", "FENIX_TC_NO_RQ", "FENIX_TC_SLICES", "FENIX_TC_PRE", "FENIX_TC_PRE_SAFETY", "FENIX_TC_PRE_M",
+           "FENIX_TC_PAIR", "FENIX_TC_RESIDENT", "FENIX_INT8", "FENIX_FP32_FILTER_TF32", "FENIX_NO_NORM_SHADOW",
+           "FENIX_DEBUG_BF16", "FENIX_GRAPH", "FENIX_DIRECT", "FENIX_DIRECT_MAX_MB", "FENIX_DEBUG_DIRECT")
+RETIRED_OPTIONS = ("FENIX_TC_PF", "FENIX_TC_ORDER", "FENIX_TC_WARM", "FENIX_DIRECT_QREG", "FENIX_DIRECT_SPIN",
+                   "FENIX_DEBUG_TIERS", "FENIX_NO_REFINE", "FENIX_TC_ERRCOL", "FENIX_TC_FULLK", "FENIX_TC_KP_LIST",
+                   "FENIX_TC_MAX_WAVES", "FENIX_TC_PRE_WIDE", "FENIX_TC_PRE_SMALL", "FENIX_RQ_STAGES", "FENIX_FIN_THREADS",
+                   "FENIX_MERGE_RANK_MIN", "FENIX_BF16_SHADOW", "fenix_tc_kp", "")
+
+
+@pytest.mark.gpu
+def test_set_option_names_and_defaults(built_library, monkeypatch):
+    """fx_set_option accepts exactly the option table's names (anything else: FX_EINVAL, "unknown option"), value = NULL
+    restores the built-in default, and fx_init reads the same names from the environment. FENIX_DIRECT shows it: one
+    query over a small shard takes the direct scan (path 3) unless the option is 0 (the tensor-core path, 2)."""
+    lib = knn.load_library()
+    rng = np.random.default_rng(7)
+    x = rng.standard_normal((20_000, 64), dtype=np.float32)
+    q = x[:1] + 0.01
+
+    def path(ctx):
+        c = knn.Corpus(ctx, len(x), x.shape[1])
+        c.append(x)
+        c.finalize()
+        rows, _ = c.search(q, "l2", 5)
+        assert rows[0, 0] == 0
+        p = c.stats().last_path
+        c.close()
+        return p
+
+    ctx = knn.Context(0)
+    try:
+        for name in OPTIONS:
+            ctx.set_option(name, 1)
+            ctx.set_option(name, None)
+        ctx.set_option("FENIX_TC_PRE_SAFETY", "2.5")
+        ctx.set_option("FENIX_TC_PRE_SAFETY", None)
+        for name in RETIRED_OPTIONS:
+            with pytest.raises(ValueError, match="unknown option"):
+                ctx.set_option(name, 1)
+            assert lib.fx_set_option(ctx._h, name.encode(), None) == knn.FX_EINVAL
+        assert path(ctx) == 3
+        ctx.set_option("FENIX_DIRECT", 0)
+        assert path(ctx) == 2
+        ctx.set_option("FENIX_DIRECT", None)
+        assert path(ctx) == 3
+    finally:
+        ctx.close()
+    monkeypatch.setenv("FENIX_DIRECT", "0")
+    monkeypatch.setenv("FENIX_TC_PF", "4")            # a retired name in the environment is ignored
+    ctx = knn.Context(0)
+    try:
+        assert path(ctx) == 2
+        ctx.set_option("FENIX_DIRECT", None)           # the built-in default, not the environment's value
+        assert path(ctx) == 3
+    finally:
+        ctx.close()
+
+
 def test_metric_names_match_reference():
     assert set(knn.METRICS) == {"cosine", "dot", "inner_product", "l2", "euclidean"}
     assert knn.metric_code("euclidean") == knn.metric_code("l2")
